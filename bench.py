@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the Groth16 prove hot path (BASELINE.json metric: "BN254 Groth16 prove ms + proofs/s; ...").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape tx_2p20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape tx_2p20] [--dump-outputs DIR]
 
 One "step" = one complete proof (witness -> 256-byte proof) of the rollup-shaped circuit named in
 config.workload.  Default workload = BASELINE.json configs[1]: the rollup circuit scaled to ~2^20
@@ -20,6 +20,9 @@ After the replica timing every run also measures, outside the headline timed reg
 --impl reference: the C restatement of the reference's CPU algorithm (oracle/c, kind "port": the reference's
 own prover is un-vendored JavaScript/WASM that cannot run in this image) on all host cores, rank 0 only.
 ZKR_BENCH_ONE_DEVICE=1 (flow test on a 1-GPU box): all ranks share cuda:0 and torch.distributed runs on gloo.
+--dump-outputs DIR: after the timed steps, the proof of the last timed step is written as DIR/proof.npy (rank k > 0:
+proof_rank<k>.npy), see dump_proof.  Circuit, witness, key and (r, s) are seeded or fixed, so two builds run with the
+same arguments can be compared output for output; both arms write the same file for the same workload.
 """
 import argparse
 import ctypes as C
@@ -104,6 +107,15 @@ class DevView:
 
     def __init__(self, ptr, nbytes):
         self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (int(ptr), False), "version": 2}
+
+
+def dump_proof(out_dir, name, proof):
+    """256 proof bytes (include/zkr.h: pi_a x|y, pi_b x.c0|x.c1|y.c0|y.c1, pi_c x|y) -> out_dir/<name>.npy, float64 of
+    shape (8, 32): one coordinate per row, its 32 little-endian bytes as exact values 0..255."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    a = np.frombuffer(bytes(proof), dtype=np.uint8).reshape(8, 32).astype(np.float64)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def log(*a):
@@ -268,6 +280,8 @@ def run_ours(args):
     sampler.start()
     ms, launches = timed(prove_dev, args.steps, args.warmup)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_proof(args.dump_outputs, "proof" if rank == 0 else "proof_rank%d" % rank, proof_dev.cpu().numpy())
     ms_e2e, _ = timed(prove_host, args.steps, max(args.warmup, 1))
 
     # e2e throughput through the batch entry point (the shape of many genTxVerifierProof calls): host witness
@@ -1108,11 +1122,13 @@ def run_reference(args):
     times = []
     for i in range(args.warmup + args.steps):
         t0 = time.time()
-        cbind.prove(pk_bin, wbytes, rs[0], rs[1], mode=mode, threads=cores)
+        proof = cbind.prove(pk_bin, wbytes, rs[0], rs[1], mode=mode, threads=cores)
         dt = time.time() - t0
         if i >= args.warmup:
             times.append(dt)
         log("[bench] reference step %d: %.2f s" % (i, dt))
+    if args.dump_outputs:
+        dump_proof(args.dump_outputs, "proof", proof)
     total = sum(times)
     val = len(times) / total
     n = r1.nVars
@@ -1165,11 +1181,15 @@ def main():
     ap.add_argument("--no-batch-2p22", action="store_true", help="skip the BASELINE configs[4] batch block")
     ap.add_argument("--sharded-ntt-logs", default="24,26")
     ap.add_argument("--sharded-msm-log", default="24", help="comma list of log2 sizes of the sharded G1 MSM")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the proof of the last timed step as DIR/proof.npy (float64, 8 coordinates x 32 bytes)")
     ap.add_argument("--make-key", default=None, help=argparse.SUPPRESS)
     ap.add_argument("--sweep", default="", help="msm,ntt: BASELINE configs[2..3] sweeps on one GPU with CPU baselines beside every row")
     ap.add_argument("--sweep-max-log", type=int, default=26)
     ap.add_argument("--sweep-out", default=None)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.make_key:
         make_key(args)
         return

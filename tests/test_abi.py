@@ -89,8 +89,19 @@ def test_napi_addon_source_compiles_and_serialises_ctx_calls():
 def test_bench_contract_flags():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+
+
+def test_bench_dump_proof_layout(tmp_path):
+    """bench.py --dump-outputs: the 256 proof bytes as float64 (8 coordinates x 32 bytes), exact and in order."""
+    import numpy as np
+    import bench
+    proof = bytes((7 * i + 3) % 256 for i in range(256))
+    bench.dump_proof(str(tmp_path / "out"), "proof", proof)
+    a = np.load(tmp_path / "out" / "proof.npy")
+    assert a.dtype == np.float64 and a.shape == (8, 32)
+    assert a.astype(np.uint8).tobytes() == proof and np.array_equal(a, np.round(a))
 
 
 def test_sharded_rows_log_python_mirror_matches_library():

@@ -335,3 +335,28 @@ def test_genproof_key_cache(gp):
     prover.genProof(b1, w, 3, 4, prover=gp)
     prover.genProof(bytes(b1), w, 3, 4, prover=gp)
     assert len(gp._keys) == n0 + 3                       # the binary form is cached by content, not reloaded per call
+
+
+def test_bench_dump_outputs(gp, tmp_path):
+    """bench.py --dump-outputs on the withdraw shape: the GPU arm's last timed proof equals what the C port of the
+    reference algorithm (--impl reference) writes for the same seeded workload, and it verifies."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import bench
+    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    env = dict(os.environ, TMPDIR=str(tmp_path))          # the reference arm's key file: fresh, outside the tree
+    arms = (("ours", ["--no-cpu", "--no-gpu-witness", "--no-two-in-flight"]), ("reference", ["--ref-threads", "2"]))
+    for impl, extra in arms:
+        p = subprocess.run([sys.executable, path, "--impl", impl, "--shape", "withdraw", "--steps", "2", "--warmup", "1",
+                            "--dump-outputs", str(tmp_path / impl)] + extra, capture_output=True, text=True, env=env,
+                           timeout=900)
+        assert p.returncode == 0, p.stderr[-3000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 2
+    got, want = (np.load(tmp_path / impl / "proof.npy") for impl, _ in arms)
+    assert got.dtype == np.float64 and got.shape == (8, 32)
+    assert np.array_equal(got, want)
+    r1, w = synth.generate(*synth.SHAPES["withdraw"], seed=11)
+    _, vk = keygen.synth_setup(gp.ctx, r1, bench.TOXIC)
+    assert gp.verify(gp.load_vkey(vk["bin"]), got.astype(np.uint8).tobytes(), w[1:r1.nPublic + 1])
