@@ -120,8 +120,7 @@ static __global__ void k_digits(const uint32_t* __restrict__ scalars, const uint
             carry = 1;
         }
         uint32_t pos = (uint32_t)w * n + i;
-        // a zero digit goes to a pseudo-random bucket (multiplicative hash of its position): with all of them in one bucket
-        // the 3 % {0, 1} witness values made a 390 K-entry run of nothing, i.e. ~12 K identity partials for one CTA to add
+        // a zero digit gets the sentinel key: it sorts behind every bucket and the accumulation never visits it (see kNegBit)
         keys[pos] = d ? d - 1 : sentinel;
         vals[pos] = pos | neg;
     }

@@ -8,7 +8,7 @@ import pytest
 from oracle import bn254 as bn
 from oracle import groth16 as g
 from simple_zk_rollups_b200 import _lib
-from helpers import pack, pack_g1, pack_g2, unpack
+from helpers import check_ap_msm_full_size, pack, pack_g1, pack_g2, scalar_sets, unpack
 
 pytestmark = pytest.mark.gpu
 R = bn.R
@@ -60,21 +60,6 @@ def msm(zctx, group, h, scalars):
 def want(group, pts, scalars):
     cur = bn.G1 if group == 1 else bn.G2
     return cur.to_affine(g.msm_naive(cur, pts, scalars))
-
-
-def scalar_sets(rng, n):
-    half = n // 2
-    return {
-        "uniform": [rng.randrange(R) for _ in range(n)],
-        "rollup_like": [rng.choice((0, 1)) if rng.random() < 0.3 else rng.randrange(R) for _ in range(n)],
-        "all_zero": [0] * n,
-        "all_one": [1] * n,
-        "all_rm1": [R - 1] * n,
-        "all_equal": [0x1234567890ABCDEF1234567890ABCDEF % R] * n,
-        "alternating": [(7 if i % 2 == 0 else R - 7) for i in range(n)],
-        "small": [rng.randrange(1 << 16) for _ in range(n)],
-        "half_window": [(1 << (rng.randrange(1, 250))) for _ in range(half)] + [rng.randrange(R) for _ in range(n - half)],
-    }
 
 
 @pytest.mark.parametrize("group,n,c", [(1, 1, 0), (1, 2, 4), (1, 37, 0), (1, 300, 5), (1, 300, 13), (1, 1500, 0),
@@ -142,52 +127,4 @@ def test_msm_arithmetic_progression_full_size(zctx, group, log_n):
     """SURVEY 8(d) config 3 at 2^20 (G1) / 2^17 (G2) with a HOST-ONLY expectation: the points P_i = (a0 + i d) G come
     from the oracle's C restatement (a chain of additions, no GPU), the expected sum is (sum k_i (a0 + i d) mod r) G
     on Python ints.  Scalar sets: uniform, rollup-like (3 % in {0, 1}) and every adversarial set of config 3 (iii)."""
-    from oracle import cbind
-    L = _lib.lib()
-    n = 1 << log_n
-    rng = random.Random(500 + group)
-    a0, d = rng.randrange(R), rng.randrange(R)
-    fb = bn.fixed_base(group)
-    base, step = fb.mul_many([a0, d])
-    enc = (lambda pt: pack_g1([pt]).tobytes()) if group == 1 else (lambda pt: pack_g2([pt]).tobytes())
-    pts = cbind.ap_points(group, enc(base), enc(step), n)
-    # anchor the generator itself on three points computed independently
-    width = 64 if group == 1 else 128
-    for i in (0, 1, n - 1):
-        want_pt = fb.mul_many([(a0 + i * d) % R])[0]
-        assert pts[width * i:width * (i + 1)].tobytes() == enc(want_pt)
-    h = C.c_void_p()
-    _lib.check(L.zkr_bases_load(zctx, group, _lib.buf_ptr(pts), n, 0, C.byref(h)))
-    s1 = n * (n - 1) // 2                       # sum i
-    k_eq = 0x1234567890ABCDEF1234567890ABCDEF % R
-    uni = np.random.default_rng(9).integers(0, 256, size=(n, 32), dtype=np.uint8)
-    uni[:, 31] &= 0x1F                          # < 2^253 < r
-    roll = uni.copy()
-    sel = np.random.default_rng(10).random(n) < 0.03
-    roll[sel] = 0
-    roll[sel, 0] = np.random.default_rng(11).integers(0, 2, size=int(sel.sum()), dtype=np.uint8)
-
-    def dot(arr):                               # sum k_i (a0 + i d) on Python ints
-        ks = [int.from_bytes(arr[i].tobytes(), "little") for i in range(n)]
-        return (a0 * sum(ks) + d * sum(i * k for i, k in enumerate(ks))) % R
-
-    const = lambda k: np.tile(np.frombuffer(int(k).to_bytes(32, "little"), dtype=np.uint8), (n, 1))
-    alt = const(7)
-    alt[1::2] = np.frombuffer(int(R - 7).to_bytes(32, "little"), dtype=np.uint8)
-    cases = {
-        "uniform": (uni, None), "rollup_like": (roll, None),
-        "all_zero": (const(0), 0), "all_one": (const(1), (a0 * n + d * s1) % R),
-        "all_rm1": (const(R - 1), (R - 1) * (a0 * n + d * s1) % R),
-        "all_equal": (const(k_eq), k_eq * (a0 * n + d * s1) % R),
-        "alternating": (alt, None),
-    }
-    for name, (arr, e) in cases.items():
-        if e is None:
-            e = dot(arr)
-        out = np.zeros(width, dtype=np.uint8)
-        sc = np.ascontiguousarray(arr).reshape(-1)
-        _lib.check(L.zkr_msm(zctx, h, _lib.buf_ptr(sc), n, 0, _lib.buf_ptr(out)))
-        v = unpack(out)
-        got = None if not any(v) else ((v[0], v[1]) if group == 1 else ((v[0], v[1]), (v[2], v[3])))
-        assert got == fb.mul_many([e])[0], name
-    L.zkr_bases_free(h)
+    check_ap_msm_full_size(zctx, group, 1 << log_n)
