@@ -362,6 +362,38 @@ static size_t eval_pols(fe* out, size_t m, const uint8_t* pk, size_t off, uint32
     return off;
 }
 
+/* websnark calcH: A, B on the 2m domain (even slots given, odd slots via iNTT_m + shifted NTT_m), pointwise multiply,
+ * iNTT_2m, upper half (SURVEY.md B.4 ii).  at, bt: the m = 2^bits evaluations A_T, B_T, Montgomery (not modified);
+ * h_out: m x 32 B standard form. */
+static void calc_h(const fe* at, const fe* bt, int bits, uint8_t* h_out, int mode, int threads) {
+    const size_t m = (size_t)1 << bits;
+    fe* ao = (fe*)malloc(sizeof(fe) * m); fe* bo = (fe*)malloc(sizeof(fe) * m);
+    fe* ab = (fe*)malloc(sizeof(fe) * 2 * m);
+    memcpy(ao, at, sizeof(fe) * m); memcpy(bo, bt, sizeof(fe) * m);
+    ntt(ao, bits, 1, mode, threads); ntt(bo, bits, 1, mode, threads);
+    fe g = fr_root(bits + 1), s = FR.one;
+    for (size_t i = 0; i < m; i++) { fe_mul(&ao[i], &ao[i], &s, &FR); fe_mul(&bo[i], &bo[i], &s, &FR); fe_mul(&s, &s, &g, &FR); }
+    ntt(ao, bits, 0, mode, threads); ntt(bo, bits, 0, mode, threads);
+    for (size_t i = 0; i < m; i++) { fe_mul(&ab[2 * i], &at[i], &bt[i], &FR); fe_mul(&ab[2 * i + 1], &ao[i], &bo[i], &FR); }
+    ntt(ab, bits + 1, 1, mode, threads);
+    for (size_t i = 0; i < m; i++) { fe t; fe_from_mont(&t, &ab[m + i], &FR); memcpy(h_out + 32 * i, t.v, 32); }
+    free(ao); free(bo); free(ab);
+}
+
+/* h of calcH from the evaluations alone (the GPU's zkr_h_from_evals_dev, computed by websnark's method rather than its
+ * L/U split).  at32, bt32: 2^bits x 32 B standard form; h_out: 2^bits x 32 B standard form.  mode, threads: as ntt. */
+int oracle_h_from_evals(const uint8_t* at32, const uint8_t* bt32, int bits, uint8_t* h_out, int mode, int threads) {
+    const size_t m = (size_t)1 << bits;
+    fe* at = (fe*)malloc(sizeof(fe) * m); fe* bt = (fe*)malloc(sizeof(fe) * m);
+    for (size_t i = 0; i < m; i++) {
+        rd_fe(&at[i], at32 + 32 * i); fe_to_mont(&at[i], &at[i], &FR);
+        rd_fe(&bt[i], bt32 + 32 * i); fe_to_mont(&bt[i], &bt[i], &FR);
+    }
+    calc_h(at, bt, bits, h_out, mode, threads);
+    free(at); free(bt);
+    return 0;
+}
+
 /* websnark groth16GenProof restated.  pk: binarifyProvingKey bytes; witness: n x 32 B standard form;
  * r32, s32: blinding scalars (standard form) or NULL for 0; out: 256 B proof (include/zkr.h layout).
  * mode 0: snarkjs-structured arithmetic (per-point double-and-add, recursive FFT), single thread;
@@ -380,21 +412,12 @@ int oracle_prove(const uint8_t* pk, size_t pk_len, const uint8_t* witness, size_
     for (uint32_t i = 0; i < n; i++) { rd_fe(&wm[i], witness + 32 * (size_t)i); fe_to_mont(&wm[i], &wm[i], &FR); }
     /* calcH */
     fe* at = (fe*)malloc(sizeof(fe) * m); fe* bt = (fe*)malloc(sizeof(fe) * m);
-    fe* ao = (fe*)malloc(sizeof(fe) * m); fe* bo = (fe*)malloc(sizeof(fe) * m);
-    fe* ab = (fe*)malloc(sizeof(fe) * 2 * (size_t)m);
     eval_pols(at, m, pk, pA, n, wm);
     eval_pols(bt, m, pk, pB, n, wm);
-    memcpy(ao, at, sizeof(fe) * m); memcpy(bo, bt, sizeof(fe) * m);
-    ntt(ao, bits, 1, mode, threads); ntt(bo, bits, 1, mode, threads);
-    fe g = fr_root(bits + 1), s = FR.one;
-    for (uint32_t i = 0; i < m; i++) { fe_mul(&ao[i], &ao[i], &s, &FR); fe_mul(&bo[i], &bo[i], &s, &FR); fe_mul(&s, &s, &g, &FR); }
-    ntt(ao, bits, 0, mode, threads); ntt(bo, bits, 0, mode, threads);
-    for (uint32_t i = 0; i < m; i++) { fe_mul(&ab[2 * (size_t)i], &at[i], &bt[i], &FR); fe_mul(&ab[2 * (size_t)i + 1], &ao[i], &bo[i], &FR); }
-    ntt(ab, bits + 1, 1, mode, threads);
     uint64_t (*h)[4] = (uint64_t (*)[4])malloc(32 * (size_t)m);
-    for (uint32_t i = 0; i < m; i++) { fe t; fe_from_mont(&t, &ab[(size_t)m + i], &FR); memcpy(h[i], t.v, 32); }
+    calc_h(at, bt, bits, (uint8_t*)h, mode, threads);
     if (h_out) memcpy(h_out, h, 32 * (size_t)m);
-    free(at); free(bt); free(ao); free(bo); free(ab); free(wm);
+    free(at); free(bt); free(wm);
     /* multiexps */
     const uint64_t (*w)[4] = (const uint64_t (*)[4])witness;
     g1_aff* p1 = (g1_aff*)malloc(sizeof(g1_aff) * (n > m ? n : m));

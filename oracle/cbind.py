@@ -24,6 +24,7 @@ def lib():
             build()
         L = C.CDLL(SO)
         L.oracle_ntt.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.oracle_h_from_evals.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]
         L.oracle_msm.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int]
         L.oracle_prove.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int, C.c_int, C.c_void_p]
@@ -76,6 +77,17 @@ def ntt(data, bits, inverse=False, coset=False, mode=1, threads=None):
     threads = threads or os.cpu_count() or 1
     lib().oracle_ntt(_p(data), bits, int(inverse), int(coset), mode, threads)
     return data
+
+
+def h_from_evals(at, bt, bits, mode=1, threads=None):
+    """h of calcH (websnark's 2m-point method) from A_T, B_T: numpy uint8, 2^bits x 32 B standard form each -> the same."""
+    import numpy as np
+    threads = threads or os.cpu_count() or 1
+    at, bt = np.ascontiguousarray(at, dtype=np.uint8), np.ascontiguousarray(bt, dtype=np.uint8)
+    assert at.size == bt.size == 32 << bits
+    out = np.zeros(32 << bits, dtype=np.uint8)
+    lib().oracle_h_from_evals(_p(at), _p(bt), bits, _p(out), mode, threads)
+    return out
 
 
 def ap_points(group, base_mont, step_mont, n):

@@ -453,26 +453,41 @@ __global__ void k_h_final(Fr* h, const Fr* S, const Fr* P, size_t n, int log_n, 
     v.store(h + (bitrev_out ? p : (size_t)j));
 }
 
+// ZKR_NTT_SPLIT="a[,b[,c[,d]]]" (experiment knob): explicit widths of up to four passes, 3..11 bits each, for the
+// transforms whose size they sum to.  Read once per process, like the other NTT knobs: a size's full twiddle tables are
+// cached per pass index (get_twfull), so a split that changed between two transforms of one size would pair pass i with
+// a table built for another chunk width.
+struct SplitKnob {
+    int v[4];
+    int cnt, sum;
+};
+
+const SplitKnob& split_knob() {
+    static const SplitKnob knob = [] {
+        SplitKnob s = {};
+        const char* e = getenv("ZKR_NTT_SPLIT");
+        for (const char* q = e; q && *q && s.cnt < 4;) {
+            s.v[s.cnt] = atoi(q);
+            s.sum += s.v[s.cnt++];
+            q = strchr(q, ',');
+            if (q) q++;
+        }
+        for (int i = 0; i < s.cnt; i++)
+            if (s.v[i] < 3 || s.v[i] > kTileLog) s.cnt = 0;
+        return s;
+    }();
+    return knob;
+}
+
 int plan_passes(int n, int* ks) {
     int np = (n + kTileLog - 1) / kTileLog;
     if (np < 1) np = 1;
     int base = n / np, rem = n % np;
     for (int i = 0; i < np; i++) ks[i] = base + (i < rem ? 1 : 0);
-    // ZKR_NTT_SPLIT="a,b[,c]" (experiment knob): explicit pass widths for transforms whose size they sum to
-    if (const char* e = getenv("ZKR_NTT_SPLIT")) {
-        int v[4], cnt = 0, sum = 0;
-        for (const char* q = e; q && *q && cnt < 4;) {
-            v[cnt] = atoi(q);
-            sum += v[cnt++];
-            q = strchr(q, ',');
-            if (q) q++;
-        }
-        bool ok = sum == n && cnt >= 1;
-        for (int i = 0; i < cnt; i++) ok = ok && v[i] >= 3 && v[i] <= kTileLog;
-        if (ok) {
-            for (int i = 0; i < cnt; i++) ks[i] = v[i];
-            np = cnt;
-        }
+    const SplitKnob& sk = split_knob();
+    if (sk.cnt >= 1 && sk.sum == n) {
+        for (int i = 0; i < sk.cnt; i++) ks[i] = sk.v[i];
+        np = sk.cnt;
     }
     return np;
 }

@@ -1,5 +1,6 @@
-"""Byte-level packing helpers and host-only MSM expectations shared by the GPU parity tests."""
+"""Byte-level packing helpers, full-range field samples and host-only MSM expectations shared by the GPU parity tests."""
 import ctypes as C
+import functools
 import random
 
 import numpy as np
@@ -48,6 +49,46 @@ def affine_std(group, out):
     if not any(v):
         return None
     return (v[0], v[1]) if group == 1 else ((v[0], v[1]), (v[2], v[3]))
+
+
+_R_LIMBS = np.array([(R >> (64 * i)) & ((1 << 64) - 1) for i in range(4)], dtype=np.uint64)
+
+
+def full_range(n, seed):
+    """n field elements uniform over [0, r) as n x 32 B standard form (numpy uint8): 254-bit draws (2^254 > r), the ones
+    >= r drawn again.  The first entries are pinned to r - 1, 0, 1 and the last to r - 1."""
+    rng = np.random.default_rng(seed)
+    out = np.empty((n, 4), dtype=np.uint64)
+    todo = np.arange(n)
+    while todo.size:
+        x = rng.integers(0, 1 << 64, size=(todo.size, 4), dtype=np.uint64)
+        x[:, 3] >>= np.uint64(2)
+        lt, eq = np.zeros(todo.size, dtype=bool), np.ones(todo.size, dtype=bool)
+        for i in (3, 2, 1, 0):                       # x < r, limbs compared from the top
+            lt |= eq & (x[:, i] < _R_LIMBS[i])
+            eq &= x[:, i] == _R_LIMBS[i]
+        out[todo[lt]] = x[lt]
+        todo = todo[~lt]
+    out = out.view(np.uint8).reshape(n, 32)
+    for i, v in list(enumerate((R - 1, 0, 1)))[:n] + [(n - 1, R - 1)]:
+        out[i] = np.frombuffer(int(v).to_bytes(32, "little"), dtype=np.uint8)
+    return out.reshape(-1)
+
+
+@functools.lru_cache(maxsize=8)
+def bitrev_index(bits):
+    """numpy index array p -> the bits-bit reversal of p (cached: do not modify)"""
+    i = np.arange(1 << bits, dtype=np.uint32)
+    r = np.zeros_like(i)
+    for b in range(bits):
+        r |= ((i >> np.uint32(b)) & np.uint32(1)) << np.uint32(bits - 1 - b)
+    r.setflags(write=False)
+    return r
+
+
+def bitrev_rows(buf, bits):
+    """2^bits x 32 B elements (flat numpy uint8) in bit-reversed order: out[p] = buf[rev(p)]"""
+    return np.ascontiguousarray(buf.reshape(1 << bits, 32)[bitrev_index(bits)]).reshape(-1)
 
 
 def scalar_sets(rng, n):

@@ -67,6 +67,22 @@ def test_c_ntt_modes():
             assert unpack(cbind.ntt(pack(x), bits, True, True, mode, 4)) == g.coset_intt(x, sh)
 
 
+@pytest.mark.parametrize("bits", range(1, 11))
+def test_c_h_from_evals(bits):
+    """oracle_h_from_evals (websnark's 2m-point calcH, the host reference of the GPU H pipeline at every size) against
+    the Python oracle's websnark and L/U methods, on full-range evaluations and on A_T = B_T = r - 1 (h = 0)."""
+    rng = random.Random(50 + bits)
+    m = 1 << bits
+    at = [R - 1, 0, 1][:m] + [rng.randrange(R) for _ in range(m - 3)]
+    bt = [rng.randrange(R) for _ in range(m - 1)] + [R - 1]
+    pk = dict(domainSize=m, polsA=[{i: at[i] for i in range(m)}], polsB=[{i: bt[i] for i in range(m)}])
+    want = g.calc_h_websnark(pk, [1])
+    assert want == g.calc_h_lu(pk, [1])
+    for mode in (0, 1):
+        assert unpack(cbind.h_from_evals(pack(at), pack(bt), bits, mode=mode, threads=3)) == want
+    assert not cbind.h_from_evals(pack([R - 1] * m), pack([R - 1] * m), bits).any()
+
+
 @pytest.mark.parametrize("group", [1, 2])
 def test_c_ap_points_equal_fixed_base(group):
     """oracle_ap_points (the host-side generator of the 2^20 arithmetic-progression MSM check) against per-point
