@@ -16,6 +16,9 @@
  *                             exported for the standalone sweeps of BASELINE.json configs[2..3]
  *   zkr_synth_setup       <-> `snarkjs setup --protocol groth`  prover/package.json:34,37
  *                             (synthetic keys only: toxic waste is an input)
+ *   zkr_setup_from_powers <-> the same, as a deployable key: from public powers of tau, then
+ *   zkr_setup_contribute      phase-2 delta contributions that anyone can check
+ *                             (zkr_setup_verify_contribution)
  *
  * Conventions
  *   - All multi-byte integers little-endian.  Field elements are 32 bytes = 8 x u32 limbs,
@@ -334,6 +337,61 @@ typedef struct zkr_r1cs_csc {
 } zkr_r1cs_csc;
 int zkr_synth_setup(zkr_ctx* ctx, const zkr_r1cs_csc* r1cs, const void* toxic, void* out_a, void* out_b1,
                     void* out_b2, void* out_c, void* out_h, void* out_vk);
+
+/* ---- setup from a powers-of-tau ceremony, phase-2 delta contributions ------------------------------------
+ * Keys an operator can deploy, unlike zkr_synth_setup's: nobody has to know the toxic waste.
+ *
+ * Security statement.  A key made here is sound if the phase-1 ceremony's tau, alpha and beta are unknown to
+ * everyone AND at least one phase-2 contributor erased their delta'.  A key straight out of zkr_setup_from_powers
+ * has gamma = delta = 1 (as snarkjs's `zkey new`) and is FORGEABLE until one contribution has been applied.
+ * Phase 1 is NOT verified here: neither the subgroup membership of the G2 powers nor the same-ratio consistency
+ * of the powers is checked; the powers are taken from a ceremony the caller already trusts.
+ *
+ * Phase-1 points, host memory, affine Fq-M in the binary key encoding (64 B G1, 128 B G2 = x.c0|x.c1|y.c0|y.c1);
+ * n_* counts the points given, only the first are read, so a ceremony of size 2^K >= m is passed as is:
+ *   tau_g1[k] = tau^k G1, n_tau_g1 >= 2m - 1      tau_g2[k] = tau^k G2, n_tau_g2 >= m
+ *   alpha_tau_g1[k] = alpha tau^k G1, >= m        beta_tau_g1[k] = beta tau^k G1, >= m      beta_g2 = beta G2
+ * H_(m-1) = tau^(m-1) Z(tau) G1 needs tau^(2m-1): with exactly 2m - 1 powers (a ceremony of size m) it is written as
+ * infinity.  No proof uses it -- h = (AB - C)/Z has degree <= m - 2 for every satisfying witness -- but only with
+ * n_tau_g1 >= 2m is the key byte-identical to zkr_synth_setup's for the same (tau, alpha, beta, 1, 1). */
+typedef struct zkr_powers {
+    uint32_t n_tau_g1, n_tau_g2, n_alpha_tau_g1, n_beta_tau_g1;
+    const void *tau_g1, *tau_g2, *alpha_tau_g1, *beta_tau_g1, *beta_g2;
+} zkr_powers;
+/* The seven outputs of zkr_synth_setup (same sizes, same encoding) for gamma = delta = 1, omega = omega_m as the NTT:
+ *   [L_j] = (1/m) sum_k omega^(-jk) [tau^k]    (inverse NTTs over curve points: tau_g1, alpha_tau_g1, beta_tau_g1, tau_g2)
+ *   A_i = sum_j a_ij [L_j]G1,  B1_i / B2_i the same over B in G1 / G2,
+ *   IC_i (i <= l) / C_i (i > l) = sum_j a_ij [beta L_j] + b_ij [alpha L_j] + c_ij [L_j],
+ *   H_k = [tau^(k+m)] - [tau^k] = [tau^k Z(tau)],
+ *   vk: alfa1 = alpha_tau_g1[0], beta1 = beta_tau_g1[0], delta1 = G1, beta2 = beta_g2, gamma2 = delta2 = G2.
+ * Every input is checked on the host before any launch: counts, coordinates < q, points on their curve, no power at
+ * infinity, R1CS rows < m and coefficients < r.  ZKR_E_INVALID otherwise; zkr_last_error names the section and index. */
+int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r1cs, const zkr_powers* powers, void* out_a, void* out_b1,
+                          void* out_b2, void* out_c, void* out_h, void* out_vk);
+#define ZKR_CONTRIB_RECORD_BYTES 96
+/* One phase-2 contribution with secret delta' (32 B std form, 0 < delta' < r; NULL = drawn from getrandom).
+ * pk / vk: a websnark binary proving key (zkr_pkey_load_bin's layout) and its vk block (zkr_vkey_load_bin's);
+ * out_pk / out_vk: caller buffers of the same sizes.  delta1, delta2 (key header and vk block) are multiplied by
+ * delta', every C and H point by delta'^-1, every other byte is copied.  out_record (96 B) is a Schnorr proof of
+ * knowledge of delta' for delta1_new = delta' delta1_old:  R = k delta1_old (k from getrandom),
+ *   c = SHA-256("zkr-phase2-delta" | delta1_old | delta1_new | R) as a 256-bit little-endian integer mod r
+ *       (points as their 64 key bytes, Fq-M),
+ *   z = k + c delta' mod r;   record = R (64 B, Fq-M) | z (32 B std).
+ * delta', its inverse and k are zeroed on the host and the device before the call returns.
+ * Contributions chain: call again on the output.  ZKR_E_INVALID for a malformed layout, pk and vk disagreeing on
+ * delta, delta1 / delta2 not valid points, or delta' = 0 or >= r. */
+int zkr_setup_contribute(zkr_ctx* ctx, const void* pk, size_t pk_len, const void* vk, size_t vk_len,
+                         const void* delta32, void* out_pk, void* out_vk, void* out_record);
+/* *valid = 1 iff new_pk / new_vk is old_pk / old_vk after one honest contribution proven by `record`:
+ *   every byte outside delta1, delta2, C and H is unchanged; each key's header delta1 / delta2 equal its vk's;
+ *   delta1 and delta2 (old and new) are valid points, not infinity, delta2 in the G2 subgroup;
+ *   e(delta1_new, G2) = e(G1, delta2_new);  z delta1_old = R + c delta1_new;  every new C / H point is on the curve
+ *   or infinity written as (0, R mod q);
+ *   e(X_new, delta2_new) = e(X_old, delta2_old), X = sum rho_i C_i + sum sigma_k H_k with fresh 128-bit CSPRNG
+ *   scalars shared by old and new (two GPU MSMs over the C|H section, host pairings).
+ * ZKR_E_INVALID only for a malformed old layout or buffer sizes (both keys have pk_len / vk_len bytes). */
+int zkr_setup_verify_contribution(zkr_ctx* ctx, const void* old_pk, const void* old_vk, const void* new_pk,
+                                  const void* new_vk, size_t pk_len, size_t vk_len, const void* record, int* valid);
 
 /* points[i] = scalars[i] * G (group 1: G1 generator (1,2); group 2: the G2 generator of TxVerifier.sol:30-35);
  * scalars n x 32 B std form, out n x 64 / 128 B affine Fq-M; host buffers.  Workload generator for the

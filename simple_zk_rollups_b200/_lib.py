@@ -8,6 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ZKR_LIB") or os.path.join(HERE, "libzkr.so")
 
 PROOF_BYTES = 256
+CONTRIB_RECORD_BYTES = 96
 
 
 class ZkrError(RuntimeError):
@@ -30,6 +31,11 @@ class R1csCsc(C.Structure):
                 ("domain_size", C.c_uint32), ("n_pool", C.c_uint32)] + \
                [(n, C.c_void_p) for n in ("ptr_a", "row_a", "cid_a", "ptr_b", "row_b", "cid_b",
                                           "ptr_c", "row_c", "cid_c", "pool")]
+
+
+class Powers(C.Structure):
+    _fields_ = [(n, C.c_uint32) for n in ("n_tau_g1", "n_tau_g2", "n_alpha_tau_g1", "n_beta_tau_g1")] + \
+               [(n, C.c_void_p) for n in ("tau_g1", "tau_g2", "alpha_tau_g1", "beta_tau_g1", "beta_g2")]
 
 
 _SIGS = {
@@ -102,6 +108,11 @@ _SIGS = {
     "zkr_ntt_sharded_rows_log": (C.c_int, [C.c_int, C.c_int]),
     "zkr_ntt_sharded": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "zkr_synth_setup": (C.c_int, [C.c_void_p, C.POINTER(R1csCsc), C.c_void_p] + [C.c_void_p] * 6),
+    "zkr_setup_from_powers": (C.c_int, [C.c_void_p, C.POINTER(R1csCsc), C.POINTER(Powers)] + [C.c_void_p] * 6),
+    "zkr_setup_contribute": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zkr_setup_verify_contribution": (C.c_int, [C.c_void_p] + [C.c_void_p] * 4 + [C.c_size_t, C.c_size_t, C.c_void_p,
+                                                                                  C.POINTER(C.c_int)]),
     "zkr_synth_points": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "zkr_test_field_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "zkr_test_curve_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),

@@ -1,0 +1,819 @@
+// Groth16 setup from a powers-of-tau ceremony and phase-2 delta contributions (C-ABI: zkr_setup_from_powers,
+// zkr_setup_contribute, zkr_setup_verify_contribution).  zkr.h states the math, the encodings and what a key made
+// here is sound under.
+//
+// Replaces the one-party `snarkjs setup --protocol groth` (prover/package.json:34,37), whose caller knows tau, alpha
+// and beta, with the usual two phases: public phase-1 powers (nobody knows tau) turned into the circuit key here,
+// then any number of phase-2 contributions that re-randomise delta and that anyone can check.
+//   * Lagrange bases: inverse NTTs over curve points (radix-2 DIT stages in global memory, one scalar_mul per
+//     butterfly whose twiddle is not 1; the bit reversal is folded into the affine -> XYZZ load).
+//   * Per-signal sums: one thread per nonzero computes coef * P[row] (no multiplication when coef = 1), then a
+//     segmented sum in chunks of kSegChunk entries, repeated over the partials until each column has one point, so a
+//     column of 10^5 entries costs log_32 levels instead of one serial thread.  The group law is exact: the order of
+//     the additions cannot change the affine bytes.
+//   * Contributions: one thread per C / H point multiplies by the single scalar delta'^-1 with 4-bit signed windows.
+//   * Verification: two bucketed MSMs (zkr_msm) with shared random 128-bit scalars over the C|H section, and host
+//     pairings (verify.cu).
+#include <algorithm>
+#include <cstddef>
+#include <cstring>
+#include <thread>
+#include <vector>
+
+#include "ec.cuh"
+#include "host_ec.cuh"
+#include "ntt_iface.cuh"
+
+using namespace zkr;
+
+namespace {
+
+constexpr uint32_t kSegChunk = 32;
+constexpr int kDigits = 64;            // 4-bit signed windows of a scalar < r < 2^254: the top one never carries out
+
+// ------------------------------------------------------------------------------------------------ point NTT
+// X[bitrev(k)] = P[k]: the DIT stages below then leave the transform in natural order
+template <class F>
+__global__ void k_pntt_load(const Affine<F>* __restrict__ in, XYZZ<F>* X, uint32_t m, int log_m) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    XYZZ<F>::from_affine(Affine<F>::load_ro(in + k)).store(X + (__brev(k) >> (32 - log_m)));
+}
+
+// One radix-2 DIT stage of the inverse transform (butterflies of span 2^s) over `blocks` vectors of m points
+// stored back to back: (u, v) -> (u + w v, u - w v), w = omega_m^(-j m / 2^(s+1)).
+template <class F>
+__global__ void k_pntt_stage(XYZZ<F>* X, uint32_t m, int log_m, int s, uint32_t blocks, const Fr* __restrict__ tw_lo,
+                             const Fr* __restrict__ tw_hi, int lb) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= blocks * (m / 2)) return;
+    const uint32_t b = t >> (log_m - 1), tb = t & (m / 2 - 1);
+    const uint32_t j = tb & ((1u << s) - 1);
+    XYZZ<F>* x = X + (size_t)b * m;
+    const uint32_t i0 = ((tb >> s) << (s + 1)) + j, i1 = i0 + (1u << s);
+    XYZZ<F> u = XYZZ<F>::load(x + i0), v = XYZZ<F>::load(x + i1);
+    if (j) {
+        const uint32_t e = j << (log_m - 1 - s);
+        const Fr w = Fr::load_ro(tw_lo + (e & ((1u << lb) - 1))) * Fr::load_ro(tw_hi + (e >> lb));
+        v = scalar_mul(v, w.from_mont());
+    }
+    XYZZ<F> d = u;
+    d.add(v.neg());
+    u.add(v);
+    u.store(x + i0);
+    d.store(x + i1);
+}
+
+// X[i] *= 1/m
+template <class F>
+__global__ void k_pntt_scale(XYZZ<F>* X, size_t n, const NttRoots* roots) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    scalar_mul(XYZZ<F>::load(X + i), roots->ninv.from_mont()).store(X + i);
+}
+
+template <class F>
+__device__ __forceinline__ void store_key_point(const XYZZ<F>& p, Affine<F>* out) {
+    Affine<F> a = {F::zero(), F::one()};      // infinity as binarifyProvingKey writes it: (0, R mod q)
+    if (!p.is_inf()) a = p.to_affine();
+    a.store(out);
+}
+
+// H_k = [tau^(k+m)] - [tau^k]; infinity where tau^(k+m) is not given (k = m - 1 with 2m - 1 powers)
+__global__ void k_h_from_powers(const G1Affine* __restrict__ tau, uint32_t n_tau, G1Affine* out, uint32_t m) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    G1XYZZ acc = G1XYZZ::identity();
+    if (k + m < n_tau) {
+        acc = G1XYZZ::from_affine(G1Affine::load_ro(tau + k + m));
+        acc.madd(G1Affine::load_ro(tau + k).neg());
+    }
+    store_key_point(acc, out + k);
+}
+
+// ------------------------------------------------------------------------------------------------ sparse sums
+// T[k] = cid-th pool coefficient (std form) * P[pidx[k]]
+template <class F>
+__global__ void k_terms(const XYZZ<F>* __restrict__ P, const uint32_t* __restrict__ pidx, const uint32_t* __restrict__ cid,
+                        const Fr* __restrict__ pool, XYZZ<F>* T, uint32_t nnz) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= nnz) return;
+    const XYZZ<F> p = XYZZ<F>::load(P + pidx[k]);
+    const Fr c = Fr::load_ro(pool + cid[k]);
+    bool one = c.v[0] == 1;
+#pragma unroll
+    for (int i = 1; i < 8; i++) one &= c.v[i] == 0;
+    (one ? p : scalar_mul(p, c)).store(T + k);
+}
+
+// out[c] = sum of in[start[c] .. start[c+1])
+template <class F>
+__global__ void k_seg_sum(const XYZZ<F>* __restrict__ in, const uint32_t* __restrict__ start, XYZZ<F>* out, uint32_t nch) {
+    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= nch) return;
+    const uint32_t e = start[c + 1];
+    XYZZ<F> acc = XYZZ<F>::load(in + start[c]);
+#pragma unroll 1
+    for (uint32_t k = start[c] + 1; k < e; k++) acc.add(XYZZ<F>::load(in + k));
+    acc.store(out + c);
+}
+
+// column i holds at most one point, in[ptr[i]]; an empty column is infinity
+template <class F>
+__global__ void k_col_affine(const XYZZ<F>* __restrict__ in, const uint32_t* __restrict__ ptr, Affine<F>* out, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    store_key_point(ptr[i + 1] > ptr[i] ? XYZZ<F>::load(in + ptr[i]) : XYZZ<F>::identity(), out + i);
+}
+
+__global__ void k_generators(G1Affine* g1, G2Affine* g2) {
+    generator<Fq>().store(g1);
+    generator<Fq2>().store(g2);
+}
+
+// ------------------------------------------------------------------------------------------------ contribution
+// Device copy of the contribution's secrets; zeroed before the call returns.
+struct Secrets {
+    Fr delta, k, c, z;                  // std form; c is public, z the Schnorr response
+    int8_t dig[3][kDigits];             // signed 4-bit windows of delta', delta'^-1, k
+};
+
+// digits in [-7, 8], scalar = sum dig[w] 16^w
+__device__ __forceinline__ void recode(const Fr& s, int8_t* dig) {
+    int carry = 0;
+    for (int w = 0; w < kDigits; w++) {
+        int d = (int)((s.v[w >> 3] >> ((w & 7) * 4)) & 15) + carry;
+        carry = d > 8;
+        dig[w] = (int8_t)(d - 16 * carry);
+    }
+}
+
+__global__ void k_contrib_prep(Secrets* s) {
+    recode(s->delta, s->dig[0]);
+    recode(s->delta.to_mont().inverse().from_mont(), s->dig[1]);
+    recode(s->k, s->dig[2]);
+}
+
+__global__ void k_contrib_z(Secrets* s) { s->z = (s->k.to_mont() + s->c.to_mont() * s->delta.to_mont()).from_mont(); }
+
+// pts[i] = scalar * pts[i] in place (key encoding in and out), scalar given by its signed 4-bit digits
+template <class F>
+__global__ void k_fixed_mul(Affine<F>* pts, size_t n, const int8_t* __restrict__ dig) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const Affine<F> a = Affine<F>::load(pts + i);
+    XYZZ<F> acc = XYZZ<F>::identity();
+    if (!a.is_inf()) {
+        XYZZ<F> t[8];       // t[d - 1] = d a
+        t[0] = XYZZ<F>::from_affine(a);
+#pragma unroll 1
+        for (int d = 1; d < 8; d++) {
+            t[d] = t[d - 1];
+            t[d].madd(a);
+        }
+        int top = kDigits - 1;
+        while (top > 0 && __ldg(dig + top) == 0) top--;
+#pragma unroll 1
+        for (int w = top; w >= 0; w--) {
+            if (w != top)
+#pragma unroll 1
+                for (int b = 0; b < 4; b++) acc = acc.dbl();
+            const int d = __ldg(dig + w);
+            if (d > 0) acc.add(t[d - 1]);
+            else if (d < 0) acc.add(t[-d - 1].neg());
+        }
+    }
+    store_key_point(acc, pts + i);
+}
+
+// z * P0 == P2 + c * P1 ?   (P0 = delta1_old, P1 = delta1_new, P2 = R; zc = z | c std form)
+__global__ void k_schnorr_check(const G1Affine* pts, const Fr* zc, int* ok) {
+    const G1XYZZ lhs = scalar_mul(G1XYZZ::from_affine(pts[0]), zc[0]);
+    G1XYZZ rhs = scalar_mul(G1XYZZ::from_affine(pts[1]), zc[1]);
+    rhs.add(G1XYZZ::from_affine(pts[2]));
+    if (lhs.is_inf() || rhs.is_inf()) {
+        *ok = lhs.is_inf() && rhs.is_inf();
+        return;
+    }
+    const G1Affine a = lhs.to_affine(), b = rhs.to_affine();
+    *ok = a.x == b.x && a.y == b.y;
+}
+
+// ------------------------------------------------------------------------------------------------ host helpers
+// Device buffers of one call, freed when the call returns, on its error paths too.
+struct DevAllocs {
+    std::vector<void*> p;
+    DevAllocs() = default;
+    DevAllocs(const DevAllocs&) = delete;
+    DevAllocs& operator=(const DevAllocs&) = delete;
+    ~DevAllocs() {
+        for (void* q : p) cudaFree(q);
+    }
+    template <class T>
+    int alloc(T** out, size_t bytes) {
+        ZKR_CUDA(cudaMalloc(out, bytes ? bytes : 1));
+        p.push_back(*out);
+        return ZKR_OK;
+    }
+    void release(void* q) {
+        auto it = std::find(p.begin(), p.end(), q);
+        if (it == p.end()) return;
+        cudaFree(q);
+        p.erase(it);
+    }
+};
+
+int up32(DevAllocs& a, const uint32_t* h, size_t count, uint32_t** d, cudaStream_t st) {
+    ZKR_TRY(a.alloc(d, 4 * count));
+    if (count) ZKR_CUDA(cudaMemcpyAsync(*d, h, 4 * count, cudaMemcpyHostToDevice, st));
+    return ZKR_OK;
+}
+
+void wipe(void* p, size_t n) {
+    volatile uint8_t* v = (volatile uint8_t*)p;
+    for (size_t i = 0; i < n; i++) v[i] = 0;
+}
+
+bool lt_r(const uint8_t* b32) {
+    uint32_t v[8];
+    memcpy(v, b32, 32);
+    for (int i = 7; i >= 0; i--)
+        if (v[i] != kRModulus[i]) return v[i] < kRModulus[i];
+    return false;
+}
+bool is_zero32(const uint8_t* b32) {
+    uint8_t acc = 0;
+    for (int i = 0; i < 32; i++) acc |= b32[i];
+    return acc == 0;
+}
+// b32 -= r while b32 >= r  (a 256-bit value is below 6 r)
+void reduce_r(uint8_t* b32) {
+    while (!lt_r(b32)) {
+        uint32_t v[8];
+        memcpy(v, b32, 32);
+        uint64_t borrow = 0;
+        for (int i = 0; i < 8; i++) {
+            const uint64_t d = (uint64_t)v[i] - kRModulus[i] - borrow;
+            v[i] = (uint32_t)d;
+            borrow = (d >> 63) & 1;
+        }
+        memcpy(b32, v, 32);
+    }
+}
+
+// ---- SHA-256 (FIPS 180-4), host, for the contribution challenge
+struct Sha256 {
+    uint32_t h[8] = {0x6a09e667u, 0xbb67ae85u, 0x3c6ef372u, 0xa54ff53au, 0x510e527fu, 0x9b05688cu, 0x1f83d9abu, 0x5be0cd19u};
+    uint8_t buf[64];
+    size_t fill = 0;
+    uint64_t bits = 0;
+
+    static uint32_t rotr(uint32_t x, int n) { return (x >> n) | (x << (32 - n)); }
+    void block(const uint8_t* p) {
+        static const uint32_t K[64] = {
+            0x428a2f98u, 0x71374491u, 0xb5c0fbcfu, 0xe9b5dba5u, 0x3956c25bu, 0x59f111f1u, 0x923f82a4u, 0xab1c5ed5u,
+            0xd807aa98u, 0x12835b01u, 0x243185beu, 0x550c7dc3u, 0x72be5d74u, 0x80deb1feu, 0x9bdc06a7u, 0xc19bf174u,
+            0xe49b69c1u, 0xefbe4786u, 0x0fc19dc6u, 0x240ca1ccu, 0x2de92c6fu, 0x4a7484aau, 0x5cb0a9dcu, 0x76f988dau,
+            0x983e5152u, 0xa831c66du, 0xb00327c8u, 0xbf597fc7u, 0xc6e00bf3u, 0xd5a79147u, 0x06ca6351u, 0x14292967u,
+            0x27b70a85u, 0x2e1b2138u, 0x4d2c6dfcu, 0x53380d13u, 0x650a7354u, 0x766a0abbu, 0x81c2c92eu, 0x92722c85u,
+            0xa2bfe8a1u, 0xa81a664bu, 0xc24b8b70u, 0xc76c51a3u, 0xd192e819u, 0xd6990624u, 0xf40e3585u, 0x106aa070u,
+            0x19a4c116u, 0x1e376c08u, 0x2748774cu, 0x34b0bcb5u, 0x391c0cb3u, 0x4ed8aa4au, 0x5b9cca4fu, 0x682e6ff3u,
+            0x748f82eeu, 0x78a5636fu, 0x84c87814u, 0x8cc70208u, 0x90befffau, 0xa4506cebu, 0xbef9a3f7u, 0xc67178f2u};
+        uint32_t w[64];
+        for (int i = 0; i < 16; i++) w[i] = (uint32_t)p[4 * i] << 24 | (uint32_t)p[4 * i + 1] << 16 | (uint32_t)p[4 * i + 2] << 8 | p[4 * i + 3];
+        for (int i = 16; i < 64; i++) {
+            const uint32_t s0 = rotr(w[i - 15], 7) ^ rotr(w[i - 15], 18) ^ (w[i - 15] >> 3);
+            const uint32_t s1 = rotr(w[i - 2], 17) ^ rotr(w[i - 2], 19) ^ (w[i - 2] >> 10);
+            w[i] = w[i - 16] + s0 + w[i - 7] + s1;
+        }
+        uint32_t a = h[0], b = h[1], c = h[2], d = h[3], e = h[4], f = h[5], g = h[6], hh = h[7];
+        for (int i = 0; i < 64; i++) {
+            const uint32_t t1 = hh + (rotr(e, 6) ^ rotr(e, 11) ^ rotr(e, 25)) + ((e & f) ^ (~e & g)) + K[i] + w[i];
+            const uint32_t t2 = (rotr(a, 2) ^ rotr(a, 13) ^ rotr(a, 22)) + ((a & b) ^ (a & c) ^ (b & c));
+            hh = g; g = f; f = e; e = d + t1; d = c; c = b; b = a; a = t1 + t2;
+        }
+        h[0] += a; h[1] += b; h[2] += c; h[3] += d; h[4] += e; h[5] += f; h[6] += g; h[7] += hh;
+    }
+    void update(const void* data, size_t n) {
+        const uint8_t* p = (const uint8_t*)data;
+        bits += 8ull * n;
+        while (n) {
+            const size_t k = std::min(n, 64 - fill);
+            memcpy(buf + fill, p, k);
+            fill += k;
+            p += k;
+            n -= k;
+            if (fill == 64) {
+                block(buf);
+                fill = 0;
+            }
+        }
+    }
+    void final(uint8_t out[32]) {
+        const uint64_t total = bits;
+        const uint8_t pad = 0x80;
+        update(&pad, 1);
+        const uint8_t zero = 0;
+        while (fill != 56) update(&zero, 1);
+        uint8_t len[8];
+        for (int i = 0; i < 8; i++) len[i] = (uint8_t)(total >> (56 - 8 * i));
+        update(len, 8);
+        for (int i = 0; i < 8; i++)
+            for (int j = 0; j < 4; j++) out[4 * i + j] = (uint8_t)(h[i] >> (24 - 8 * j));
+    }
+};
+
+// c = SHA-256("zkr-phase2-delta" | delta1_old | delta1_new | R) as a little-endian integer mod r
+void challenge(const uint8_t* d1_old, const uint8_t* d1_new, const uint8_t* R, uint8_t c[32]) {
+    static const char kTag[] = "zkr-phase2-delta";
+    Sha256 s;
+    s.update(kTag, sizeof(kTag) - 1);
+    s.update(d1_old, 64);
+    s.update(d1_new, 64);
+    s.update(R, 64);
+    s.final(c);
+    reduce_r(c);
+}
+
+// ---- websnark binary key layout (binarify.ts:152-202): 10 x u32 header, fixed block, then seven sections
+constexpr size_t kPkFixed = 40;                     // alfa1 | beta1 | delta1 | beta2 | delta2
+constexpr size_t kPkDelta1 = kPkFixed + 128, kPkDelta2 = kPkFixed + 320, kPkPols = kPkFixed + 448;
+constexpr size_t kVkDelta1 = 128, kVkDelta2 = 448, kVkIC = 576;
+struct KeyLayout {
+    uint32_t n, l, m, pA, pB, pPA, pPB1, pPB2, pPC, pPH;
+};
+bool key_layout(const void* pk, size_t len, size_t vk_len, KeyLayout* v) {
+    if (len < kPkPols) return false;
+    memcpy(v, pk, 40);
+    const uint64_t n = v->n, l = v->l, m = v->m;
+    return n >= 1 && l + 1 <= n && m >= 2 && (m & (m - 1)) == 0 && v->pA == kPkPols && v->pA <= v->pB && v->pB <= v->pPA &&
+           (uint64_t)v->pPA + 64 * n == v->pPB1 && (uint64_t)v->pPB1 + 64 * n == v->pPB2 &&
+           (uint64_t)v->pPB2 + 128 * n == v->pPC && (uint64_t)v->pPC + 64 * (n - l - 1) == v->pPH &&
+           (uint64_t)v->pPH + 64 * m == len && vk_len == kVkIC + 64 * (l + 1);
+}
+
+// ---- setup_from_powers input checks
+const char* point_problem(int code) {
+    switch (code) {
+        case PT_INFINITY: return "is the point at infinity";
+        case PT_RANGE: return "has a coordinate >= q";
+        default: return "is not on the curve";
+    }
+}
+// count >= need points given, and the first `used` of them (every point the setup reads) valid
+int check_section(const char* name, int group, const void* pts, uint32_t count, uint32_t need, uint32_t used) {
+    if (count < need || !pts) {
+        set_error("zkr_setup_from_powers: %s has %u points, %u needed", name, pts ? count : 0u, need);
+        return ZKR_E_INVALID;
+    }
+    need = used;
+    const size_t sz = group == 1 ? 64 : 128;
+    const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, need / 4096 + 1}));
+    std::vector<uint32_t> bad(nt, need);
+    std::vector<int> code(nt, PT_OK);
+    std::vector<std::thread> th;
+    for (unsigned t = 0; t < nt; t++)
+        th.emplace_back([&, t] {
+            const uint32_t lo = (uint32_t)((uint64_t)need * t / nt), hi = (uint32_t)((uint64_t)need * (t + 1) / nt);
+            for (uint32_t i = lo; i < hi; i++) {
+                const int c = host_point_check(group, (const uint8_t*)pts + sz * i, false);
+                if (c != PT_OK) {
+                    bad[t] = i;
+                    code[t] = c;
+                    return;
+                }
+            }
+        });
+    for (auto& t : th) t.join();
+    for (unsigned t = 0; t < nt; t++)
+        if (bad[t] < need) {
+            set_error("zkr_setup_from_powers: %s[%u] %s", name, bad[t], point_problem(code[t]));
+            return ZKR_E_INVALID;
+        }
+    return ZKR_OK;
+}
+
+// CSC columns of one sum: for column i, entries [ptr[i], ptr[i+1]) of (point index, pool index)
+struct Cols {
+    std::vector<uint32_t> ptr, pidx, cid;
+};
+
+// d_out[i] = sum over column i of pool[cid] * P[pidx], key encoding
+template <class F>
+int combine(zkr_ctx* ctx, cudaStream_t st, const XYZZ<F>* d_pts, const Cols& c, const Fr* d_pool, Affine<F>* d_out) {
+    const uint32_t n = (uint32_t)c.ptr.size() - 1;
+    const uint32_t nnz = c.ptr[n];
+    DevAllocs a;
+    XYZZ<F>* T = nullptr;
+    if (nnz) {
+        uint32_t *d_idx, *d_cid;
+        ZKR_TRY(up32(a, c.pidx.data(), nnz, &d_idx, st));
+        ZKR_TRY(up32(a, c.cid.data(), nnz, &d_cid, st));
+        ZKR_TRY(a.alloc(&T, sizeof(XYZZ<F>) * (size_t)nnz));
+        ZKR_LAUNCH(ctx, k_terms<F>, ceil_div(nnz, 128), 128, 0, st, d_pts, d_idx, d_cid, d_pool, T, nnz);
+        ZKR_CUDA(cudaStreamSynchronize(st));
+        a.release(d_idx);
+        a.release(d_cid);
+    }
+    std::vector<uint32_t> ptr = c.ptr;
+    for (;;) {
+        uint32_t mx = 0;
+        for (uint32_t i = 0; i < n; i++) mx = std::max(mx, ptr[i + 1] - ptr[i]);
+        if (mx <= 1) break;
+        std::vector<uint32_t> start, next(n + 1, 0);
+        for (uint32_t i = 0; i < n; i++) {
+            for (uint32_t s = ptr[i]; s < ptr[i + 1]; s += kSegChunk) start.push_back(s);
+            next[i + 1] = (uint32_t)start.size();
+        }
+        start.push_back(ptr[n]);
+        const uint32_t nch = (uint32_t)start.size() - 1;
+        uint32_t* d_start;
+        XYZZ<F>* U;
+        ZKR_TRY(up32(a, start.data(), start.size(), &d_start, st));
+        ZKR_TRY(a.alloc(&U, sizeof(XYZZ<F>) * (size_t)nch));
+        ZKR_LAUNCH(ctx, k_seg_sum<F>, ceil_div(nch, 128), 128, 0, st, T, d_start, U, nch);
+        ZKR_CUDA(cudaStreamSynchronize(st));
+        a.release(d_start);
+        a.release(T);
+        T = U;
+        ptr.swap(next);
+    }
+    uint32_t* d_ptr;
+    ZKR_TRY(up32(a, ptr.data(), ptr.size(), &d_ptr, st));
+    ZKR_LAUNCH(ctx, k_col_affine<F>, ceil_div(n, 128), 128, 0, st, T, d_ptr, d_out, n);
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    return ZKR_OK;
+}
+
+// Inverse NTT of `blocks` vectors of m points each, in place: natural order in (after k_pntt_load), natural out.
+template <class F>
+int point_intt(zkr_ctx* ctx, cudaStream_t st, XYZZ<F>* X, uint32_t blocks, int log_m, const NttTables* tv) {
+    const uint32_t m = 1u << log_m, nb = blocks * (m / 2);
+    for (int s = 0; s < log_m; s++)
+        ZKR_LAUNCH(ctx, k_pntt_stage<F>, ceil_div(nb, 128), 128, 0, st, X, m, log_m, s, blocks, tv->tw_lo_i, tv->tw_hi_i, tv->lb);
+    ZKR_LAUNCH(ctx, k_pntt_scale<F>, ceil_div((size_t)blocks * m, 128), 128, 0, st, X, (size_t)blocks * m, tv->roots);
+    return ZKR_OK;
+}
+
+template <class F>
+int load_points(zkr_ctx* ctx, cudaStream_t st, const void* h_pts, Affine<F>* d_stage, XYZZ<F>* X, int log_m) {
+    const uint32_t m = 1u << log_m;
+    ZKR_CUDA(cudaMemcpyAsync(d_stage, h_pts, sizeof(Affine<F>) * (size_t)m, cudaMemcpyHostToDevice, st));
+    ZKR_LAUNCH(ctx, k_pntt_load<F>, ceil_div(m, 128), 128, 0, st, d_stage, X, m, log_m);
+    return ZKR_OK;
+}
+
+template <class F>
+int download(cudaStream_t st, void* h, const Affine<F>* d, size_t count) {
+    if (count) ZKR_CUDA(cudaMemcpyAsync(h, d, sizeof(Affine<F>) * count, cudaMemcpyDeviceToHost, st));
+    return ZKR_OK;
+}
+
+int check_r1cs(const zkr_r1cs_csc* r) {
+    const uint32_t n = r->n_vars, m = r->domain_size;
+    if (!r->pool || !r->n_pool) {
+        set_error("zkr_setup_from_powers: empty coefficient pool");
+        return ZKR_E_INVALID;
+    }
+    for (uint32_t i = 0; i < r->n_pool; i++)
+        if (!lt_r((const uint8_t*)r->pool + 32 * (size_t)i)) {
+            set_error("zkr_setup_from_powers: pool[%u] is >= r", i);
+            return ZKR_E_INVALID;
+        }
+    const uint32_t* hp[3][3] = {{r->ptr_a, r->row_a, r->cid_a}, {r->ptr_b, r->row_b, r->cid_b}, {r->ptr_c, r->row_c, r->cid_c}};
+    for (int k = 0; k < 3; k++) {
+        const uint32_t *ptr = hp[k][0], *row = hp[k][1], *cid = hp[k][2];
+        bool ok = ptr && ptr[0] == 0 && (ptr[n] == 0 || (row && cid));
+        for (uint32_t i = 0; ok && i < n; i++) ok = ptr[i] <= ptr[i + 1];
+        for (uint32_t e = 0; ok && e < ptr[n]; e++) ok = row[e] < m && cid[e] < r->n_pool;
+        if (!ok) {
+            set_error("zkr_setup_from_powers: matrix %c: column pointers not monotone, a row >= domain_size or a pool index "
+                      ">= n_pool", "ABC"[k]);
+            return ZKR_E_INVALID;
+        }
+    }
+    return ZKR_OK;
+}
+
+Cols columns(const uint32_t* ptr, const uint32_t* row, const uint32_t* cid, uint32_t n, uint32_t offset) {
+    Cols c;
+    c.ptr.assign(ptr, ptr + n + 1);
+    c.pidx.resize(ptr[n]);
+    for (uint32_t e = 0; e < ptr[n]; e++) c.pidx[e] = row[e] + offset;
+    c.cid.assign(cid, cid + ptr[n]);
+    return c;
+}
+
+}  // namespace
+
+extern "C" int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r, const zkr_powers* pw, void* out_a, void* out_b1,
+                                     void* out_b2, void* out_c, void* out_h, void* out_vk) {
+    if (!ctx || !r || !pw || !out_a || !out_b1 || !out_b2 || !out_c || !out_h || !out_vk) return ZKR_E_INVALID;
+    const uint32_t n = r->n_vars, l = r->n_public, m = r->domain_size;
+    if (n == 0 || l + 1 > n || (m & (m - 1)) || m < 2 || m > (1u << 27) || r->n_constraints + l + 1 > m) {
+        set_error("zkr_setup_from_powers: inconsistent R1CS shape");
+        return ZKR_E_INVALID;
+    }
+    ZKR_TRY(check_r1cs(r));
+    const uint32_t n_tau = std::min(pw->n_tau_g1, 2 * m);      // tau^(2m-1), when given, makes H_(m-1)
+    ZKR_TRY(check_section("tau_g1", 1, pw->tau_g1, pw->n_tau_g1, 2 * m - 1, n_tau));
+    ZKR_TRY(check_section("tau_g2", 2, pw->tau_g2, pw->n_tau_g2, m, m));
+    ZKR_TRY(check_section("alpha_tau_g1", 1, pw->alpha_tau_g1, pw->n_alpha_tau_g1, m, m));
+    ZKR_TRY(check_section("beta_tau_g1", 1, pw->beta_tau_g1, pw->n_beta_tau_g1, m, m));
+    ZKR_TRY(check_section("beta_g2", 2, pw->beta_g2, 1, 1, 1));
+
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = ctx->s[0];
+    int log_m = 0;
+    while ((1u << log_m) < m) log_m++;
+    NttTables* tabs;
+    ZKR_TRY(ntt_get_tables(ctx, log_m, &tabs));
+    const NttTables* tv = tabs;
+
+    // P1 = [L | alpha L | beta L] (G1), P2 = L (G2), XYZZ
+    DevAllocs a;
+    G1Affine *d_tau, *d_stage1, *d_out1, *d_gen1;
+    G2Affine *d_stage2, *d_out2, *d_gen2;
+    G1XYZZ* P1;
+    G2XYZZ* P2;
+    Fr* d_pool;
+    ZKR_TRY(a.alloc(&d_tau, sizeof(G1Affine) * (size_t)n_tau));
+    ZKR_TRY(a.alloc(&d_stage1, sizeof(G1Affine) * (size_t)m));
+    ZKR_TRY(a.alloc(&d_stage2, sizeof(G2Affine) * (size_t)m));
+    ZKR_TRY(a.alloc(&d_out1, sizeof(G1Affine) * (size_t)std::max(n, m)));
+    ZKR_TRY(a.alloc(&d_out2, sizeof(G2Affine) * (size_t)n));
+    ZKR_TRY(a.alloc(&d_gen1, sizeof(G1Affine)));
+    ZKR_TRY(a.alloc(&d_gen2, sizeof(G2Affine)));
+    ZKR_TRY(a.alloc(&P1, sizeof(G1XYZZ) * 3 * (size_t)m));
+    ZKR_TRY(a.alloc(&P2, sizeof(G2XYZZ) * (size_t)m));
+    ZKR_TRY(a.alloc(&d_pool, 32 * (size_t)r->n_pool));
+    ZKR_CUDA(cudaMemcpyAsync(d_pool, r->pool, 32 * (size_t)r->n_pool, cudaMemcpyHostToDevice, st));
+    ZKR_CUDA(cudaMemcpyAsync(d_tau, pw->tau_g1, sizeof(G1Affine) * (size_t)n_tau, cudaMemcpyHostToDevice, st));
+
+    // H straight from the powers
+    ZKR_LAUNCH(ctx, k_h_from_powers, ceil_div(m, 128), 128, 0, st, d_tau, n_tau, d_out1, m);
+    ZKR_TRY(download(st, out_h, d_out1, m));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+
+    // Lagrange bases
+    ZKR_LAUNCH(ctx, k_pntt_load<Fq>, ceil_div(m, 128), 128, 0, st, d_tau, P1, m, log_m);
+    ZKR_TRY(load_points<Fq>(ctx, st, pw->alpha_tau_g1, d_stage1, P1 + m, log_m));
+    ZKR_TRY(load_points<Fq>(ctx, st, pw->beta_tau_g1, d_stage1, P1 + 2 * (size_t)m, log_m));
+    ZKR_TRY(load_points<Fq2>(ctx, st, pw->tau_g2, d_stage2, P2, log_m));
+    ZKR_TRY(point_intt<Fq>(ctx, st, P1, 3, log_m, tv));
+    ZKR_TRY(point_intt<Fq2>(ctx, st, P2, 1, log_m, tv));
+
+    // per-signal sums
+    const Cols ca = columns(r->ptr_a, r->row_a, r->cid_a, n, 0);
+    const Cols cb = columns(r->ptr_b, r->row_b, r->cid_b, n, 0);
+    ZKR_TRY(combine<Fq>(ctx, st, P1, ca, d_pool, d_out1));
+    ZKR_TRY(download(st, out_a, d_out1, n));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    ZKR_TRY(combine<Fq>(ctx, st, P1, cb, d_pool, d_out1));
+    ZKR_TRY(download(st, out_b1, d_out1, n));
+    ZKR_TRY(combine<Fq2>(ctx, st, P2, cb, d_pool, d_out2));
+    ZKR_TRY(download(st, out_b2, d_out2, n));
+    // IC / C: a [beta L] + b [alpha L] + c [L], the three matrices' entries of a column back to back
+    Cols cc;
+    cc.ptr.assign(n + 1, 0);
+    const uint32_t* hp[3][3] = {{r->ptr_a, r->row_a, r->cid_a}, {r->ptr_b, r->row_b, r->cid_b}, {r->ptr_c, r->row_c, r->cid_c}};
+    const uint32_t block[3] = {2 * m, m, 0};
+    for (uint32_t i = 0; i < n; i++) {
+        for (int k = 0; k < 3; k++)
+            for (uint32_t e = hp[k][0][i]; e < hp[k][0][i + 1]; e++) {
+                cc.pidx.push_back(hp[k][1][e] + block[k]);
+                cc.cid.push_back(hp[k][2][e]);
+            }
+        cc.ptr[i + 1] = (uint32_t)cc.pidx.size();
+    }
+    ZKR_TRY(combine<Fq>(ctx, st, P1, cc, d_pool, d_out1));
+    char* vk = (char*)out_vk;
+    ZKR_TRY(download(st, vk + kVkIC, d_out1, l + 1));
+    ZKR_TRY(download(st, out_c, d_out1 + l + 1, n - l - 1));
+    // vk: alfa1 | beta1 | delta1 = G1 | beta2 | gamma2 = G2 | delta2 = G2
+    ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_gen1, d_gen2);
+    ZKR_TRY(download(st, vk + 128, d_gen1, 1));
+    ZKR_TRY(download(st, vk + 320, d_gen2, 1));
+    ZKR_TRY(download(st, vk + 448, d_gen2, 1));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    memcpy(vk, pw->alpha_tau_g1, 64);
+    memcpy(vk + 64, pw->beta_tau_g1, 64);
+    memcpy(vk + 192, pw->beta_g2, 128);
+    return ZKR_OK;
+}
+
+extern "C" int zkr_setup_contribute(zkr_ctx* ctx, const void* pk, size_t pk_len, const void* vk, size_t vk_len,
+                                    const void* delta32, void* out_pk, void* out_vk, void* out_record) {
+    if (!ctx || !pk || !vk || !out_pk || !out_vk || !out_record) return ZKR_E_INVALID;
+    KeyLayout L;
+    if (!key_layout(pk, pk_len, vk_len, &L)) {
+        set_error("zkr_setup_contribute: proving key / vk layout inconsistent (len %zu, vk %zu)", pk_len, vk_len);
+        return ZKR_E_INVALID;
+    }
+    const uint8_t* p = (const uint8_t*)pk;
+    const uint8_t* v = (const uint8_t*)vk;
+    if (memcmp(p + kPkDelta1, v + kVkDelta1, 64) || memcmp(p + kPkDelta2, v + kVkDelta2, 128)) {
+        set_error("zkr_setup_contribute: the key header and the vk disagree on delta");
+        return ZKR_E_INVALID;
+    }
+    if (host_point_check(1, p + kPkDelta1, false) != PT_OK || host_point_check(2, p + kPkDelta2, true) != PT_OK) {
+        set_error("zkr_setup_contribute: delta1 / delta2 is not a valid point");
+        return ZKR_E_INVALID;
+    }
+    if (delta32 && (is_zero32((const uint8_t*)delta32) || !lt_r((const uint8_t*)delta32))) {
+        set_error("zkr_setup_contribute: delta must be in [1, r)");
+        return ZKR_E_INVALID;
+    }
+    // host secrets: delta' then k, both nonzero
+    uint8_t sec[64];
+    int rc = ZKR_OK;
+    if (delta32) memcpy(sec, delta32, 32);
+    else
+        do rc = draw_scalar(sec);
+        while (rc == ZKR_OK && is_zero32(sec));
+    while (rc == ZKR_OK && ((rc = draw_scalar(sec + 32)) == ZKR_OK) && is_zero32(sec + 32)) {}
+    if (rc != ZKR_OK) {
+        wipe(sec, sizeof(sec));
+        return rc;
+    }
+
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = ctx->s[0];
+    const size_t nch = (size_t)(L.n - L.l - 1) + L.m;          // C | H, contiguous
+    Secrets* d_sec = nullptr;
+    G1Affine *d_ch = nullptr, *d_g1 = nullptr;
+    G2Affine* d_g2 = nullptr;
+    uint8_t small[64 * 2 + 128];                               // delta1_new | R | delta2_new
+    auto field = [&](size_t off) { return (char*)d_sec + off; };
+    DevAllocs a;
+    auto run = [&]() -> int {
+        ZKR_TRY(a.alloc(&d_sec, sizeof(Secrets)));
+        ZKR_CUDA(cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st));
+        ZKR_CUDA(cudaMemcpyAsync(d_sec, sec, 64, cudaMemcpyHostToDevice, st));       // delta, k
+        ZKR_TRY(a.alloc(&d_ch, 64 * nch));
+        ZKR_TRY(a.alloc(&d_g1, 128));
+        ZKR_TRY(a.alloc(&d_g2, 128));
+        ZKR_CUDA(cudaMemcpyAsync(d_ch, p + L.pPC, 64 * nch, cudaMemcpyHostToDevice, st));
+        ZKR_CUDA(cudaMemcpyAsync(d_g1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
+        ZKR_CUDA(cudaMemcpyAsync(d_g1 + 1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
+        ZKR_CUDA(cudaMemcpyAsync(d_g2, p + kPkDelta2, 128, cudaMemcpyHostToDevice, st));
+        const int8_t* dig = (const int8_t*)field(offsetof(Secrets, dig));
+        ZKR_LAUNCH(ctx, k_contrib_prep, 1, 1, 0, st, d_sec);
+        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, ceil_div(nch, 128), 128, 0, st, d_ch, nch, dig + kDigits);
+        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, 1, 1, 0, st, d_g1, (size_t)1, dig);
+        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, 1, 1, 0, st, d_g1 + 1, (size_t)1, dig + 2 * kDigits);
+        ZKR_LAUNCH(ctx, k_fixed_mul<Fq2>, 1, 1, 0, st, d_g2, (size_t)1, dig);
+        ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_pk + L.pPC, d_ch, 64 * nch, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaMemcpyAsync(small, d_g1, 128, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaMemcpyAsync(small + 128, d_g2, 128, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaStreamSynchronize(st));
+        uint8_t c[32];
+        challenge(p + kPkDelta1, small, small + 64, c);
+        ZKR_CUDA(cudaMemcpyAsync(field(offsetof(Secrets, c)), c, 32, cudaMemcpyHostToDevice, st));
+        ZKR_LAUNCH(ctx, k_contrib_z, 1, 1, 0, st, d_sec);
+        ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_record + 64, field(offsetof(Secrets, z)), 32, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st));
+        ZKR_CUDA(cudaStreamSynchronize(st));
+        return ZKR_OK;
+    };
+    rc = run();
+    wipe(sec, sizeof(sec));
+    if (d_sec) {            // on an error path too: the secrets never outlive the call
+        cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st);
+        cudaStreamSynchronize(st);
+    }
+    if (rc != ZKR_OK) return rc;
+
+    uint8_t* op = (uint8_t*)out_pk;
+    uint8_t* ov = (uint8_t*)out_vk;
+    memcpy(op, p, L.pPC);
+    memcpy(ov, v, vk_len);
+    memcpy(op + kPkDelta1, small, 64);
+    memcpy(ov + kVkDelta1, small, 64);
+    memcpy(op + kPkDelta2, small + 128, 128);
+    memcpy(ov + kVkDelta2, small + 128, 128);
+    memcpy(out_record, small + 64, 64);
+    return ZKR_OK;
+}
+
+extern "C" int zkr_setup_verify_contribution(zkr_ctx* ctx, const void* old_pk, const void* old_vk, const void* new_pk,
+                                             const void* new_vk, size_t pk_len, size_t vk_len, const void* record,
+                                             int* valid) {
+    if (!ctx || !old_pk || !old_vk || !new_pk || !new_vk || !record || !valid) return ZKR_E_INVALID;
+    *valid = 0;
+    KeyLayout L;
+    if (!key_layout(old_pk, pk_len, vk_len, &L)) {
+        set_error("zkr_setup_verify_contribution: proving key / vk layout inconsistent (len %zu, vk %zu)", pk_len, vk_len);
+        return ZKR_E_INVALID;
+    }
+    const uint8_t *po = (const uint8_t*)old_pk, *pn = (const uint8_t*)new_pk;
+    const uint8_t *vo = (const uint8_t*)old_vk, *vn = (const uint8_t*)new_vk;
+    const uint8_t* R = (const uint8_t*)record;
+    // every byte outside delta1, delta2, C and H
+    const size_t pk_same[3][2] = {{0, kPkDelta1}, {kPkDelta1 + 64, kPkDelta2}, {kPkDelta2 + 128, L.pPC}};
+    const size_t vk_same[3][2] = {{0, kVkDelta1}, {kVkDelta1 + 64, kVkDelta2}, {kVkDelta2 + 128, vk_len}};
+    for (int i = 0; i < 3; i++)
+        if (memcmp(po + pk_same[i][0], pn + pk_same[i][0], pk_same[i][1] - pk_same[i][0]) ||
+            memcmp(vo + vk_same[i][0], vn + vk_same[i][0], vk_same[i][1] - vk_same[i][0]))
+            return ZKR_OK;
+    const uint8_t* keys[2][2] = {{po, vo}, {pn, vn}};
+    for (auto& k : keys) {
+        if (memcmp(k[0] + kPkDelta1, k[1] + kVkDelta1, 64) || memcmp(k[0] + kPkDelta2, k[1] + kVkDelta2, 128)) return ZKR_OK;
+        if (host_point_check(1, k[0] + kPkDelta1, false) != PT_OK || host_point_check(2, k[0] + kPkDelta2, true) != PT_OK)
+            return ZKR_OK;
+    }
+    if (host_point_check(1, R, false) != PT_OK || !lt_r(R + 64)) return ZKR_OK;
+
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = ctx->s[0];
+    // e(delta1_new, G2) = e(G1, delta2_new)
+    uint8_t gen[64 + 128];
+    {
+        DevAllocs a;
+        G1Affine* d_g1;
+        G2Affine* d_g2;
+        ZKR_TRY(a.alloc(&d_g1, 64));
+        ZKR_TRY(a.alloc(&d_g2, 128));
+        ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_g1, d_g2);
+        ZKR_CUDA(cudaMemcpyAsync(gen, d_g1, 64, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaMemcpyAsync(gen + 64, d_g2, 128, cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaStreamSynchronize(st));
+    }
+    {
+        const void* P[2] = {pn + kPkDelta1, gen};
+        const void* Q[2] = {gen + 64, pn + kPkDelta2};
+        const bool neg[2] = {true, false};
+        if (!host_pairing_is_one(P, neg, Q, 2)) return ZKR_OK;
+    }
+    // z delta1_old = R + c delta1_new
+    {
+        uint8_t pts[192], zc[64];
+        memcpy(pts, po + kPkDelta1, 64);
+        memcpy(pts + 64, pn + kPkDelta1, 64);
+        memcpy(pts + 128, R, 64);
+        memcpy(zc, R + 64, 32);
+        challenge(po + kPkDelta1, pn + kPkDelta1, R, zc + 32);
+        G1Affine* d_pts;
+        Fr* d_zc;
+        int* d_ok;
+        int ok = 0;
+        DevAllocs a;
+        ZKR_TRY(a.alloc(&d_pts, 192));
+        ZKR_TRY(a.alloc(&d_zc, 64));
+        ZKR_TRY(a.alloc(&d_ok, sizeof(int)));
+        ZKR_CUDA(cudaMemcpyAsync(d_pts, pts, 192, cudaMemcpyHostToDevice, st));
+        ZKR_CUDA(cudaMemcpyAsync(d_zc, zc, 64, cudaMemcpyHostToDevice, st));
+        ZKR_LAUNCH(ctx, k_schnorr_check, 1, 1, 0, st, d_pts, d_zc, d_ok);
+        ZKR_CUDA(cudaMemcpyAsync(&ok, d_ok, sizeof(int), cudaMemcpyDeviceToHost, st));
+        ZKR_CUDA(cudaStreamSynchronize(st));
+        if (!ok) return ZKR_OK;
+    }
+    // every new C / H point in range and on the curve (the MSM formulas do not see the curve constant), and an
+    // infinity written as an honest contribution writes it, (0, R mod q): R mod q is the generator's x
+    const size_t nch = (size_t)(L.n - L.l - 1) + L.m;
+    {
+        const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, (unsigned)(nch / 4096) + 1}));
+        std::vector<char> good(nt, 1);
+        std::vector<std::thread> th;
+        for (unsigned t = 0; t < nt; t++)
+            th.emplace_back([&, t] {
+                for (size_t i = nch * t / nt; i < nch * (t + 1) / nt; i++) {
+                    const uint8_t* pt = pn + L.pPC + 64 * i;
+                    const int c = host_point_check(1, pt, false);
+                    if (c != PT_OK && (c != PT_INFINITY || memcmp(pt + 32, gen, 32))) {
+                        good[t] = 0;
+                        return;
+                    }
+                }
+            });
+        for (auto& t : th) t.join();
+        for (char ok : good)
+            if (!ok) return ZKR_OK;
+    }
+    // e(X_new, delta2_new) = e(X_old, delta2_old), X = sum rho_i C_i + sum sigma_k H_k, 128-bit rho / sigma
+    std::vector<uint8_t> sc(32 * nch, 0);
+    {
+        std::vector<uint8_t> rnd(16 * nch);
+        ZKR_TRY(os_random(rnd.data(), rnd.size()));
+        for (size_t i = 0; i < nch; i++) memcpy(&sc[32 * i], &rnd[16 * i], 16);
+    }
+    uint8_t X[2][64];
+    const uint8_t* src[2] = {po, pn};
+    for (int s = 0; s < 2; s++) {
+        zkr_bases* b = nullptr;
+        ZKR_TRY(zkr_bases_load(ctx, 1, src[s] + L.pPC, nch, 0, &b));
+        uint8_t xs[64];
+        const int rc = zkr_msm(ctx, b, sc.data(), nch, 0, xs);
+        zkr_bases_free(b);
+        ZKR_TRY(rc);
+        if (!host_g1_std_to_mont(xs, X[s])) {
+            set_error("zkr_setup_verify_contribution: MSM result out of range");
+            return ZKR_E_CUDA;
+        }
+    }
+    const void* P[2] = {X[1], X[0]};
+    const void* Q[2] = {pn + kPkDelta2, po + kPkDelta2};
+    const bool neg[2] = {false, true};
+    *valid = host_pairing_is_one(P, neg, Q, 2) ? 1 : 0;
+    return ZKR_OK;
+}

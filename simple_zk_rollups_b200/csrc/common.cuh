@@ -15,6 +15,11 @@ namespace zkr {
 
 void set_error(const char* fmt, ...);
 int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
+// OS CSPRNG (getrandom), prover.cu: `bytes` random bytes / one scalar uniform in [0, r), 32 B std form
+int os_random(void* out, size_t bytes);
+int draw_scalar(void* out32);
+// the scalar field modulus r, 8 x u32 little-endian (prover.cu)
+extern const uint32_t kRModulus[8];
 
 #define ZKR_CUDA(expr)                                                          \
     do {                                                                        \

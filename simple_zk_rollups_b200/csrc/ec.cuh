@@ -227,6 +227,30 @@ __device__ __noinline__ void xyzz_dbl_mem(XYZZ<F>* dst) {
     *dst = x.dbl();
 }
 
+template <class F>
+__device__ __forceinline__ Affine<F> generator();
+template <>
+__device__ __forceinline__ Affine<Fq> generator<Fq>() {   // (1, 2): TxVerifier.sol:24-26
+    Fq one = Fq::one();
+    return {one, one + one};
+}
+template <>
+__device__ __forceinline__ Affine<Fq2> generator<Fq2>() {   // TxVerifier.sol:30-35 (real part second there)
+    const uint32_t x0[8] = {0xd992f6edu, 0x46debd5cu, 0xf75edaddu, 0x674322d4u, 0x5e5c4479u, 0x426a0066u, 0x121f1e76u, 0x1800deefu};
+    const uint32_t x1[8] = {0xaef312c2u, 0x97e485b7u, 0x35a9e712u, 0xf1aa4933u, 0x31fb5d25u, 0x7260bfb7u, 0x920d483au, 0x198e9393u};
+    const uint32_t y0[8] = {0x66fa7daau, 0x4ce6cc01u, 0x0c43d37bu, 0xe3d1e769u, 0x8dcb408fu, 0x4aab7180u, 0xdb8c6debu, 0x12c85ea5u};
+    const uint32_t y1[8] = {0xd122975bu, 0x55acdadcu, 0x70b38ef3u, 0xbc4b3133u, 0x690c3395u, 0xec9e99adu, 0x585ff075u, 0x090689d0u};
+    Fq a, b, c, d;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        a.v[i] = x0[i];
+        b.v[i] = x1[i];
+        c.v[i] = y0[i];
+        d.v[i] = y1[i];
+    }
+    return {{a.to_mont(), b.to_mont()}, {c.to_mont(), d.to_mont()}};
+}
+
 // k * p, k a 256-bit standard-form integer (LSB-first double-and-add); O(1) uses per proof only.
 template <class F>
 __device__ __forceinline__ XYZZ<F> scalar_mul(XYZZ<F> p, Fr k) {

@@ -674,30 +674,35 @@ static int check_range_flags(zkr_ctx* ctx, const zkr_pkey* pk) {
 // Blinding scalar for a caller that passed NULL: uniform in [0, r) from the OS CSPRNG (getrandom), by rejection on
 // 254-bit draws -- what websnark's groth16GenProof does internally.  The snarkjs debug mode (r = s = 0, deterministic,
 // not zero-knowledge) has to be asked for with explicit zero buffers.
-static int draw_scalar(void* out32) {
-    static const uint32_t kR[8] = {0xf0000001u, 0x43e1f593u, 0x79b97091u, 0x2833e848u,
-                                   0x8181585du, 0xb85045b6u, 0xe131a029u, 0x30644e72u};
+int zkr::os_random(void* out, size_t bytes) {
+    size_t got = 0;
+    while (got < bytes) {
+        ssize_t k = getrandom((char*)out + got, bytes - got, 0);
+        if (k < 0) {
+            set_error("getrandom failed: no entropy source for the random scalars");
+            return ZKR_E_INVALID;
+        }
+        got += (size_t)k;
+    }
+    return ZKR_OK;
+}
+const uint32_t zkr::kRModulus[8] = {0xf0000001u, 0x43e1f593u, 0x79b97091u, 0x2833e848u,
+                                    0x8181585du, 0xb85045b6u, 0xe131a029u, 0x30644e72u};
+int zkr::draw_scalar(void* out32) {
     for (int tries = 0; tries < 256; tries++) {
         uint32_t v[8];
-        size_t got = 0;
-        while (got < sizeof(v)) {
-            ssize_t k = getrandom((char*)v + got, sizeof(v) - got, 0);
-            if (k < 0) {
-                set_error("getrandom failed: no entropy source for the blinding scalars");
-                return ZKR_E_INVALID;
-            }
-            got += (size_t)k;
-        }
+        ZKR_TRY(os_random(v, sizeof(v)));
         v[7] &= 0x3fffffffu;
         bool less = false;
         for (int i = 7; i >= 0; i--) {
-            if (v[i] != kR[i]) {
-                less = v[i] < kR[i];
+            if (v[i] != kRModulus[i]) {
+                less = v[i] < kRModulus[i];
                 break;
             }
         }
         if (less) {
             memcpy(out32, v, 32);
+            explicit_bzero(v, sizeof(v));       // the scalar may be a secret (a phase-2 delta'): no stack copy survives
             return ZKR_OK;
         }
     }

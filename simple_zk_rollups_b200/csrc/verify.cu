@@ -23,6 +23,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "host_ec.cuh"
 #include "keyjson_iface.cuh"
 
 namespace zkr {
@@ -737,6 +738,46 @@ G2A g2_from_mont(const uint8_t* b) {
 }
 
 }  // namespace pr
+
+// ---- host_ec.cuh: byte-level checks and pairings for the setup ceremony (ceremony.cu)
+int host_point_check(int group, const void* mont, bool subgroup) {
+    const uint8_t* b = (const uint8_t*)mont;
+    const int coords = group == 1 ? 2 : 4;
+    bool xz = true;
+    for (int i = 0; i < 16 * coords; i++) xz &= b[i] == 0;
+    if (xz) return PT_INFINITY;
+    for (int i = 0; i < coords; i++) {
+        uint64_t v[4];
+        memcpy(v, b + 32 * i, 32);
+        if (pr::geq_p(v)) return PT_RANGE;
+    }
+    if (group == 1) return pr::on_curve(pr::g1_from_mont(b)) ? PT_OK : PT_OFF_CURVE;
+    const pr::G2A q = pr::g2_from_mont(b);
+    if (!pr::on_curve(q)) return PT_OFF_CURVE;
+    return !subgroup || pr::g2_in_subgroup(q) ? PT_OK : PT_SUBGROUP;
+}
+
+bool host_pairing_is_one(const void* const* g1_mont, const bool* negate, const void* const* g2_mont, int n) {
+    pr::G1A P[8];
+    pr::G2A Q[8];
+    for (int i = 0; i < n; i++) {
+        P[i] = pr::g1_from_mont((const uint8_t*)g1_mont[i]);
+        if (negate[i] && !P[i].inf) P[i].y = pr::neg(P[i].y);
+        Q[i] = pr::g2_from_mont((const uint8_t*)g2_mont[i]);
+    }
+    bool ok = true;
+    const bool one = pr::pairing_product_is_one(P, Q, n, &ok);
+    return ok && one;
+}
+
+bool host_g1_std_to_mont(const void* std64, void* mont64) {
+    pr::G1A p;
+    if (!pr::g1_from_std((const uint8_t*)std64, p)) return false;
+    memcpy(mont64, p.inf ? pr::kZero.v : p.x.v, 32);
+    memcpy((uint8_t*)mont64 + 32, p.inf ? pr::kZero.v : p.y.v, 32);
+    return true;
+}
+
 }  // namespace zkr
 
 using namespace zkr;

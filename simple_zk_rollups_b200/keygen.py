@@ -1,7 +1,9 @@
-"""Synthetic proving / verifying keys for rollup-shaped R1CS, made on the GPU (zkr_synth_setup).
+"""Proving / verifying keys for rollup-shaped R1CS, made on the GPU.
 
-Stands where the reference runs `snarkjs setup --protocol groth` (prover/package.json:34,37); the
-toxic waste is an explicit input, so these are TEST / BENCHMARK keys.  Output is the websnark
+Stands where the reference runs `snarkjs setup --protocol groth` (prover/package.json:34,37).  synth_setup takes the
+toxic waste as an explicit input, so its keys are TEST / BENCHMARK keys.  setup_from_powers builds the key from a
+public powers-of-tau ceremony and contribute() re-randomises delta (phase 2); verify_contribution() checks a
+contribution.  Such a key is sound once at least one contributor erased their delta'.  Output is the websnark
 binary proving key -- byte-identical to binarifyProvingKey(snarkjs pk JSON) for the same
 (R1CS, toxic waste) -- plus the verifying key as Python ints (and as the binary block zkr_vkey_load_bin takes, vk["bin"]).
 """
@@ -45,10 +47,8 @@ def _g2(buf):
     return None if v[0] == 0 and v[1] == 0 else ((v[0], v[1]), (v[2], v[3]))
 
 
-def synth_setup(ctx, r1cs, toxic):
-    """r1cs: simple_zk_rollups_b200.synth.R1CS; toxic = (tau, alpha, beta, gamma, delta) ints.
-    -> (pk_bin: np.ndarray[uint8], vk: dict of int points)."""
-    L = _lib.lib()
+def _r1cs_desc(r1cs):
+    """(zkr_r1cs_csc, csc dict, arrays to keep alive) for r1cs with the input-consistency rows in polsA."""
     n, l = r1cs.nVars, r1cs.nPublic
     bits, m = r1cs.domain()
     csc = r1cs.csc(with_inputs=True)
@@ -63,16 +63,31 @@ def synth_setup(ctx, r1cs, toxic):
         setattr(desc, "row_" + k, row.ctypes.data)
         setattr(desc, "cid_" + k, cid.ctypes.data)
     pool = np.frombuffer(b"".join(int(c).to_bytes(32, "little") for c in r1cs.pool), dtype=np.uint8).copy()
+    keep.append(pool)
     desc.pool = pool.ctypes.data
-    tox = np.frombuffer(b"".join(int(t % R).to_bytes(32, "little") for t in toxic), dtype=np.uint8).copy()
-    out_a = np.empty(64 * n, dtype=np.uint8)
-    out_b1 = np.empty(64 * n, dtype=np.uint8)
-    out_b2 = np.empty(128 * n, dtype=np.uint8)
-    out_c = np.empty(64 * (n - l - 1), dtype=np.uint8)
-    out_h = np.empty(64 * m, dtype=np.uint8)
-    out_vk = np.empty(192 + 384 + 64 * (l + 1), dtype=np.uint8)
-    _lib.check(L.zkr_synth_setup(ctx, C.byref(desc), _lib.buf_ptr(tox), *[_lib.buf_ptr(x) for x in
-                                 (out_a, out_b1, out_b2, out_c, out_h, out_vk)]))
+    return desc, csc, keep
+
+
+def _outputs(n, l, m):
+    """out_a, out_b1, out_b2, out_c, out_h, out_vk host buffers (zkr.h zkr_synth_setup)."""
+    return (np.empty(64 * n, dtype=np.uint8), np.empty(64 * n, dtype=np.uint8), np.empty(128 * n, dtype=np.uint8),
+            np.empty(64 * (n - l - 1), dtype=np.uint8), np.empty(64 * m, dtype=np.uint8),
+            np.empty(192 + 384 + 64 * (l + 1), dtype=np.uint8))
+
+
+def vk_dict(vkb, n_public):
+    """The verifying key as Python ints from its binary block (alfa1|beta1|delta1|beta2|gamma2|delta2|IC, Fq-M)."""
+    vkb = bytes(vkb)
+    return dict(protocol="groth", nPublic=n_public, vk_alfa_1=_g1(vkb[0:64]), vk_beta_2=_g2(vkb[192:320]),
+                vk_gamma_2=_g2(vkb[320:448]), vk_delta_2=_g2(vkb[448:576]),
+                IC=[_g1(vkb[576 + 64 * i:640 + 64 * i]) for i in range(n_public + 1)],
+                bin=vkb)                 # the block zkr_vkey_load_bin takes
+
+
+def _assemble(r1cs, csc, out_a, out_b1, out_b2, out_c, out_h, out_vk):
+    """websnark binary proving key (binarify.ts:152-202) around the point sections, and the vk dict."""
+    n, l = r1cs.nVars, r1cs.nPublic
+    bits, m = r1cs.domain()
     pool_mont = np.frombuffer(b"".join(((int(c) << 256) % R).to_bytes(32, "little") for c in r1cs.pool),
                               dtype=np.uint32).reshape(-1, 8)
     secA = _pols_section(*[_u32(x) for x in csc["A"]], pool_mont, n)
@@ -89,8 +104,78 @@ def synth_setup(ctx, r1cs, toxic):
     pk_bin = np.concatenate([np.frombuffer(head + fixed, dtype=np.uint8), secA, secB, out_a, out_b1, out_b2,
                              out_c, out_h])
     assert pk_bin.size == off
-    vk = dict(protocol="groth", nPublic=l, vk_alfa_1=_g1(vkb[0:64]), vk_beta_2=_g2(vkb[192:320]),
-              vk_gamma_2=_g2(vkb[320:448]), vk_delta_2=_g2(vkb[448:576]),
-              IC=[_g1(vkb[576 + 64 * i:640 + 64 * i]) for i in range(l + 1)],
-              bin=vkb)                 # the block zkr_vkey_load_bin takes
-    return pk_bin, vk
+    return pk_bin, vk_dict(vkb, l)
+
+
+def synth_setup(ctx, r1cs, toxic):
+    """r1cs: simple_zk_rollups_b200.synth.R1CS; toxic = (tau, alpha, beta, gamma, delta) ints.
+    -> (pk_bin: np.ndarray[uint8], vk: dict of int points)."""
+    L = _lib.lib()
+    desc, csc, keep = _r1cs_desc(r1cs)
+    outs = _outputs(r1cs.nVars, r1cs.nPublic, r1cs.domain()[1])
+    tox = np.frombuffer(b"".join(int(t % R).to_bytes(32, "little") for t in toxic), dtype=np.uint8).copy()
+    _lib.check(L.zkr_synth_setup(ctx, C.byref(desc), _lib.buf_ptr(tox), *[_lib.buf_ptr(x) for x in outs]))
+    return _assemble(r1cs, csc, *outs)
+
+
+_POWER_SECTIONS = (("tau_g1", 64), ("tau_g2", 128), ("alpha_tau_g1", 64), ("beta_tau_g1", 64))
+
+
+def setup_from_powers(ctx, r1cs, powers):
+    """Circuit key from phase-1 powers of tau (zkr_setup_from_powers; zkr.h has the math and the security statement).
+    powers: dict of byte buffers (bytes / uint8 arrays) of affine Fq-M points in the key encoding: "tau_g1"
+    (>= 2m - 1 points, 2m for H_(m-1)), "tau_g2", "alpha_tau_g1", "beta_tau_g1" (>= m each) and "beta_g2" (one point).
+    -> (pk_bin, vk) as synth_setup, for gamma = delta = 1: NOT deployable before one contribute()."""
+    L = _lib.lib()
+    desc, csc, keep = _r1cs_desc(r1cs)
+    pw = _lib.Powers()
+    for name, size in _POWER_SECTIONS + (("beta_g2", 128),):
+        buf = np.frombuffer(bytes(powers[name]), dtype=np.uint8)
+        if buf.size % size:
+            raise ValueError("%s: %d bytes is not a whole number of %d-byte points" % (name, buf.size, size))
+        keep.append(buf)
+        setattr(pw, name, buf.ctypes.data if buf.size else None)
+        if name != "beta_g2":
+            setattr(pw, "n_" + name, min(buf.size // size, 0xFFFFFFFF))
+        elif buf.size != 128:
+            raise ValueError("beta_g2 must be one 128-byte G2 point")
+    outs = _outputs(r1cs.nVars, r1cs.nPublic, r1cs.domain()[1])
+    _lib.check(L.zkr_setup_from_powers(ctx, C.byref(desc), C.byref(pw), *[_lib.buf_ptr(x) for x in outs]))
+    return _assemble(r1cs, csc, *outs)
+
+
+def _vk_bin(vk):
+    return np.frombuffer(bytes(vk["bin"] if isinstance(vk, dict) else vk), dtype=np.uint8)
+
+
+def contribute(ctx, pk_bin, vk, delta=None):
+    """One phase-2 contribution (zkr_setup_contribute): delta1, delta2 times delta', C and H times 1/delta'.
+    delta: int in [1, r) (tests, reproducible keys) or None = drawn from the OS CSPRNG and never seen by Python.
+    -> (new pk_bin, new vk dict, 96-byte record R | z proving knowledge of delta')."""
+    L = _lib.lib()
+    pk = np.ascontiguousarray(pk_bin, dtype=np.uint8)
+    vkb = _vk_bin(vk)
+    out_pk = np.empty_like(pk)
+    out_vk = np.empty_like(vkb)
+    rec = np.empty(_lib.CONTRIB_RECORD_BYTES, dtype=np.uint8)
+    d = None if delta is None else int(delta).to_bytes(32, "little")
+    _lib.check(L.zkr_setup_contribute(ctx, _lib.buf_ptr(pk), pk.size, _lib.buf_ptr(vkb), vkb.size, _lib.buf_ptr(d),
+                                      _lib.buf_ptr(out_pk), _lib.buf_ptr(out_vk), _lib.buf_ptr(rec)))
+    n_public = struct.unpack_from("<I", pk[:8].tobytes(), 4)[0]
+    return out_pk, vk_dict(out_vk, n_public), rec.tobytes()
+
+
+def verify_contribution(ctx, old_pk, old_vk, new_pk, new_vk, record):
+    """True iff (new_pk, new_vk) is (old_pk, old_vk) after the contribution `record` proves (zkr.h lists the checks)."""
+    L = _lib.lib()
+    po = np.ascontiguousarray(old_pk, dtype=np.uint8)
+    pn = np.ascontiguousarray(new_pk, dtype=np.uint8)
+    vo, vn = _vk_bin(old_vk), _vk_bin(new_vk)
+    rec = bytes(record)
+    if pn.size != po.size or vn.size != vo.size or len(rec) != _lib.CONTRIB_RECORD_BYTES:
+        raise ValueError("old and new keys differ in size, or the record is not %d bytes" % _lib.CONTRIB_RECORD_BYTES)
+    valid = C.c_int(0)
+    _lib.check(L.zkr_setup_verify_contribution(ctx, _lib.buf_ptr(po), _lib.buf_ptr(vo), _lib.buf_ptr(pn),
+                                               _lib.buf_ptr(vn), po.size, vo.size, _lib.buf_ptr(rec),
+                                               C.byref(valid)))
+    return bool(valid.value)
