@@ -49,7 +49,7 @@ struct DevBuf {
     size_t cap = 0;
 };
 
-constexpr int kNumStreams = 7;      // s[0..4]: the proof's five chains, s[5]: the hExps MSM (ZKR_H_SPLIT), s[6]: witness uploads
+constexpr int kNumStreams = 6;      // s[0..4]: the proof's five chains, s[5]: witness uploads
 
 // Per-kernel device timing for bench.py's roofline: rings of CUDA event pairs recorded on the
 // launching stream around selected kernels while profiling is enabled.

@@ -1,9 +1,6 @@
 // libzkr context / error plumbing (C-ABI: zkr_ctx_*, zkr_strerror, zkr_last_error, zkr_version).
 // zkr_ctx_create stands where the reference calls buildBn128()
 // (/root/reference/operator/src/snarks/common.ts:23) -- but it is created once, not per proof.
-#include <cstdlib>
-#include <cstring>
-
 #include "common.cuh"
 
 namespace zkr {
@@ -75,26 +72,15 @@ extern "C" int zkr_ctx_create(int device, zkr_ctx** out) {
     zkr_ctx* c = new zkr_ctx();
     c->device = device;
     c->sm_count = prop.multiProcessorCount;
+    // Equal (default) stream priorities on purpose.  Round 1 (profiles/r01_sched_sweep.json, 2^20, real blinding
+    // scalars): nine priority assignments over the five chains land within 17.12 .. 17.63 ms of the 17.22 ms of equal
+    // priorities (H + A + B1 high: 18.3 ms); two and three proofs in flight per GPU gain 3 % in proofs/s
+    // (profiles/r01_pipeline_check.json).  Round 2 (profiles/r02_schedule_ab.json, r02_priority_hsplit_ab.json): no
+    // assignment is faster with two proofs in flight, as the throughput API runs.  The GPU is saturated by the proof's
+    // bulk kernels; ordering them does not change the total.  (A first sweep with r = s = 0 favoured "B2 highest": with
+    // zero scalars the two blinding multiplications are free, which hides that they then end up on the critical path.)
     for (int i = 0; i < kNumStreams; i++) {
-        // Equal stream priorities on purpose.  tools/prio_sweep.py (profiles/r01_sched_sweep.json, 2^20, real blinding
-        // scalars): nine priority assignments over the five chains land within 17.12 .. 17.63 ms of the 17.22 ms of
-        // equal priorities (H + A + B1 high: 18.3 ms); two and three proofs in flight per GPU gain 3 % in proofs/s
-        // (profiles/r01_pipeline_check.json).  The GPU is saturated by the proof's bulk kernels; ordering them does
-        // not change the total.  (A first sweep with r = s = 0 favoured "B2 highest": with zero scalars the two
-        // blinding multiplications are free, which hides that they then end up on the critical path.)
-        // s[0] = H chain, s[1] = A, s[2] = B1, s[3] = B2, s[4] = C, s[5] = the hExps MSM when ZKR_H_SPLIT=1.  ZKR_STREAM_PRIO="p0,p1,..." overrides (0 =
-        // default, negative = higher).
-        static const int kDefaultPrio[kNumStreams] = {0, 0, 0, 0, 0, 0, 0};
-        int prio = kDefaultPrio[i];
-        if (const char* e = getenv("ZKR_STREAM_PRIO")) {
-            const char* q = e;
-            for (int k = 0; k < i && q; k++) {
-                q = strchr(q, ',');
-                if (q) q++;
-            }
-            if (q) prio = atoi(q);
-        }
-        ZKR_CUDA(cudaStreamCreateWithPriority(&c->s[i], cudaStreamNonBlocking, prio));
+        ZKR_CUDA(cudaStreamCreateWithFlags(&c->s[i], cudaStreamNonBlocking));
         ZKR_CUDA(cudaEventCreateWithFlags(&c->ev_join[i], cudaEventDisableTiming));
     }
     ZKR_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));

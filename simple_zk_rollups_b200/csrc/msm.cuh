@@ -42,11 +42,7 @@ constexpr int kLazyDefault = 7;
 constexpr int kLevelLog = 4;          // boundary levels: 16 entries per thread ...
 constexpr int kLevelLogBig = 2;       // ... except while the list is long: 4 per thread keeps ~4x more warps in flight
 constexpr size_t kLevelBigMin = 1u << 16;
-inline int level_log(size_t cnt) {
-    const int forced = getenv("ZKR_LEVEL_LOG_BIG") ? atoi(getenv("ZKR_LEVEL_LOG_BIG")) : 0;   // experiment knob
-    const int big = forced >= 2 && forced <= kLevelLog ? forced : kLevelLogBig;   // 1 would never shrink the list (2 in, 2 out)
-    return cnt >= kLevelBigMin ? big : kLevelLog;
-}
+inline int level_log(size_t cnt) { return cnt >= kLevelBigMin ? kLevelLogBig : kLevelLog; }
 constexpr uint32_t kNegBit = 0x80000000u;
 // Zero digits carry the sentinel key 2^(c-1): they sort behind every bucket and the accumulation kernel never visits
 // them.  Folding them into the buckets as "skip" entries saves a key bit (two radix passes instead of three at c = 17)
@@ -66,7 +62,7 @@ struct MsmPlan {
             if (cost < best_cost) { best_cost = cost; best = c; }
         }
         if (c_forced <= 0)
-            if (const char* e = getenv("ZKR_MSM_C")) c_forced = atoi(e);      // experiment knob (tools/prio_sweep.py)
+            if (const char* e = getenv("ZKR_MSM_C")) c_forced = atoi(e);      // A/B knob (profiles/r02_window_sweep.json)
         if (c_forced > 0 && (uint64_t)((255 + c_forced - 1) / c_forced) * n >= (1ull << 31)) c_forced = 0;
         p.c = c_forced > 0 ? c_forced : best;
         p.W = (255 + p.c - 1) / p.c;
@@ -594,12 +590,9 @@ struct MsmWork {                      // per-bases device work buffers
 //                 scalars, same compaction map, same window plan: pi_b's B2' for B1') produced in this proof; the
 //                 caller has made `st` wait for that set's ev_sorted.
 //   ev_sorted   : recorded on st once the sorted pairs are final.
-//   ev_accum    : recorded on st after the level-1 accumulation (the bulk of the MSM) has been queued.
-//   wait_accum  : st waits for this event right before the level-1 accumulation is queued (digit extraction and the
-//                 sort, small kernels, may run ahead of it).
 struct MsmHooks {
     const zkr_bases* sorted_from = nullptr;
-    cudaEvent_t ev_sorted = nullptr, ev_accum = nullptr, wait_accum = nullptr;
+    cudaEvent_t ev_sorted = nullptr;
 };
 
 }  // namespace zkr
@@ -780,7 +773,6 @@ int msm_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* d
     const size_t smem = (size_t)(kAccumThreads / 32) * 2 * 32 * (L + 1) * 4;
     XYZZ<F>* buckets = (XYZZ<F>*)wk.buckets;
     const int pslot = ctx->prof_begin(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, st, (double)total);
-    if (hooks && hooks->wait_accum) ZKR_CUDA(cudaStreamWaitEvent(st, hooks->wait_accum, 0));
     // Boundary partials -> buckets: the one-launch gather up to 20-bit windows (every proof size), the round-1 recursive
     // levels above: at 22-bit windows the 12-bit top window puts n / 4096 extra entries into each of the 4096 lowest buckets,
     // i.e. thousands of moderately heavy buckets, which the whole-CTA heavy path handles badly (2^24: 48 vs 40.6 ms,
@@ -805,7 +797,6 @@ int msm_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* d
     else lrc = launch(k_accum_affine<F, kPrefetch, 0>);
     if (lrc != ZKR_OK) return lrc;
     ctx->prof_end(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, pslot, st);
-    if (hooks && hooks->ev_accum) ZKR_CUDA(cudaEventRecord(hooks->ev_accum, st));
     if (!use_levels) {
         ZKR_LAUNCH(ctx, k_bucket_gather<F>, kHeavyBlocks + ceil_div(nb, kGatherThreads), kGatherThreads, XB * kGatherThreads,
                    st, skeys, total, b->logL, wk.run_lo, (const XYZZ<F>*)wk.bnd[0], buckets, nb);

@@ -15,12 +15,10 @@ int bases_build_g2(zkr_ctx* ctx, zkr_bases* b, const char* p, size_t n, int c, c
     return bases_build<Fq2>(ctx, b, p, n, c, st, sidx);
 }
 int msm_run_g2(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* sc, void* out, const zkr_bases* sorted_from,
-               cudaEvent_t ev_sorted, cudaEvent_t ev_accum, cudaEvent_t wait_accum) {
+               cudaEvent_t ev_sorted) {
     MsmHooks h;
     h.sorted_from = sorted_from;
     h.ev_sorted = ev_sorted;
-    h.ev_accum = ev_accum;
-    h.wait_accum = wait_accum;
     return msm_run<Fq2>(ctx, st, b, sc, (XYZZ<Fq2>*)out, &h);
 }
 }  // namespace zkr

@@ -16,14 +16,11 @@ int bases_build_g2(zkr_ctx*, zkr_bases*, const char* h_points, size_t n, int c_f
 // d_out: XYZZ point (128 B for G1, 256 B for G2), Montgomery
 // Optional hooks (prover.cu): sorted_from = another base set whose sorted (bucket, point) pairs of THIS proof are
 // consumed instead of extracting digits and sorting again (bases_share_sort must hold, and the stream must already
-// wait for that set's ev_sorted); ev_sorted / ev_accum are recorded on the stream after the sort / after the
-// level-1 accumulation has been queued; the stream waits for wait_accum right before its level-1 accumulation.
+// wait for that set's ev_sorted); ev_sorted is recorded on the stream once the sorted pairs are final.
 int msm_run_g1(zkr_ctx*, cudaStream_t, const zkr_bases*, const uint32_t* d_scalars, void* d_out,
-               const zkr_bases* sorted_from = nullptr, cudaEvent_t ev_sorted = nullptr, cudaEvent_t ev_accum = nullptr,
-               cudaEvent_t wait_accum = nullptr);
+               const zkr_bases* sorted_from = nullptr, cudaEvent_t ev_sorted = nullptr);
 int msm_run_g2(zkr_ctx*, cudaStream_t, const zkr_bases*, const uint32_t* d_scalars, void* d_out,
-               const zkr_bases* sorted_from = nullptr, cudaEvent_t ev_sorted = nullptr, cudaEvent_t ev_accum = nullptr,
-               cudaEvent_t wait_accum = nullptr);
+               const zkr_bases* sorted_from = nullptr, cudaEvent_t ev_sorted = nullptr);
 // same scalars, same compaction map, same window plan: one radix sort can serve both (B1' and B2' of a key)
 bool bases_share_sort(const zkr_bases* a, const zkr_bases* b);
 int g1_result_to_affine_std(zkr_ctx*, cudaStream_t, const void* d_xyzz, void* d_out64);

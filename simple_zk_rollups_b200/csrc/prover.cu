@@ -53,7 +53,7 @@ struct zkr_pkey {
     // B1' and B2' take the same scalars through the same compaction map and window plan (B1_i is the point at infinity
     // exactly when B2_i is): one digit extraction + radix sort, done on pi_b's stream, serves both MSMs
     bool share_b_sort = false;
-    cudaEvent_t ev_b2_sorted = nullptr, ev_b2_accum = nullptr;
+    cudaEvent_t ev_b2_sorted = nullptr;
     size_t bytes = 0;
 };
 
@@ -156,31 +156,31 @@ __global__ void __launch_bounds__(32 * kBlindWarps) k_blind_muls(char* res, cons
 constexpr size_t kBlindSmem = sizeof(G1XYZZ) * (256 + kBlindWarps);
 
 // block 0: pi_a, block 1: pi_b, block 2: pi_c = C + H + T1 + T2; affine, standard form
-// Three single-thread blocks, nothing left to overlap them: the inversion is the whole kernel.  fermat == 0 (default)
-// uses the binary extended Euclid of fp_inv.cuh, fermat != 0 the a^(p-2) ladder (ZKR_FINISH_FERMAT=1, for A/B timing).
-__global__ void k_finish(const char* res, char* proof, int fermat) {
+// Three single-thread blocks, nothing left to overlap them: the inversion is the whole kernel, so it is the binary
+// extended Euclid of fp_inv.cuh (faster than the a^(p-2) ladder here: profiles/r01_small_circuits_finish_ab.json).
+__global__ void k_finish(const char* res, char* proof) {
     if (blockIdx.x == 0) {
         const G1XYZZ p = G1XYZZ::load(res + R_A);
-        G1Affine a = fermat ? p.to_affine() : p.to_affine_vartime();
+        G1Affine a = p.to_affine_vartime();
         a.x.from_mont().store(proof);
         a.y.from_mont().store(proof + 32);
     } else if (blockIdx.x == 1) {
         const G2XYZZ p = G2XYZZ::load(res + R_B2);
-        G2Affine a = fermat ? p.to_affine() : p.to_affine_vartime();
+        G2Affine a = p.to_affine_vartime();
         a.x.from_mont().store(proof + 64);
         a.y.from_mont().store(proof + 128);
     } else {
         G1XYZZ c = G1XYZZ::load(res + R_C);
 #pragma unroll 1
         for (int i = 0; i < 3; i++) c.add(G1XYZZ::load(res + (i == 0 ? R_H : (i == 1 ? R_T1 : R_T2))));
-        G1Affine a = fermat ? c.to_affine() : c.to_affine_vartime();
+        G1Affine a = c.to_affine_vartime();
         a.x.from_mont().store(proof + 192);
         a.y.from_mont().store(proof + 224);
     }
 }
 
-// sharded prove: res[e] = sum over ranks of the gathered partial results (block e: B2 in G2; A, B1, C, H and, when
-// every rank blinded its own partials, T1, T2 in G1)
+// sharded prove: res[e] = sum over ranks of the gathered partial results (block e: B2 in G2; A, B1, C, H, T1, T2 in
+// G1; every rank blinds its own partials, so the blinding terms are partial sums too)
 __global__ void k_sum_res(const char* slots, int world, char* res) {
     const int offs[7] = {R_B2, R_A, R_B1, R_C, R_H, R_T1, R_T2};
     const int off = offs[blockIdx.x];
@@ -267,7 +267,6 @@ void pkey_release(zkr_pkey* pk) {
     for (auto& e : pk->ev)
         if (e) cudaEventDestroy(e);
     if (pk->ev_b2_sorted) cudaEventDestroy(pk->ev_b2_sorted);
-    if (pk->ev_b2_accum) cudaEventDestroy(pk->ev_b2_accum);
     zkr_bases* bs[] = {pk->A, pk->B1, pk->B2, pk->C, pk->H};
     for (zkr_bases* b : bs) bases_release(b);
     delete pk;
@@ -291,8 +290,7 @@ static void shard_range(uint64_t total, int rank, int world, uint64_t* lo, uint6
 //     H-group rank:  P + MH / g_h + x W        other rank:  y W         g_h x + (world - g_h) y = 1
 // in units of one G1 point of a 2^20 MSM (P = H pipeline, MH = m, W = n (2 + 2.4) + nc; a G2 point costs 2.4 G1
 // points, the H pipeline 0.85 m: profiles/r02_launch_shares.md).  ZKR_SHARD_TASKS=0 restores the uniform split with
-// the H pipeline on every rank; ZKR_SHARD_GH / ZKR_SHARD_X override g_h / x (tools/gpu_jobs/r02_sharded_tasks.sh).
-// Every rank of a job must see the same values.
+// the H pipeline on every rank; every rank of a job must see the same value.
 struct ShardPlan {
     int g_h = 1;
     double x = 1, y = 1;
@@ -306,11 +304,9 @@ static ShardPlan shard_plan(int world, uint64_t n, uint64_t nc, uint64_t m) {
     if (world == 1 || (e && atoi(e) == 0)) return p;
     p.uniform = false;
     p.g_h = world <= 2 ? 1 : world / 2;
-    if ((e = getenv("ZKR_SHARD_GH")) && atoi(e) >= 1 && atoi(e) < world) p.g_h = atoi(e);
     const double P = 0.85 * (double)m, MH = (double)m, W = (double)n * 4.4 + (double)nc;
     const double T = (p.g_h * P + MH + W) / world;
     p.x = (T - P - MH / p.g_h) / W;
-    if ((e = getenv("ZKR_SHARD_X"))) p.x = atof(e);
     if (p.x < 0.06) p.x = 0;                       // not worth four more latency chains beside the H chain
     if (p.x * p.g_h > 1) p.x = 1.0 / p.g_h;
     p.y = (1.0 - p.g_h * p.x) / (world - p.g_h);
@@ -474,11 +470,7 @@ static int pkey_load(zkr_ctx* ctx, const void* vbuf, size_t len, int rank, int w
     cudaMemsetAsync(pk->err, 0, sizeof(int), st);
     for (auto& e : pk->ev) cudaEventCreate(&e);
     cudaEventCreateWithFlags(&pk->ev_b2_sorted, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&pk->ev_b2_accum, cudaEventDisableTiming);
-    {
-        const char* e = getenv("ZKR_SHARE_SORT");       // A/B knob; default on
-        pk->share_b_sort = bases_share_sort(pk->B1, pk->B2) && !(e && atoi(e) == 0);
-    }
+    pk->share_b_sort = bases_share_sort(pk->B1, pk->B2);
     NttTables* t;
     PK_TRY(ntt_get_tables(ctx, pk->log_m, &t));
     zkr_bases* bs[] = {pk->A, pk->B1, pk->B2, pk->C, pk->H};
@@ -540,114 +532,60 @@ static int prove_enqueue(zkr_ctx* ctx, const zkr_pkey* pk, char* d_proof, bool t
     ZKR_LAUNCH(ctx, k_prep_scalars, 1, 1, 0, us, wext, n, (const Fr*)pk->rs_dev, pk->err);
     ZKR_LAUNCH(ctx, k_witness_range, ceil_div(n, 256), 256, 0, us, wext, n, pk->err);
     const bool par = !ctx->serial;
-    // ZKR_H_SPLIT=1 (experiment knob): the hExps MSM runs on its own stream (s[5]) behind the NTT pipeline (s[0]), so the
-    // two parts of the H chain can be given different stream priorities (ZKR_STREAM_PRIO)
-    static const bool h_split = getenv("ZKR_H_SPLIT") && atoi(getenv("ZKR_H_SPLIT")) != 0;
-    const int n_fork = (par && h_split) ? 6 : 5;
-    if (par) ZKR_TRY(ctx->fork(n_fork));
+    // one stream per chain: s[0] = H, s[1] = A, s[2] = B1, s[3] = B2, s[4] = C
+    if (par) ZKR_TRY(ctx->fork(5));
     cudaStream_t sH = par ? ctx->s[0] : us, sA = par ? ctx->s[1] : us, sB1 = par ? ctx->s[2] : us,
                  sB2 = par ? ctx->s[3] : us, sC = par ? ctx->s[4] : us;
     const uint32_t* w = (const uint32_t*)wext;
-    // experiment knob (tools/prio_sweep.py): ZKR_H_FIRST=1 runs sparse LC + the NTT pipeline before any MSM starts
-    const bool h_first = getenv("ZKR_H_FIRST") && atoi(getenv("ZKR_H_FIRST")) != 0;
-    const bool has_h = pk->h_count != 0;   // false: a rank outside the H group of a sharded proof (shard_plan)
-    auto h_front = [&]() -> int {
-        if (timed) cudaEventRecord(ev[0], sH);
-        if (!has_h) {
-            if (timed) cudaEventRecord(ev[1], sH);
-            if (timed) cudaEventRecord(ev[2], sH);
-            return ZKR_OK;
-        }
+    // heaviest first: the G2 MSM costs ~3 G1 MSMs
+    if (timed) cudaEventRecord(ev[6], sB2);
+    ZKR_TRY(msm_run_g2(ctx, sB2, pk->B2, w, pk->res + R_B2, nullptr, pk->ev_b2_sorted));
+    if (timed) cudaEventRecord(ev[7], sB2);
+    // H chain: sparse LC, H pipeline, hExps MSM
+    if (timed) cudaEventRecord(ev[0], sH);
+    if (pk->h_count != 0) {
         ZKR_LAUNCH(ctx, k_sparse_lc, dim3(ceil_div(m, 128), 2), 128, 0, sH, pk->a_ptr, pk->a_sig, pk->a_coef, pk->b_ptr,
                    pk->b_sig, pk->b_coef, wext, pk->at, pk->bt, m);
         if (timed) cudaEventRecord(ev[1], sH);
         ZKR_TRY(h_pipeline(ctx, sH, pk->at, pk->bt, pk->st, pk->h, pk->log_m, true));
         if (timed) cudaEventRecord(ev[2], sH);
-        return ZKR_OK;
-    };
-    if (h_first && par) {
-        ZKR_TRY(h_front());
-        ZKR_CUDA(cudaEventRecord(ctx->ev_join[0], sH));
-        cudaStream_t others[4] = {sA, sB1, sB2, sC};
-        for (cudaStream_t o : others) ZKR_CUDA(cudaStreamWaitEvent(o, ctx->ev_join[0], 0));
+        ZKR_TRY(msm_run_g1(ctx, sH, pk->H, (const uint32_t*)(pk->h + pk->h_lo), pk->res + R_H));
+    } else {   // a rank outside the H group of a sharded proof (shard_plan)
+        if (timed) cudaEventRecord(ev[1], sH);
+        if (timed) cudaEventRecord(ev[2], sH);
+        ZKR_CUDA(cudaMemsetAsync(pk->res + R_H, 0, 128, sH));   // the identity (ZZ = 0)
     }
-    // heaviest first: the G2 MSM costs ~3 G1 MSMs
-    // ZKR_DELAY (experiment knob): chains named in it (A, B = B1', C, H = the hExps MSM) start their MSM only once the
-    // G2 accumulation kernel is done, so that their bulk overlaps the G2 chain's latency-bound tail.  Lower case
-    // (a, b, c, h): only the chain's level-1 accumulation waits; its digit extraction and sort run ahead.
-    static const char* delay = getenv("ZKR_DELAY") ? getenv("ZKR_DELAY") : "";
-    auto delayed = [&](char who, cudaStream_t s) -> int {
-        if (par && strchr(delay, who)) ZKR_CUDA(cudaStreamWaitEvent(s, pk->ev_b2_accum, 0));
-        return ZKR_OK;
-    };
-    auto late = [&](char who) -> cudaEvent_t { return (par && strchr(delay, who)) ? pk->ev_b2_accum : nullptr; };
-    if (timed) cudaEventRecord(ev[6], sB2);
-    ZKR_TRY(msm_run_g2(ctx, sB2, pk->B2, w, pk->res + R_B2, nullptr, pk->ev_b2_sorted, pk->ev_b2_accum));
-    if (timed) cudaEventRecord(ev[7], sB2);
-    // H chain
-    if (!(h_first && par)) ZKR_TRY(h_front());
-    cudaStream_t sHm = sH;
-    if (par && h_split) {
-        sHm = ctx->s[5];
-        ZKR_CUDA(cudaEventRecord(ctx->ev_join[6], sH));
-        ZKR_CUDA(cudaStreamWaitEvent(sHm, ctx->ev_join[6], 0));
-    }
-    ZKR_TRY(delayed('H', sHm));
-    if (has_h) {
-        ZKR_TRY(msm_run_g1(ctx, sHm, pk->H, (const uint32_t*)(pk->h + pk->h_lo), pk->res + R_H, nullptr, nullptr, nullptr, late('h')));
-    } else {
-        ZKR_CUDA(cudaMemsetAsync(pk->res + R_H, 0, 128, sHm));   // the identity (ZZ = 0)
-    }
-    if (timed) cudaEventRecord(ev[3], sHm);
+    if (timed) cudaEventRecord(ev[3], sH);
     // A, then s * pi_a
     if (timed) cudaEventRecord(ev[4], sA);
-    ZKR_TRY(delayed('A', sA));
-    ZKR_TRY(msm_run_g1(ctx, sA, pk->A, w, pk->res + R_A, nullptr, nullptr, nullptr, late('a')));
+    ZKR_TRY(msm_run_g1(ctx, sA, pk->A, w, pk->res + R_A));
     if (timed) cudaEventRecord(ev[5], sA);
     if (timed) cudaEventRecord(ev[8], sB1);
-    ZKR_TRY(delayed('B', sB1));
-    if (pk->share_b_sort) {
-        ZKR_CUDA(cudaStreamWaitEvent(sB1, pk->ev_b2_sorted, 0));
-        ZKR_TRY(msm_run_g1(ctx, sB1, pk->B1, w, pk->res + R_B1, pk->B2, nullptr, nullptr, late('b')));
-    } else {
-        ZKR_TRY(msm_run_g1(ctx, sB1, pk->B1, w, pk->res + R_B1, nullptr, nullptr, nullptr, late('b')));
-    }
+    if (pk->share_b_sort) ZKR_CUDA(cudaStreamWaitEvent(sB1, pk->ev_b2_sorted, 0));
+    ZKR_TRY(msm_run_g1(ctx, sB1, pk->B1, w, pk->res + R_B1, pk->share_b_sort ? pk->B2 : nullptr));
     if (timed) cudaEventRecord(ev[9], sB1);
     if (timed) cudaEventRecord(ev[10], sC);
-    ZKR_TRY(delayed('C', sC));
-    ZKR_TRY(msm_run_g1(ctx, sC, pk->C, w, pk->res + R_C, nullptr, nullptr, nullptr, late('c')));
+    ZKR_TRY(msm_run_g1(ctx, sC, pk->C, w, pk->res + R_C));
     if (timed) cudaEventRecord(ev[11], sC);
-    // the two blinding scalar multiplications T1 = s * pi_a, T2 = r * pib1 need A and B1
-    auto blind = [&]() -> int {
-        if (par) {
-            ZKR_CUDA(cudaEventRecord(ctx->ev_join[2], sB1));
-            ZKR_CUDA(cudaStreamWaitEvent(sA, ctx->ev_join[2], 0));
-        }
-        ZKR_LAUNCH(ctx, k_blind_muls, 2, 32 * kBlindWarps, kBlindSmem, sA, pk->res, wext, n);
-        return ZKR_OK;
-    };
+    // the two blinding scalar multiplications T1 = s * pi_a, T2 = r * pib1 need A and B1.  A sharded proof's results are
+    // partial sums over this rank's point ranges; scalar multiplication is linear, so each rank blinds its own partial
+    // A / B1 behind the A chain (off the critical H chain) and the gather sums seven partials.
+    if (par) {
+        ZKR_CUDA(cudaEventRecord(ctx->ev_join[2], sB1));
+        ZKR_CUDA(cudaStreamWaitEvent(sA, ctx->ev_join[2], 0));
+    }
+    ZKR_LAUNCH(ctx, k_blind_muls, 2, 32 * kBlindWarps, kBlindSmem, sA, pk->res, wext, n);
+    if (par) ZKR_TRY(ctx->join(5));
     if (comm && comm->world > 1) {
-        // sharded: the results are partial sums over this rank's point ranges.  Scalar multiplication is linear, so each
-        // rank blinds its own partial A / B1 behind the A chain (off the critical H chain) and the gather sums seven
-        // partials; ZKR_SHARDED_BLIND_LATE=1 (A/B knob) blinds the summed A / B1 after the gather instead.
-        static const bool blind_late = getenv("ZKR_SHARDED_BLIND_LATE") && atoi(getenv("ZKR_SHARDED_BLIND_LATE")) != 0;
-        if (!blind_late) ZKR_TRY(blind());
-        if (par) ZKR_TRY(ctx->join(n_fork));
         if (timed) cudaEventRecord(ev[16], us);
         int parity = 0;
         ZKR_TRY(comm_allgather_small(comm, us, pk->res, R_TOTAL, &parity));
         if (timed) cudaEventRecord(ev[17], us);
-        ZKR_LAUNCH(ctx, k_sum_res, blind_late ? 5 : 7, 1, 0, us, comm_gather_slot(comm, comm->rank, parity, 0), comm->world,
-                   pk->res);
+        ZKR_LAUNCH(ctx, k_sum_res, 7, 1, 0, us, comm_gather_slot(comm, comm->rank, parity, 0), comm->world, pk->res);
         if (timed) cudaEventRecord(ev[18], us);
-        if (blind_late) ZKR_LAUNCH(ctx, k_blind_muls, 2, 32 * kBlindWarps, kBlindSmem, us, pk->res, wext, n);
-    } else {
-        ZKR_TRY(blind());
-        if (par) ZKR_TRY(ctx->join(n_fork));
     }
     if (timed) cudaEventRecord(ev[12], us);
-    static const int finish_fermat = getenv("ZKR_FINISH_FERMAT") ? atoi(getenv("ZKR_FINISH_FERMAT")) : 0;   // experiment knob
-    ZKR_LAUNCH(ctx, k_finish, 3, 1, 0, us, (const char*)pk->res, d_proof, finish_fermat);
+    ZKR_LAUNCH(ctx, k_finish, 3, 1, 0, us, (const char*)pk->res, d_proof);
     if (timed) cudaEventRecord(ev[13], us);
     return ZKR_OK;
 }
