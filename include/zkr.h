@@ -344,8 +344,9 @@ int zkr_synth_setup(zkr_ctx* ctx, const zkr_r1cs_csc* r1cs, const void* toxic, v
  * Security statement.  A key made here is sound if the phase-1 ceremony's tau, alpha and beta are unknown to
  * everyone AND at least one phase-2 contributor erased their delta'.  A key straight out of zkr_setup_from_powers
  * has gamma = delta = 1 (as snarkjs's `zkey new`) and is FORGEABLE until one contribution has been applied.
- * Phase 1 is NOT verified here: neither the subgroup membership of the G2 powers nor the same-ratio consistency
- * of the powers is checked; the powers are taken from a ceremony the caller already trusts.
+ * zkr_setup_from_powers does NOT verify phase 1: neither the subgroup membership of the G2 powers nor the same-ratio
+ * consistency of the powers is checked.  Check them first with zkr_powers_verify (and every phase-1 contribution
+ * with zkr_powers_verify_contribution, below), or take them from a ceremony the caller already trusts.
  *
  * Phase-1 points, host memory, affine Fq-M in the binary key encoding (64 B G1, 128 B G2 = x.c0|x.c1|y.c0|y.c1);
  * n_* counts the points given, only the first are read, so a ceremony of size 2^K >= m is passed as is:
@@ -365,7 +366,8 @@ typedef struct zkr_powers {
  *   H_k = [tau^(k+m)] - [tau^k] = [tau^k Z(tau)],
  *   vk: alfa1 = alpha_tau_g1[0], beta1 = beta_tau_g1[0], delta1 = G1, beta2 = beta_g2, gamma2 = delta2 = G2.
  * Every input is checked on the host before any launch: counts, coordinates < q, points on their curve, no power at
- * infinity, R1CS rows < m and coefficients < r.  ZKR_E_INVALID otherwise; zkr_last_error names the section and index. */
+ * infinity, R1CS rows < m and coefficients < r.  ZKR_E_INVALID otherwise; zkr_last_error names the section and index.
+ * The powers themselves are not verified (G2 subgroup, same ratios): zkr_powers_verify does that. */
 int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r1cs, const zkr_powers* powers, void* out_a, void* out_b1,
                           void* out_b2, void* out_c, void* out_h, void* out_vk);
 #define ZKR_CONTRIB_RECORD_BYTES 96
@@ -392,6 +394,49 @@ int zkr_setup_contribute(zkr_ctx* ctx, const void* pk, size_t pk_len, const void
  * ZKR_E_INVALID only for a malformed old layout or buffer sizes (both keys have pk_len / vk_len bytes). */
 int zkr_setup_verify_contribution(zkr_ctx* ctx, const void* old_pk, const void* old_vk, const void* new_pk,
                                   const void* new_vk, size_t pk_len, size_t vk_len, const void* record, int* valid);
+
+/* ---- phase 1: contributions to the powers of tau, and their verification ------------------------------------
+ * The powers zkr_setup_from_powers takes, made and checked on the GPU.  Points as in zkr_powers (host memory, affine
+ * Fq-M, key encoding).  Counts are free within n_tau_g1 >= 2, n_tau_g2 >= 2, n_alpha_tau_g1 >= 1, n_beta_tau_g1 >= 1,
+ * each <= 2^28 (2m G1 powers for the largest m zkr_setup_from_powers takes); snarkjs's 2^(K+1) - 1 / 2^K is one case.
+ * Malformed counts or NULL sections are ZKR_E_INVALID with the section named.  An empty ceremony has every point a
+ * generator (tau = alpha = beta = 1). */
+#define ZKR_POWERS_RECORD_BYTES 288
+/* One contribution with secrets (tau', alpha', beta') = secrets96 (3 x 32 B std form, each in [1, r); NULL = each
+ * drawn from getrandom, redrawn if zero).  Outputs (caller buffers of the input's counts):
+ *   tau_g1'[k] = tau'^k tau_g1[k]               tau_g2'[k] = tau'^k tau_g2[k]
+ *   alpha_tau_g1'[k] = alpha' tau'^k alpha_tau_g1[k]   beta_tau_g1'[k] = beta' tau'^k beta_tau_g1[k]
+ *   beta_g2' = beta' beta_g2
+ * so contributing to the powers of (tau, alpha, beta) gives exactly the powers of (tau tau', alpha alpha', beta beta').
+ * out_record (288 B) is three Schnorr proofs of knowledge, for tau', alpha', beta' in that order, each R (64 B, Fq-M) |
+ * z (32 B std).  For the secret s' with base P_old and P_new = s' P_old:  R = k P_old (k from getrandom, nonzero),
+ *   c = SHA-256("zkr-phase1-" name | P_old | P_new | R) mod r  (name "tau" / "alpha" / "beta", points as their 64 key
+ *       bytes, the digest a 256-bit little-endian integer),  z = k + c s' mod r,
+ * with bases P_old = tau_g1[1], alpha_tau_g1[0], beta_tau_g1[0] of the input.  The format is this library's own, not
+ * snarkjs's .ptau contribution.  The input is checked on the host before any launch (counts, coordinates < q, on the
+ * curve, no infinity; not the G2 subgroup: that is zkr_powers_verify's job), and so are the secrets: ZKR_E_INVALID with
+ * the section and index, or the secret, in the message.  The secrets, the tables of tau'^k and the nonces are zeroed on
+ * the host and the device before the call returns, on error paths too. */
+int zkr_powers_contribute(zkr_ctx* ctx, const zkr_powers* in, const void* secrets96, void* out_tau_g1, void* out_tau_g2,
+                          void* out_alpha_tau_g1, void* out_beta_tau_g1, void* out_beta_g2, void* out_record);
+/* *valid = 1 iff the powers are well formed:
+ *   1. every point has coordinates < q, is on its curve and is not infinity (x encoding 0); every G2 point (tau_g2,
+ *      beta_g2) is in the order-r subgroup ([r]Q = O, one GPU thread per point);
+ *   2. tau_g1[0] is the G1 generator and tau_g2[0] the G2 generator, byte for byte;
+ *   3. e(sum rho_k T1[k+1] + sigma_k A[k+1] + pi_k B[k+1], G2) = e(sum rho_k T1[k] + sigma_k A[k] + pi_k B[k], tau_g2[1])
+ *      (T1 = tau_g1, A = alpha_tau_g1, B = beta_tau_g1; fresh 128-bit CSPRNG scalars; GPU MSMs, host pairings);
+ *   4. e(G1, sum rho'_k T2[k+1]) = e(tau_g1[1], sum rho'_k T2[k])  (T2 = tau_g2);
+ *   5. e(beta_tau_g1[0], G2) = e(G1, beta_g2).
+ * Unlike other verdict-returning calls, *valid = 0 also sets zkr_last_error() to the first failed check, e.g.
+ * "tau_g2[5] is not in the order-r subgroup" or "G1 same-ratio check failed". */
+int zkr_powers_verify(zkr_ctx* ctx, const zkr_powers* p, int* valid);
+/* *valid = 1 iff new_p is old_p after the contribution `record` proves:  the three old bases are valid points; each
+ * proof's R is a valid point and z < r;  z P_old = R + c P_new for tau, alpha and beta;  and new_p passes every check
+ * of zkr_powers_verify.  old_p is assumed verified when it was made: a transcript is checked link by link.  The first
+ * failed check is in zkr_last_error(), as for zkr_powers_verify.  ZKR_E_INVALID for malformed counts or pointers, and
+ * for counts that differ between old_p and new_p. */
+int zkr_powers_verify_contribution(zkr_ctx* ctx, const zkr_powers* old_p, const zkr_powers* new_p, const void* record,
+                                   int* valid);
 
 /* points[i] = scalars[i] * G (group 1: G1 generator (1,2); group 2: the G2 generator of TxVerifier.sol:30-35);
  * scalars n x 32 B std form, out n x 64 / 128 B affine Fq-M; host buffers.  Workload generator for the

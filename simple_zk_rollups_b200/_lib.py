@@ -9,6 +9,7 @@ LIB_PATH = os.environ.get("ZKR_LIB") or os.path.join(HERE, "libzkr.so")
 
 PROOF_BYTES = 256
 CONTRIB_RECORD_BYTES = 96
+POWERS_RECORD_BYTES = 288
 
 
 class ZkrError(RuntimeError):
@@ -113,6 +114,10 @@ _SIGS = {
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "zkr_setup_verify_contribution": (C.c_int, [C.c_void_p] + [C.c_void_p] * 4 + [C.c_size_t, C.c_size_t, C.c_void_p,
                                                                                   C.POINTER(C.c_int)]),
+    "zkr_powers_contribute": (C.c_int, [C.c_void_p, C.POINTER(Powers), C.c_void_p] + [C.c_void_p] * 6),
+    "zkr_powers_verify": (C.c_int, [C.c_void_p, C.POINTER(Powers), C.POINTER(C.c_int)]),
+    "zkr_powers_verify_contribution": (C.c_int, [C.c_void_p, C.POINTER(Powers), C.POINTER(Powers), C.c_void_p,
+                                                 C.POINTER(C.c_int)]),
     "zkr_synth_points": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "zkr_test_field_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "zkr_test_curve_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),

@@ -14,14 +14,7 @@
 //   * Contributions: one thread per C / H point multiplies by the single scalar delta'^-1 with 4-bit signed windows.
 //   * Verification: two bucketed MSMs (zkr_msm) with shared random 128-bit scalars over the C|H section, and host
 //     pairings (verify.cu).
-#include <algorithm>
-#include <cstddef>
-#include <cstring>
-#include <thread>
-#include <vector>
-
-#include "ec.cuh"
-#include "host_ec.cuh"
+#include "ceremony.cuh"
 #include "ntt_iface.cuh"
 
 using namespace zkr;
@@ -29,7 +22,6 @@ using namespace zkr;
 namespace {
 
 constexpr uint32_t kSegChunk = 32;
-constexpr int kDigits = 64;            // 4-bit signed windows of a scalar < r < 2^254: the top one never carries out
 
 // ------------------------------------------------------------------------------------------------ point NTT
 // X[bitrev(k)] = P[k]: the DIT stages below then leave the transform in natural order
@@ -70,13 +62,6 @@ __global__ void k_pntt_scale(XYZZ<F>* X, size_t n, const NttRoots* roots) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     scalar_mul(XYZZ<F>::load(X + i), roots->ninv.from_mont()).store(X + i);
-}
-
-template <class F>
-__device__ __forceinline__ void store_key_point(const XYZZ<F>& p, Affine<F>* out) {
-    Affine<F> a = {F::zero(), F::one()};      // infinity as binarifyProvingKey writes it: (0, R mod q)
-    if (!p.is_inf()) a = p.to_affine();
-    a.store(out);
 }
 
 // H_k = [tau^(k+m)] - [tau^k]; infinity where tau^(k+m) is not given (k = m - 1 with 2m - 1 powers)
@@ -126,27 +111,12 @@ __global__ void k_col_affine(const XYZZ<F>* __restrict__ in, const uint32_t* __r
     store_key_point(ptr[i + 1] > ptr[i] ? XYZZ<F>::load(in + ptr[i]) : XYZZ<F>::identity(), out + i);
 }
 
-__global__ void k_generators(G1Affine* g1, G2Affine* g2) {
-    generator<Fq>().store(g1);
-    generator<Fq2>().store(g2);
-}
-
 // ------------------------------------------------------------------------------------------------ contribution
 // Device copy of the contribution's secrets; zeroed before the call returns.
 struct Secrets {
     Fr delta, k, c, z;                  // std form; c is public, z the Schnorr response
     int8_t dig[3][kDigits];             // signed 4-bit windows of delta', delta'^-1, k
 };
-
-// digits in [-7, 8], scalar = sum dig[w] 16^w
-__device__ __forceinline__ void recode(const Fr& s, int8_t* dig) {
-    int carry = 0;
-    for (int w = 0; w < kDigits; w++) {
-        int d = (int)((s.v[w >> 3] >> ((w & 7) * 4)) & 15) + carry;
-        carry = d > 8;
-        dig[w] = (int8_t)(d - 16 * carry);
-    }
-}
 
 __global__ void k_contrib_prep(Secrets* s) {
     recode(s->delta, s->dig[0]);
@@ -186,142 +156,13 @@ __global__ void k_fixed_mul(Affine<F>* pts, size_t n, const int8_t* __restrict__
     store_key_point(acc, pts + i);
 }
 
-// z * P0 == P2 + c * P1 ?   (P0 = delta1_old, P1 = delta1_new, P2 = R; zc = z | c std form)
-__global__ void k_schnorr_check(const G1Affine* pts, const Fr* zc, int* ok) {
-    const G1XYZZ lhs = scalar_mul(G1XYZZ::from_affine(pts[0]), zc[0]);
-    G1XYZZ rhs = scalar_mul(G1XYZZ::from_affine(pts[1]), zc[1]);
-    rhs.add(G1XYZZ::from_affine(pts[2]));
-    if (lhs.is_inf() || rhs.is_inf()) {
-        *ok = lhs.is_inf() && rhs.is_inf();
-        return;
-    }
-    const G1Affine a = lhs.to_affine(), b = rhs.to_affine();
-    *ok = a.x == b.x && a.y == b.y;
-}
-
 // ------------------------------------------------------------------------------------------------ host helpers
-// Device buffers of one call, freed when the call returns, on its error paths too.
-struct DevAllocs {
-    std::vector<void*> p;
-    DevAllocs() = default;
-    DevAllocs(const DevAllocs&) = delete;
-    DevAllocs& operator=(const DevAllocs&) = delete;
-    ~DevAllocs() {
-        for (void* q : p) cudaFree(q);
-    }
-    template <class T>
-    int alloc(T** out, size_t bytes) {
-        ZKR_CUDA(cudaMalloc(out, bytes ? bytes : 1));
-        p.push_back(*out);
-        return ZKR_OK;
-    }
-    void release(void* q) {
-        auto it = std::find(p.begin(), p.end(), q);
-        if (it == p.end()) return;
-        cudaFree(q);
-        p.erase(it);
-    }
-};
 
 int up32(DevAllocs& a, const uint32_t* h, size_t count, uint32_t** d, cudaStream_t st) {
     ZKR_TRY(a.alloc(d, 4 * count));
     if (count) ZKR_CUDA(cudaMemcpyAsync(*d, h, 4 * count, cudaMemcpyHostToDevice, st));
     return ZKR_OK;
 }
-
-void wipe(void* p, size_t n) {
-    volatile uint8_t* v = (volatile uint8_t*)p;
-    for (size_t i = 0; i < n; i++) v[i] = 0;
-}
-
-bool lt_r(const uint8_t* b32) {
-    uint32_t v[8];
-    memcpy(v, b32, 32);
-    for (int i = 7; i >= 0; i--)
-        if (v[i] != kRModulus[i]) return v[i] < kRModulus[i];
-    return false;
-}
-bool is_zero32(const uint8_t* b32) {
-    uint8_t acc = 0;
-    for (int i = 0; i < 32; i++) acc |= b32[i];
-    return acc == 0;
-}
-// b32 -= r while b32 >= r  (a 256-bit value is below 6 r)
-void reduce_r(uint8_t* b32) {
-    while (!lt_r(b32)) {
-        uint32_t v[8];
-        memcpy(v, b32, 32);
-        uint64_t borrow = 0;
-        for (int i = 0; i < 8; i++) {
-            const uint64_t d = (uint64_t)v[i] - kRModulus[i] - borrow;
-            v[i] = (uint32_t)d;
-            borrow = (d >> 63) & 1;
-        }
-        memcpy(b32, v, 32);
-    }
-}
-
-// ---- SHA-256 (FIPS 180-4), host, for the contribution challenge
-struct Sha256 {
-    uint32_t h[8] = {0x6a09e667u, 0xbb67ae85u, 0x3c6ef372u, 0xa54ff53au, 0x510e527fu, 0x9b05688cu, 0x1f83d9abu, 0x5be0cd19u};
-    uint8_t buf[64];
-    size_t fill = 0;
-    uint64_t bits = 0;
-
-    static uint32_t rotr(uint32_t x, int n) { return (x >> n) | (x << (32 - n)); }
-    void block(const uint8_t* p) {
-        static const uint32_t K[64] = {
-            0x428a2f98u, 0x71374491u, 0xb5c0fbcfu, 0xe9b5dba5u, 0x3956c25bu, 0x59f111f1u, 0x923f82a4u, 0xab1c5ed5u,
-            0xd807aa98u, 0x12835b01u, 0x243185beu, 0x550c7dc3u, 0x72be5d74u, 0x80deb1feu, 0x9bdc06a7u, 0xc19bf174u,
-            0xe49b69c1u, 0xefbe4786u, 0x0fc19dc6u, 0x240ca1ccu, 0x2de92c6fu, 0x4a7484aau, 0x5cb0a9dcu, 0x76f988dau,
-            0x983e5152u, 0xa831c66du, 0xb00327c8u, 0xbf597fc7u, 0xc6e00bf3u, 0xd5a79147u, 0x06ca6351u, 0x14292967u,
-            0x27b70a85u, 0x2e1b2138u, 0x4d2c6dfcu, 0x53380d13u, 0x650a7354u, 0x766a0abbu, 0x81c2c92eu, 0x92722c85u,
-            0xa2bfe8a1u, 0xa81a664bu, 0xc24b8b70u, 0xc76c51a3u, 0xd192e819u, 0xd6990624u, 0xf40e3585u, 0x106aa070u,
-            0x19a4c116u, 0x1e376c08u, 0x2748774cu, 0x34b0bcb5u, 0x391c0cb3u, 0x4ed8aa4au, 0x5b9cca4fu, 0x682e6ff3u,
-            0x748f82eeu, 0x78a5636fu, 0x84c87814u, 0x8cc70208u, 0x90befffau, 0xa4506cebu, 0xbef9a3f7u, 0xc67178f2u};
-        uint32_t w[64];
-        for (int i = 0; i < 16; i++) w[i] = (uint32_t)p[4 * i] << 24 | (uint32_t)p[4 * i + 1] << 16 | (uint32_t)p[4 * i + 2] << 8 | p[4 * i + 3];
-        for (int i = 16; i < 64; i++) {
-            const uint32_t s0 = rotr(w[i - 15], 7) ^ rotr(w[i - 15], 18) ^ (w[i - 15] >> 3);
-            const uint32_t s1 = rotr(w[i - 2], 17) ^ rotr(w[i - 2], 19) ^ (w[i - 2] >> 10);
-            w[i] = w[i - 16] + s0 + w[i - 7] + s1;
-        }
-        uint32_t a = h[0], b = h[1], c = h[2], d = h[3], e = h[4], f = h[5], g = h[6], hh = h[7];
-        for (int i = 0; i < 64; i++) {
-            const uint32_t t1 = hh + (rotr(e, 6) ^ rotr(e, 11) ^ rotr(e, 25)) + ((e & f) ^ (~e & g)) + K[i] + w[i];
-            const uint32_t t2 = (rotr(a, 2) ^ rotr(a, 13) ^ rotr(a, 22)) + ((a & b) ^ (a & c) ^ (b & c));
-            hh = g; g = f; f = e; e = d + t1; d = c; c = b; b = a; a = t1 + t2;
-        }
-        h[0] += a; h[1] += b; h[2] += c; h[3] += d; h[4] += e; h[5] += f; h[6] += g; h[7] += hh;
-    }
-    void update(const void* data, size_t n) {
-        const uint8_t* p = (const uint8_t*)data;
-        bits += 8ull * n;
-        while (n) {
-            const size_t k = std::min(n, 64 - fill);
-            memcpy(buf + fill, p, k);
-            fill += k;
-            p += k;
-            n -= k;
-            if (fill == 64) {
-                block(buf);
-                fill = 0;
-            }
-        }
-    }
-    void final(uint8_t out[32]) {
-        const uint64_t total = bits;
-        const uint8_t pad = 0x80;
-        update(&pad, 1);
-        const uint8_t zero = 0;
-        while (fill != 56) update(&zero, 1);
-        uint8_t len[8];
-        for (int i = 0; i < 8; i++) len[i] = (uint8_t)(total >> (56 - 8 * i));
-        update(len, 8);
-        for (int i = 0; i < 8; i++)
-            for (int j = 0; j < 4; j++) out[4 * i + j] = (uint8_t)(h[i] >> (24 - 8 * j));
-    }
-};
 
 // c = SHA-256("zkr-phase2-delta" | delta1_old | delta1_new | R) as a little-endian integer mod r
 void challenge(const uint8_t* d1_old, const uint8_t* d1_new, const uint8_t* R, uint8_t c[32]) {
@@ -353,45 +194,6 @@ bool key_layout(const void* pk, size_t len, size_t vk_len, KeyLayout* v) {
 }
 
 // ---- setup_from_powers input checks
-const char* point_problem(int code) {
-    switch (code) {
-        case PT_INFINITY: return "is the point at infinity";
-        case PT_RANGE: return "has a coordinate >= q";
-        default: return "is not on the curve";
-    }
-}
-// count >= need points given, and the first `used` of them (every point the setup reads) valid
-int check_section(const char* name, int group, const void* pts, uint32_t count, uint32_t need, uint32_t used) {
-    if (count < need || !pts) {
-        set_error("zkr_setup_from_powers: %s has %u points, %u needed", name, pts ? count : 0u, need);
-        return ZKR_E_INVALID;
-    }
-    need = used;
-    const size_t sz = group == 1 ? 64 : 128;
-    const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, need / 4096 + 1}));
-    std::vector<uint32_t> bad(nt, need);
-    std::vector<int> code(nt, PT_OK);
-    std::vector<std::thread> th;
-    for (unsigned t = 0; t < nt; t++)
-        th.emplace_back([&, t] {
-            const uint32_t lo = (uint32_t)((uint64_t)need * t / nt), hi = (uint32_t)((uint64_t)need * (t + 1) / nt);
-            for (uint32_t i = lo; i < hi; i++) {
-                const int c = host_point_check(group, (const uint8_t*)pts + sz * i, false);
-                if (c != PT_OK) {
-                    bad[t] = i;
-                    code[t] = c;
-                    return;
-                }
-            }
-        });
-    for (auto& t : th) t.join();
-    for (unsigned t = 0; t < nt; t++)
-        if (bad[t] < need) {
-            set_error("zkr_setup_from_powers: %s[%u] %s", name, bad[t], point_problem(code[t]));
-            return ZKR_E_INVALID;
-        }
-    return ZKR_OK;
-}
 
 // CSC columns of one sum: for column i, entries [ptr[i], ptr[i+1]) of (point index, pool index)
 struct Cols {
@@ -516,11 +318,11 @@ extern "C" int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r, const 
     }
     ZKR_TRY(check_r1cs(r));
     const uint32_t n_tau = std::min(pw->n_tau_g1, 2 * m);      // tau^(2m-1), when given, makes H_(m-1)
-    ZKR_TRY(check_section("tau_g1", 1, pw->tau_g1, pw->n_tau_g1, 2 * m - 1, n_tau));
-    ZKR_TRY(check_section("tau_g2", 2, pw->tau_g2, pw->n_tau_g2, m, m));
-    ZKR_TRY(check_section("alpha_tau_g1", 1, pw->alpha_tau_g1, pw->n_alpha_tau_g1, m, m));
-    ZKR_TRY(check_section("beta_tau_g1", 1, pw->beta_tau_g1, pw->n_beta_tau_g1, m, m));
-    ZKR_TRY(check_section("beta_g2", 2, pw->beta_g2, 1, 1, 1));
+    ZKR_TRY(check_section("zkr_setup_from_powers", "tau_g1", 1, pw->tau_g1, pw->n_tau_g1, 2 * m - 1, n_tau));
+    ZKR_TRY(check_section("zkr_setup_from_powers", "tau_g2", 2, pw->tau_g2, pw->n_tau_g2, m, m));
+    ZKR_TRY(check_section("zkr_setup_from_powers", "alpha_tau_g1", 1, pw->alpha_tau_g1, pw->n_alpha_tau_g1, m, m));
+    ZKR_TRY(check_section("zkr_setup_from_powers", "beta_tau_g1", 1, pw->beta_tau_g1, pw->n_beta_tau_g1, m, m));
+    ZKR_TRY(check_section("zkr_setup_from_powers", "beta_g2", 2, pw->beta_g2, 1, 1, 1));
 
     DeviceGuard g(ctx->device);
     cudaStream_t st = ctx->s[0];

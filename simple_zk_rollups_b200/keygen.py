@@ -6,6 +6,8 @@ public powers-of-tau ceremony and contribute() re-randomises delta (phase 2); ve
 contribution.  Such a key is sound once at least one contributor erased their delta'.  Output is the websnark
 binary proving key -- byte-identical to binarifyProvingKey(snarkjs pk JSON) for the same
 (R1CS, toxic waste) -- plus the verifying key as Python ints (and as the binary block zkr_vkey_load_bin takes, vk["bin"]).
+The powers themselves come from phase 1 here too: powers_new() is the empty ceremony, powers_contribute() adds one
+contribution, powers_verify_contribution() checks one, and powers_verify() checks the powers before setup_from_powers.
 """
 import ctypes as C
 import struct
@@ -121,13 +123,8 @@ def synth_setup(ctx, r1cs, toxic):
 _POWER_SECTIONS = (("tau_g1", 64), ("tau_g2", 128), ("alpha_tau_g1", 64), ("beta_tau_g1", 64))
 
 
-def setup_from_powers(ctx, r1cs, powers):
-    """Circuit key from phase-1 powers of tau (zkr_setup_from_powers; zkr.h has the math and the security statement).
-    powers: dict of byte buffers (bytes / uint8 arrays) of affine Fq-M points in the key encoding: "tau_g1"
-    (>= 2m - 1 points, 2m for H_(m-1)), "tau_g2", "alpha_tau_g1", "beta_tau_g1" (>= m each) and "beta_g2" (one point).
-    -> (pk_bin, vk) as synth_setup, for gamma = delta = 1: NOT deployable before one contribute()."""
-    L = _lib.lib()
-    desc, csc, keep = _r1cs_desc(r1cs)
+def _powers_desc(powers, keep):
+    """zkr_powers for a powers dict; the buffers it points to are appended to keep."""
     pw = _lib.Powers()
     for name, size in _POWER_SECTIONS + (("beta_g2", 128),):
         buf = np.frombuffer(bytes(powers[name]), dtype=np.uint8)
@@ -139,6 +136,17 @@ def setup_from_powers(ctx, r1cs, powers):
             setattr(pw, "n_" + name, min(buf.size // size, 0xFFFFFFFF))
         elif buf.size != 128:
             raise ValueError("beta_g2 must be one 128-byte G2 point")
+    return pw
+
+
+def setup_from_powers(ctx, r1cs, powers):
+    """Circuit key from phase-1 powers of tau (zkr_setup_from_powers; zkr.h has the math and the security statement).
+    powers: dict of byte buffers (bytes / uint8 arrays) of affine Fq-M points in the key encoding: "tau_g1"
+    (>= 2m - 1 points, 2m for H_(m-1)), "tau_g2", "alpha_tau_g1", "beta_tau_g1" (>= m each) and "beta_g2" (one point).
+    -> (pk_bin, vk) as synth_setup, for gamma = delta = 1: NOT deployable before one contribute()."""
+    L = _lib.lib()
+    desc, csc, keep = _r1cs_desc(r1cs)
+    pw = _powers_desc(powers, keep)
     outs = _outputs(r1cs.nVars, r1cs.nPublic, r1cs.domain()[1])
     _lib.check(L.zkr_setup_from_powers(ctx, C.byref(desc), C.byref(pw), *[_lib.buf_ptr(x) for x in outs]))
     return _assemble(r1cs, csc, *outs)
@@ -179,3 +187,65 @@ def verify_contribution(ctx, old_pk, old_vk, new_pk, new_vk, record):
                                                _lib.buf_ptr(vn), po.size, vo.size, _lib.buf_ptr(rec),
                                                C.byref(valid)))
     return bool(valid.value)
+
+
+# ------------------------------------------------------------------------------------------------ phase 1
+def _gen_points(ctx, group, n):
+    one = (1).to_bytes(32, "little")
+    out = np.empty(64 if group == 1 else 128, dtype=np.uint8)
+    _lib.check(_lib.lib().zkr_synth_points(ctx, group, _lib.buf_ptr(one), 1, _lib.buf_ptr(out)))
+    return out.tobytes() * n
+
+
+def powers_new(ctx, m, n_tau_g1=None):
+    """The empty ceremony (tau = alpha = beta = 1): every point a generator; tau_g1 has n_tau_g1 points (default 2m),
+    tau_g2, alpha_tau_g1 and beta_tau_g1 m each.  A powers dict as setup_from_powers takes."""
+    n_tau_g1 = 2 * m if n_tau_g1 is None else n_tau_g1
+    return {"tau_g1": _gen_points(ctx, 1, n_tau_g1), "tau_g2": _gen_points(ctx, 2, m),
+            "alpha_tau_g1": _gen_points(ctx, 1, m), "beta_tau_g1": _gen_points(ctx, 1, m),
+            "beta_g2": _gen_points(ctx, 2, 1)}
+
+
+def powers_contribute(ctx, powers, tau=None, alpha=None, beta=None):
+    """One phase-1 contribution (zkr_powers_contribute): the powers of (tau tau', alpha alpha', beta beta').
+    tau, alpha, beta: ints in [1, r) (tests, reproducible transcripts), or all None = drawn from the OS CSPRNG and never
+    seen by Python.  -> (new powers dict, 288-byte record: Schnorr proofs of knowledge of tau', alpha', beta')."""
+    given = [x is not None for x in (tau, alpha, beta)]
+    if any(given) and not all(given):
+        raise ValueError("give all three secrets or none")
+    keep = []
+    pw = _powers_desc(powers, keep)
+    out = {name: np.empty(len(bytes(powers[name])), dtype=np.uint8) for name, _ in _POWER_SECTIONS + (("beta_g2", 128),)}
+    rec = np.empty(_lib.POWERS_RECORD_BYTES, dtype=np.uint8)
+    sec = None if tau is None else b"".join(int(x).to_bytes(32, "little") for x in (tau, alpha, beta))
+    _lib.check(_lib.lib().zkr_powers_contribute(ctx, C.byref(pw), _lib.buf_ptr(sec), *[
+        _lib.buf_ptr(out[name]) for name in ("tau_g1", "tau_g2", "alpha_tau_g1", "beta_tau_g1", "beta_g2")],
+        _lib.buf_ptr(rec)))
+    return {name: buf.tobytes() for name, buf in out.items()}, rec.tobytes()
+
+
+def _verdict(valid):
+    return (True, "") if valid.value else (False, _lib.lib().zkr_last_error().decode())
+
+
+def powers_verify(ctx, powers):
+    """(ok, reason): ok iff the powers are well formed (zkr_powers_verify lists the checks); reason names the first
+    failed check."""
+    keep = []
+    pw = _powers_desc(powers, keep)
+    valid = C.c_int(0)
+    _lib.check(_lib.lib().zkr_powers_verify(ctx, C.byref(pw), C.byref(valid)))
+    return _verdict(valid)
+
+
+def powers_verify_contribution(ctx, old, new, record):
+    """(ok, reason): ok iff `new` is `old` after the contribution `record` proves, and `new` is well formed."""
+    rec = bytes(record)
+    if len(rec) != _lib.POWERS_RECORD_BYTES:
+        raise ValueError("the record is not %d bytes" % _lib.POWERS_RECORD_BYTES)
+    keep = []
+    po, pn = _powers_desc(old, keep), _powers_desc(new, keep)
+    valid = C.c_int(0)
+    _lib.check(_lib.lib().zkr_powers_verify_contribution(ctx, C.byref(po), C.byref(pn), _lib.buf_ptr(rec),
+                                                         C.byref(valid)))
+    return _verdict(valid)
