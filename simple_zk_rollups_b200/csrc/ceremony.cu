@@ -112,69 +112,16 @@ __global__ void k_col_affine(const XYZZ<F>* __restrict__ in, const uint32_t* __r
 }
 
 // ------------------------------------------------------------------------------------------------ contribution
-// Device copy of the contribution's secrets; zeroed before the call returns.
+// Device copy of the contribution's secrets, std form
 struct Secrets {
-    Fr delta, k, c, z;                  // std form; c is public, z the Schnorr response
-    int8_t dig[3][kDigits];             // signed 4-bit windows of delta', delta'^-1, k
+    Fr delta, k;                        // delta' and the Schnorr nonce
+    Fr dinv;                            // delta'^-1
+    Fr c, z;                            // challenge and response (public)
 };
 
-__global__ void k_contrib_prep(Secrets* s) {
-    recode(s->delta, s->dig[0]);
-    recode(s->delta.to_mont().inverse().from_mont(), s->dig[1]);
-    recode(s->k, s->dig[2]);
-}
-
-__global__ void k_contrib_z(Secrets* s) { s->z = (s->k.to_mont() + s->c.to_mont() * s->delta.to_mont()).from_mont(); }
-
-// pts[i] = scalar * pts[i] in place (key encoding in and out), scalar given by its signed 4-bit digits
-template <class F>
-__global__ void k_fixed_mul(Affine<F>* pts, size_t n, const int8_t* __restrict__ dig) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const Affine<F> a = Affine<F>::load(pts + i);
-    XYZZ<F> acc = XYZZ<F>::identity();
-    if (!a.is_inf()) {
-        XYZZ<F> t[8];       // t[d - 1] = d a
-        t[0] = XYZZ<F>::from_affine(a);
-#pragma unroll 1
-        for (int d = 1; d < 8; d++) {
-            t[d] = t[d - 1];
-            t[d].madd(a);
-        }
-        int top = kDigits - 1;
-        while (top > 0 && __ldg(dig + top) == 0) top--;
-#pragma unroll 1
-        for (int w = top; w >= 0; w--) {
-            if (w != top)
-#pragma unroll 1
-                for (int b = 0; b < 4; b++) acc = acc.dbl();
-            const int d = __ldg(dig + w);
-            if (d > 0) acc.add(t[d - 1]);
-            else if (d < 0) acc.add(t[-d - 1].neg());
-        }
-    }
-    store_key_point(acc, pts + i);
-}
+__global__ void k_delta_inverse(Secrets* s) { s->dinv = s->delta.to_mont().inverse().from_mont(); }
 
 // ------------------------------------------------------------------------------------------------ host helpers
-
-int up32(DevAllocs& a, const uint32_t* h, size_t count, uint32_t** d, cudaStream_t st) {
-    ZKR_TRY(a.alloc(d, 4 * count));
-    if (count) ZKR_CUDA(cudaMemcpyAsync(*d, h, 4 * count, cudaMemcpyHostToDevice, st));
-    return ZKR_OK;
-}
-
-// c = SHA-256("zkr-phase2-delta" | delta1_old | delta1_new | R) as a little-endian integer mod r
-void challenge(const uint8_t* d1_old, const uint8_t* d1_new, const uint8_t* R, uint8_t c[32]) {
-    static const char kTag[] = "zkr-phase2-delta";
-    Sha256 s;
-    s.update(kTag, sizeof(kTag) - 1);
-    s.update(d1_old, 64);
-    s.update(d1_new, 64);
-    s.update(R, 64);
-    s.final(c);
-    reduce_r(c);
-}
 
 // ---- websnark binary key layout (binarify.ts:152-202): 10 x u32 header, fixed block, then seven sections
 constexpr size_t kPkFixed = 40;                     // alfa1 | beta1 | delta1 | beta2 | delta2
@@ -209,8 +156,8 @@ int combine(zkr_ctx* ctx, cudaStream_t st, const XYZZ<F>* d_pts, const Cols& c, 
     XYZZ<F>* T = nullptr;
     if (nnz) {
         uint32_t *d_idx, *d_cid;
-        ZKR_TRY(up32(a, c.pidx.data(), nnz, &d_idx, st));
-        ZKR_TRY(up32(a, c.cid.data(), nnz, &d_cid, st));
+        ZKR_TRY(a.upload(&d_idx, c.pidx.data(), nnz, st));
+        ZKR_TRY(a.upload(&d_cid, c.cid.data(), nnz, st));
         ZKR_TRY(a.alloc(&T, sizeof(XYZZ<F>) * (size_t)nnz));
         ZKR_LAUNCH(ctx, k_terms<F>, ceil_div(nnz, 128), 128, 0, st, d_pts, d_idx, d_cid, d_pool, T, nnz);
         ZKR_CUDA(cudaStreamSynchronize(st));
@@ -231,7 +178,7 @@ int combine(zkr_ctx* ctx, cudaStream_t st, const XYZZ<F>* d_pts, const Cols& c, 
         const uint32_t nch = (uint32_t)start.size() - 1;
         uint32_t* d_start;
         XYZZ<F>* U;
-        ZKR_TRY(up32(a, start.data(), start.size(), &d_start, st));
+        ZKR_TRY(a.upload(&d_start, start.data(), start.size(), st));
         ZKR_TRY(a.alloc(&U, sizeof(XYZZ<F>) * (size_t)nch));
         ZKR_LAUNCH(ctx, k_seg_sum<F>, ceil_div(nch, 128), 128, 0, st, T, d_start, U, nch);
         ZKR_CUDA(cudaStreamSynchronize(st));
@@ -241,7 +188,7 @@ int combine(zkr_ctx* ctx, cudaStream_t st, const XYZZ<F>* d_pts, const Cols& c, 
         ptr.swap(next);
     }
     uint32_t* d_ptr;
-    ZKR_TRY(up32(a, ptr.data(), ptr.size(), &d_ptr, st));
+    ZKR_TRY(a.upload(&d_ptr, ptr.data(), ptr.size(), st));
     ZKR_LAUNCH(ctx, k_col_affine<F>, ceil_div(n, 128), 128, 0, st, T, d_ptr, d_out, n);
     ZKR_CUDA(cudaStreamSynchronize(st));
     return ZKR_OK;
@@ -334,23 +281,19 @@ extern "C" int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r, const 
 
     // P1 = [L | alpha L | beta L] (G1), P2 = L (G2), XYZZ
     DevAllocs a;
-    G1Affine *d_tau, *d_stage1, *d_out1, *d_gen1;
-    G2Affine *d_stage2, *d_out2, *d_gen2;
+    G1Affine *d_tau, *d_stage1, *d_out1;
+    G2Affine *d_stage2, *d_out2;
     G1XYZZ* P1;
     G2XYZZ* P2;
     Fr* d_pool;
-    ZKR_TRY(a.alloc(&d_tau, sizeof(G1Affine) * (size_t)n_tau));
     ZKR_TRY(a.alloc(&d_stage1, sizeof(G1Affine) * (size_t)m));
     ZKR_TRY(a.alloc(&d_stage2, sizeof(G2Affine) * (size_t)m));
     ZKR_TRY(a.alloc(&d_out1, sizeof(G1Affine) * (size_t)std::max(n, m)));
     ZKR_TRY(a.alloc(&d_out2, sizeof(G2Affine) * (size_t)n));
-    ZKR_TRY(a.alloc(&d_gen1, sizeof(G1Affine)));
-    ZKR_TRY(a.alloc(&d_gen2, sizeof(G2Affine)));
     ZKR_TRY(a.alloc(&P1, sizeof(G1XYZZ) * 3 * (size_t)m));
     ZKR_TRY(a.alloc(&P2, sizeof(G2XYZZ) * (size_t)m));
-    ZKR_TRY(a.alloc(&d_pool, 32 * (size_t)r->n_pool));
-    ZKR_CUDA(cudaMemcpyAsync(d_pool, r->pool, 32 * (size_t)r->n_pool, cudaMemcpyHostToDevice, st));
-    ZKR_CUDA(cudaMemcpyAsync(d_tau, pw->tau_g1, sizeof(G1Affine) * (size_t)n_tau, cudaMemcpyHostToDevice, st));
+    ZKR_TRY(a.upload(&d_pool, r->pool, r->n_pool, st));
+    ZKR_TRY(a.upload(&d_tau, pw->tau_g1, n_tau, st));
 
     // H straight from the powers
     ZKR_LAUNCH(ctx, k_h_from_powers, ceil_div(m, 128), 128, 0, st, d_tau, n_tau, d_out1, m);
@@ -393,14 +336,14 @@ extern "C" int zkr_setup_from_powers(zkr_ctx* ctx, const zkr_r1cs_csc* r, const 
     ZKR_TRY(download(st, vk + kVkIC, d_out1, l + 1));
     ZKR_TRY(download(st, out_c, d_out1 + l + 1, n - l - 1));
     // vk: alfa1 | beta1 | delta1 = G1 | beta2 | gamma2 = G2 | delta2 = G2
-    ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_gen1, d_gen2);
-    ZKR_TRY(download(st, vk + 128, d_gen1, 1));
-    ZKR_TRY(download(st, vk + 320, d_gen2, 1));
-    ZKR_TRY(download(st, vk + 448, d_gen2, 1));
-    ZKR_CUDA(cudaStreamSynchronize(st));
+    uint8_t gen[192];
+    ZKR_TRY(generators(ctx, st, gen));
     memcpy(vk, pw->alpha_tau_g1, 64);
     memcpy(vk + 64, pw->beta_tau_g1, 64);
+    memcpy(vk + 128, gen, 64);
     memcpy(vk + 192, pw->beta_g2, 128);
+    memcpy(vk + 320, gen + 64, 128);
+    memcpy(vk + 448, gen + 64, 128);
     return ZKR_OK;
 }
 
@@ -427,64 +370,42 @@ extern "C" int zkr_setup_contribute(zkr_ctx* ctx, const void* pk, size_t pk_len,
         return ZKR_E_INVALID;
     }
     // host secrets: delta' then k, both nonzero
-    uint8_t sec[64];
-    int rc = ZKR_OK;
-    if (delta32) memcpy(sec, delta32, 32);
-    else
-        do rc = draw_scalar(sec);
-        while (rc == ZKR_OK && is_zero32(sec));
-    while (rc == ZKR_OK && ((rc = draw_scalar(sec + 32)) == ZKR_OK) && is_zero32(sec + 32)) {}
-    if (rc != ZKR_OK) {
-        wipe(sec, sizeof(sec));
-        return rc;
-    }
+    HostSecret<64> sec;
+    if (delta32) memcpy(sec.b, delta32, 32);
+    else ZKR_TRY(draw_nonzero(sec.b));
+    ZKR_TRY(draw_nonzero(sec.b + 32));
 
     DeviceGuard g(ctx->device);
     cudaStream_t st = ctx->s[0];
     const size_t nch = (size_t)(L.n - L.l - 1) + L.m;          // C | H, contiguous
-    Secrets* d_sec = nullptr;
-    G1Affine *d_ch = nullptr, *d_g1 = nullptr;
-    G2Affine* d_g2 = nullptr;
-    uint8_t small[64 * 2 + 128];                               // delta1_new | R | delta2_new
-    auto field = [&](size_t off) { return (char*)d_sec + off; };
     DevAllocs a;
-    auto run = [&]() -> int {
-        ZKR_TRY(a.alloc(&d_sec, sizeof(Secrets)));
-        ZKR_CUDA(cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st));
-        ZKR_CUDA(cudaMemcpyAsync(d_sec, sec, 64, cudaMemcpyHostToDevice, st));       // delta, k
-        ZKR_TRY(a.alloc(&d_ch, 64 * nch));
-        ZKR_TRY(a.alloc(&d_g1, 128));
-        ZKR_TRY(a.alloc(&d_g2, 128));
-        ZKR_CUDA(cudaMemcpyAsync(d_ch, p + L.pPC, 64 * nch, cudaMemcpyHostToDevice, st));
-        ZKR_CUDA(cudaMemcpyAsync(d_g1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
-        ZKR_CUDA(cudaMemcpyAsync(d_g1 + 1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
-        ZKR_CUDA(cudaMemcpyAsync(d_g2, p + kPkDelta2, 128, cudaMemcpyHostToDevice, st));
-        const int8_t* dig = (const int8_t*)field(offsetof(Secrets, dig));
-        ZKR_LAUNCH(ctx, k_contrib_prep, 1, 1, 0, st, d_sec);
-        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, ceil_div(nch, 128), 128, 0, st, d_ch, nch, dig + kDigits);
-        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, 1, 1, 0, st, d_g1, (size_t)1, dig);
-        ZKR_LAUNCH(ctx, k_fixed_mul<Fq>, 1, 1, 0, st, d_g1 + 1, (size_t)1, dig + 2 * kDigits);
-        ZKR_LAUNCH(ctx, k_fixed_mul<Fq2>, 1, 1, 0, st, d_g2, (size_t)1, dig);
-        ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_pk + L.pPC, d_ch, 64 * nch, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaMemcpyAsync(small, d_g1, 128, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaMemcpyAsync(small + 128, d_g2, 128, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaStreamSynchronize(st));
-        uint8_t c[32];
-        challenge(p + kPkDelta1, small, small + 64, c);
-        ZKR_CUDA(cudaMemcpyAsync(field(offsetof(Secrets, c)), c, 32, cudaMemcpyHostToDevice, st));
-        ZKR_LAUNCH(ctx, k_contrib_z, 1, 1, 0, st, d_sec);
-        ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_record + 64, field(offsetof(Secrets, z)), 32, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st));
-        ZKR_CUDA(cudaStreamSynchronize(st));
-        return ZKR_OK;
-    };
-    rc = run();
-    wipe(sec, sizeof(sec));
-    if (d_sec) {            // on an error path too: the secrets never outlive the call
-        cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st);
-        cudaStreamSynchronize(st);
-    }
-    if (rc != ZKR_OK) return rc;
+    Secrets* d_sec;
+    G1Affine *d_ch, *d_g1;
+    G2Affine* d_g2;
+    ZKR_TRY(a.alloc_secret(&d_sec, sizeof(Secrets), st));
+    ZKR_CUDA(cudaMemcpyAsync(d_sec, sec.b, 64, cudaMemcpyHostToDevice, st));      // delta, k
+    ZKR_TRY(a.upload(&d_ch, p + L.pPC, nch, st));
+    ZKR_TRY(a.alloc(&d_g1, 128));
+    ZKR_CUDA(cudaMemcpyAsync(d_g1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
+    ZKR_CUDA(cudaMemcpyAsync(d_g1 + 1, p + kPkDelta1, 64, cudaMemcpyHostToDevice, st));
+    ZKR_TRY(a.upload(&d_g2, p + kPkDelta2, 1, st));
+    // C | H by delta'^-1; delta1, delta2 by delta'; R = k delta1_old
+    ZKR_LAUNCH(ctx, k_delta_inverse, 1, 1, 0, st, d_sec);
+    ZKR_LAUNCH(ctx, k_scale_points<Fq>, ceil_div(nch, 128), 128, 0, st, d_ch, nch, nullptr, nullptr, &d_sec->dinv);
+    ZKR_LAUNCH(ctx, k_scale_points<Fq>, 1, 1, 0, st, d_g1, (size_t)1, nullptr, nullptr, &d_sec->delta);
+    ZKR_LAUNCH(ctx, k_scale_points<Fq>, 1, 1, 0, st, d_g1 + 1, (size_t)1, nullptr, nullptr, &d_sec->k);
+    ZKR_LAUNCH(ctx, k_scale_points<Fq2>, 1, 1, 0, st, d_g2, (size_t)1, nullptr, nullptr, &d_sec->delta);
+    uint8_t small[64 * 2 + 128];                               // delta1_new | R | delta2_new
+    ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_pk + L.pPC, d_ch, 64 * nch, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaMemcpyAsync(small, d_g1, 128, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaMemcpyAsync(small + 128, d_g2, 128, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    uint8_t c[32];
+    challenge("zkr-phase2-delta", p + kPkDelta1, small, small + 64, c);
+    ZKR_CUDA(cudaMemcpyAsync(&d_sec->c, c, 32, cudaMemcpyHostToDevice, st));
+    ZKR_LAUNCH(ctx, k_schnorr_z, 1, 1, 0, st, &d_sec->delta, &d_sec->k, &d_sec->c, &d_sec->z, 1);
+    ZKR_CUDA(cudaMemcpyAsync((uint8_t*)out_record + 64, &d_sec->z, 32, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
 
     uint8_t* op = (uint8_t*)out_pk;
     uint8_t* ov = (uint8_t*)out_vk;
@@ -529,18 +450,8 @@ extern "C" int zkr_setup_verify_contribution(zkr_ctx* ctx, const void* old_pk, c
     DeviceGuard g(ctx->device);
     cudaStream_t st = ctx->s[0];
     // e(delta1_new, G2) = e(G1, delta2_new)
-    uint8_t gen[64 + 128];
-    {
-        DevAllocs a;
-        G1Affine* d_g1;
-        G2Affine* d_g2;
-        ZKR_TRY(a.alloc(&d_g1, 64));
-        ZKR_TRY(a.alloc(&d_g2, 128));
-        ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_g1, d_g2);
-        ZKR_CUDA(cudaMemcpyAsync(gen, d_g1, 64, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaMemcpyAsync(gen + 64, d_g2, 128, cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaStreamSynchronize(st));
-    }
+    uint8_t gen[192];
+    ZKR_TRY(generators(ctx, st, gen));
     {
         const void* P[2] = {pn + kPkDelta1, gen};
         const void* Q[2] = {gen + 64, pn + kPkDelta2};
@@ -548,50 +459,14 @@ extern "C" int zkr_setup_verify_contribution(zkr_ctx* ctx, const void* old_pk, c
         if (!host_pairing_is_one(P, neg, Q, 2)) return ZKR_OK;
     }
     // z delta1_old = R + c delta1_new
-    {
-        uint8_t pts[192], zc[64];
-        memcpy(pts, po + kPkDelta1, 64);
-        memcpy(pts + 64, pn + kPkDelta1, 64);
-        memcpy(pts + 128, R, 64);
-        memcpy(zc, R + 64, 32);
-        challenge(po + kPkDelta1, pn + kPkDelta1, R, zc + 32);
-        G1Affine* d_pts;
-        Fr* d_zc;
-        int* d_ok;
-        int ok = 0;
-        DevAllocs a;
-        ZKR_TRY(a.alloc(&d_pts, 192));
-        ZKR_TRY(a.alloc(&d_zc, 64));
-        ZKR_TRY(a.alloc(&d_ok, sizeof(int)));
-        ZKR_CUDA(cudaMemcpyAsync(d_pts, pts, 192, cudaMemcpyHostToDevice, st));
-        ZKR_CUDA(cudaMemcpyAsync(d_zc, zc, 64, cudaMemcpyHostToDevice, st));
-        ZKR_LAUNCH(ctx, k_schnorr_check, 1, 1, 0, st, d_pts, d_zc, d_ok);
-        ZKR_CUDA(cudaMemcpyAsync(&ok, d_ok, sizeof(int), cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaStreamSynchronize(st));
-        if (!ok) return ZKR_OK;
-    }
+    bool ok;
+    ZKR_TRY(schnorr_holds(ctx, st, "zkr-phase2-delta", po + kPkDelta1, pn + kPkDelta1, R, R + 64, &ok));
+    if (!ok) return ZKR_OK;
     // every new C / H point in range and on the curve (the MSM formulas do not see the curve constant), and an
     // infinity written as an honest contribution writes it, (0, R mod q): R mod q is the generator's x
     const size_t nch = (size_t)(L.n - L.l - 1) + L.m;
-    {
-        const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, (unsigned)(nch / 4096) + 1}));
-        std::vector<char> good(nt, 1);
-        std::vector<std::thread> th;
-        for (unsigned t = 0; t < nt; t++)
-            th.emplace_back([&, t] {
-                for (size_t i = nch * t / nt; i < nch * (t + 1) / nt; i++) {
-                    const uint8_t* pt = pn + L.pPC + 64 * i;
-                    const int c = host_point_check(1, pt, false);
-                    if (c != PT_OK && (c != PT_INFINITY || memcmp(pt + 32, gen, 32))) {
-                        good[t] = 0;
-                        return;
-                    }
-                }
-            });
-        for (auto& t : th) t.join();
-        for (char ok : good)
-            if (!ok) return ZKR_OK;
-    }
+    int code;
+    if (first_bad_point(1, pn + L.pPC, nch, gen, &code) < nch) return ZKR_OK;
     // e(X_new, delta2_new) = e(X_old, delta2_old), X = sum rho_i C_i + sum sigma_k H_k, 128-bit rho / sigma
     std::vector<uint8_t> sc(32 * nch, 0);
     {

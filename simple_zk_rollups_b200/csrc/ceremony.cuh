@@ -3,7 +3,6 @@
 // that includes it gets its own copy of the kernels and host functions.
 #pragma once
 #include <algorithm>
-#include <cstddef>
 #include <cstring>
 #include <thread>
 #include <vector>
@@ -16,6 +15,8 @@ namespace {
 using namespace zkr;
 
 constexpr int kDigits = 64;            // 4-bit signed windows of a scalar < r < 2^254: the top one never carries out
+constexpr int kTabLog = 14;            // k_scale_points' tables: tau'^k = lo[k mod 2^14] * hi[k >> 14], k < 2^28
+constexpr uint32_t kTab = 1u << kTabLog;
 
 // ------------------------------------------------------------------------------------------------ device
 
@@ -31,17 +32,58 @@ __global__ void k_generators(G1Affine* g1, G2Affine* g2) {
     generator<Fq2>().store(g2);
 }
 
-// digits in [-7, 8], scalar = sum dig[w] 16^w
-__device__ __forceinline__ void recode(const Fr& s, int8_t* dig) {
-    int carry = 0;
-    for (int w = 0; w < kDigits; w++) {
-        int d = (int)((s.v[w >> 3] >> ((w & 7) * 4)) & 15) + carry;
-        carry = d > 8;
-        dig[w] = (int8_t)(d - 16 * carry);
+// pts[k] = s_k pts[k] in place, key encoding in and out, one thread per point.  s_k = lo[k mod 2^14] hi[k >> 14]
+// (Montgomery form; 1 when lo is null) times *c_std (std form; 1 when c_std is null).
+// The scalar's signed 4-bit windows d_w in [-7, 8] are the nibbles of s + 0x77..7 minus 7 (s < r < 2^254, so the sum
+// does not carry out of 256 bits).  They are read from the top by shifting the sum left, so the digits stay in
+// registers; all 64 windows run, as the identity doubles for free.
+template <class F>
+__global__ void k_scale_points(Affine<F>* pts, size_t n, const Fr* __restrict__ lo, const Fr* __restrict__ hi,
+                               const Fr* c_std) {
+    const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    Fr s = lo ? Fr::load_ro(lo + (k & (kTab - 1))) * Fr::load_ro(hi + (k >> kTabLog)) : Fr::one();
+    if (c_std) s = s * Fr::load(c_std).to_mont();
+    s = s.from_mont();
+    uint32_t d[8];
+    uint64_t cy = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        cy += (uint64_t)s.v[i] + 0x77777777u;
+        d[i] = (uint32_t)cy;
+        cy >>= 32;
     }
+    const Affine<F> a = Affine<F>::load(pts + k);
+    XYZZ<F> acc = XYZZ<F>::identity();
+    if (!a.is_inf()) {
+        XYZZ<F> t[8];       // t[j - 1] = j a
+        t[0] = XYZZ<F>::from_affine(a);
+#pragma unroll 1
+        for (int j = 1; j < 8; j++) {
+            t[j] = t[j - 1];
+            t[j].madd(a);
+        }
+#pragma unroll 1
+        for (int w = kDigits - 1; w >= 0; w--) {
+#pragma unroll 1
+            for (int b = 0; b < 4; b++) acc = acc.dbl();
+            const int dg = (int)(d[7] >> 28) - 7;
+#pragma unroll
+            for (int i = 7; i > 0; i--) d[i] = d[i] << 4 | d[i - 1] >> 28;
+            d[0] <<= 4;
+            if (dg > 0) acc.add(t[dg - 1]);
+            else if (dg < 0) acc.add(t[-dg - 1].neg());
+        }
+    }
+    store_key_point(acc, pts + k);
 }
 
-// z * P0 == P2 + c * P1 ?   (P0 = delta1_old, P1 = delta1_new, P2 = R; zc = z | c std form)
+// z[j] = k[j] + c[j] s[j] mod r, std form: the responses of n Schnorr proofs (secret s, nonce k, challenge c)
+__global__ void k_schnorr_z(const Fr* s, const Fr* k, const Fr* c, Fr* z, int n) {
+    for (int j = 0; j < n; j++) z[j] = (k[j].to_mont() + c[j].to_mont() * s[j].to_mont()).from_mont();
+}
+
+// z * P0 == P2 + c * P1 ?   (P0 = P_old, P1 = P_new, P2 = R; zc = z | c std form)
 __global__ void k_schnorr_check(const G1Affine* pts, const Fr* zc, int* ok) {
     const G1XYZZ lhs = scalar_mul(G1XYZZ::from_affine(pts[0]), zc[0]);
     G1XYZZ rhs = scalar_mul(G1XYZZ::from_affine(pts[1]), zc[1]);
@@ -56,33 +98,17 @@ __global__ void k_schnorr_check(const G1Affine* pts, const Fr* zc, int* ok) {
 
 // ------------------------------------------------------------------------------------------------ host
 
-// Device buffers of one call, freed when the call returns, on its error paths too.
-struct DevAllocs {
-    std::vector<void*> p;
-    DevAllocs() = default;
-    DevAllocs(const DevAllocs&) = delete;
-    DevAllocs& operator=(const DevAllocs&) = delete;
-    ~DevAllocs() {
-        for (void* q : p) cudaFree(q);
-    }
-    template <class T>
-    int alloc(T** out, size_t bytes) {
-        ZKR_CUDA(cudaMalloc(out, bytes ? bytes : 1));
-        p.push_back(*out);
-        return ZKR_OK;
-    }
-    void release(void* q) {
-        auto it = std::find(p.begin(), p.end(), q);
-        if (it == p.end()) return;
-        cudaFree(q);
-        p.erase(it);
-    }
-};
-
 void wipe(void* p, size_t n) {
     volatile uint8_t* v = (volatile uint8_t*)p;
     for (size_t i = 0; i < n; i++) v[i] = 0;
 }
+
+// Host copy of a call's secrets, wiped when it goes out of scope, on error paths too
+template <size_t N>
+struct HostSecret {
+    uint8_t b[N];
+    ~HostSecret() { wipe(b, N); }
+};
 
 bool lt_r(const uint8_t* b32) {
     uint32_t v[8];
@@ -95,6 +121,12 @@ bool is_zero32(const uint8_t* b32) {
     uint8_t acc = 0;
     for (int i = 0; i < 32; i++) acc |= b32[i];
     return acc == 0;
+}
+// a uniform scalar in [1, r) from the OS CSPRNG, 32 B std form
+int draw_nonzero(uint8_t* out32) {
+    do ZKR_TRY(draw_scalar(out32));
+    while (is_zero32(out32));
+    return ZKR_OK;
 }
 // b32 -= r while b32 >= r  (a 256-bit value is below 6 r)
 void reduce_r(uint8_t* b32) {
@@ -181,36 +213,99 @@ const char* point_problem(int code) {
         default: return "is not on the curve";
     }
 }
-// count >= need points given (errors name the entry point fn), and the first `used` of them (every point the setup reads) valid
-int check_section(const char* fn, const char* name, int group, const void* pts, uint32_t count, uint32_t need, uint32_t used) {
-    if (count < need || !pts) {
-        set_error("%s: %s has %u points, %u needed", fn, name, pts ? count : 0u, need);
-        return ZKR_E_INVALID;
-    }
-    need = used;
+// The first of the n points at pts (64 B each for group 1, 128 B for group 2) that fails host_point_check without the
+// subgroup test, or n; *code is its PointCheck code.  With inf_y, infinity written as (0, inf_y) passes: the key's
+// encoding, inf_y = R mod q.  Threaded.
+size_t first_bad_point(int group, const void* pts, size_t n, const void* inf_y, int* code) {
     const size_t sz = group == 1 ? 64 : 128;
-    const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, need / 4096 + 1}));
-    std::vector<uint32_t> bad(nt, need);
-    std::vector<int> code(nt, PT_OK);
+    const unsigned nt = std::max(1u, std::min({std::thread::hardware_concurrency(), 16u, (unsigned)(n / 4096) + 1}));
+    std::vector<size_t> bad(nt, n);
+    std::vector<int> cd(nt, PT_OK);
     std::vector<std::thread> th;
     for (unsigned t = 0; t < nt; t++)
         th.emplace_back([&, t] {
-            const uint32_t lo = (uint32_t)((uint64_t)need * t / nt), hi = (uint32_t)((uint64_t)need * (t + 1) / nt);
-            for (uint32_t i = lo; i < hi; i++) {
-                const int c = host_point_check(group, (const uint8_t*)pts + sz * i, false);
-                if (c != PT_OK) {
+            for (size_t i = n * t / nt; i < n * (t + 1) / nt; i++) {
+                const uint8_t* pt = (const uint8_t*)pts + sz * i;
+                const int c = host_point_check(group, pt, false);
+                if (c != PT_OK && !(c == PT_INFINITY && inf_y && !memcmp(pt + sz / 2, inf_y, sz / 2))) {
                     bad[t] = i;
-                    code[t] = c;
+                    cd[t] = c;
                     return;
                 }
             }
         });
     for (auto& t : th) t.join();
     for (unsigned t = 0; t < nt; t++)
-        if (bad[t] < need) {
-            set_error("%s: %s[%u] %s", fn, name, bad[t], point_problem(code[t]));
-            return ZKR_E_INVALID;
+        if (bad[t] < n) {
+            *code = cd[t];
+            return bad[t];
         }
+    *code = PT_OK;
+    return n;
+}
+
+// count >= need points given (errors name the entry point fn), and the first `used` of them (every point the setup reads) valid
+int check_section(const char* fn, const char* name, int group, const void* pts, uint32_t count, uint32_t need, uint32_t used) {
+    if (count < need || !pts) {
+        set_error("%s: %s has %u points, %u needed", fn, name, pts ? count : 0u, need);
+        return ZKR_E_INVALID;
+    }
+    int code;
+    const size_t bad = first_bad_point(group, pts, used, nullptr, &code);
+    if (bad < used) {
+        set_error("%s: %s[%zu] %s", fn, name, bad, point_problem(code));
+        return ZKR_E_INVALID;
+    }
+    return ZKR_OK;
+}
+
+// gen = the G1 and G2 generators in the key encoding, 64 + 128 B
+int generators(zkr_ctx* ctx, cudaStream_t st, uint8_t gen[192]) {
+    DevAllocs a;
+    G1Affine* d_g1;
+    G2Affine* d_g2;
+    ZKR_TRY(a.alloc(&d_g1, 64));
+    ZKR_TRY(a.alloc(&d_g2, 128));
+    ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_g1, d_g2);
+    ZKR_CUDA(cudaMemcpyAsync(gen, d_g1, 64, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaMemcpyAsync(gen + 64, d_g2, 128, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    return ZKR_OK;
+}
+
+// c = SHA-256(tag | P_old | P_new | R) as a little-endian integer mod r: the challenge of a Schnorr proof of knowledge
+// of s for P_new = s P_old (G1, key encoding)
+void challenge(const char* tag, const uint8_t* p_old, const uint8_t* p_new, const uint8_t* R, uint8_t c[32]) {
+    Sha256 s;
+    s.update(tag, strlen(tag));
+    s.update(p_old, 64);
+    s.update(p_new, 64);
+    s.update(R, 64);
+    s.final(c);
+    reduce_r(c);
+}
+
+// *ok = (z P_old == R + c P_new) for the challenge c of (tag, P_old, P_new, R); points checked, z < r
+int schnorr_holds(zkr_ctx* ctx, cudaStream_t st, const char* tag, const uint8_t* p_old, const uint8_t* p_new,
+                  const uint8_t* R, const uint8_t* z, bool* ok) {
+    uint8_t pts[192], zc[64];
+    memcpy(pts, p_old, 64);
+    memcpy(pts + 64, p_new, 64);
+    memcpy(pts + 128, R, 64);
+    memcpy(zc, z, 32);
+    challenge(tag, p_old, p_new, R, zc + 32);
+    DevAllocs a;
+    G1Affine* d_pts;
+    Fr* d_zc;
+    int* d_ok;
+    int flag = 0;
+    ZKR_TRY(a.upload(&d_pts, pts, 3, st));
+    ZKR_TRY(a.upload(&d_zc, zc, 2, st));
+    ZKR_TRY(a.alloc(&d_ok, sizeof(int)));
+    ZKR_LAUNCH(ctx, k_schnorr_check, 1, 1, 0, st, d_pts, d_zc, d_ok);
+    ZKR_CUDA(cudaMemcpyAsync(&flag, d_ok, sizeof(int), cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    *ok = flag != 0;
     return ZKR_OK;
 }
 

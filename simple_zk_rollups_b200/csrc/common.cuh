@@ -104,4 +104,57 @@ struct DeviceGuard {
 
 inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// Device buffers of one call, freed when the call returns, on its error paths too.  A secret buffer is zeroed when it
+// is allocated, and zeroed again on its stream before it is freed, so what it held never outlives the call.
+struct DevAllocs {
+    struct Buf {
+        void* p;
+        size_t wipe;            // bytes zeroed on `st` before the free; 0 for public buffers
+        cudaStream_t st;
+    };
+    std::vector<Buf> bufs;
+
+    DevAllocs() = default;
+    DevAllocs(const DevAllocs&) = delete;
+    DevAllocs& operator=(const DevAllocs&) = delete;
+    ~DevAllocs() {
+        for (const Buf& b : bufs)
+            if (b.wipe) {
+                cudaMemsetAsync(b.p, 0, b.wipe, b.st);
+                cudaStreamSynchronize(b.st);
+            }
+        for (const Buf& b : bufs) cudaFree(b.p);
+    }
+    template <class T>
+    int alloc(T** out, size_t bytes) {
+        ZKR_CUDA(cudaMalloc(out, bytes ? bytes : 1));
+        bufs.push_back({*out, 0, nullptr});
+        return ZKR_OK;
+    }
+    template <class T>
+    int alloc_secret(T** out, size_t bytes, cudaStream_t st) {
+        ZKR_TRY(alloc(out, bytes));
+        bufs.back().wipe = bytes;
+        bufs.back().st = st;
+        ZKR_CUDA(cudaMemsetAsync(*out, 0, bytes, st));
+        return ZKR_OK;
+    }
+    // *d = a new buffer holding the `count` elements of T at host address h
+    template <class T>
+    int upload(T** d, const void* h, size_t count, cudaStream_t st) {
+        ZKR_TRY(alloc(d, sizeof(T) * count));
+        if (count) ZKR_CUDA(cudaMemcpyAsync(*d, h, sizeof(T) * count, cudaMemcpyHostToDevice, st));
+        return ZKR_OK;
+    }
+    // frees a public buffer before the call returns
+    void release(void* q) {
+        for (size_t i = 0; i < bufs.size(); i++)
+            if (bufs[i].p == q) {
+                cudaFree(q);
+                bufs.erase(bufs.begin() + i);
+                return;
+            }
+    }
+};
+
 }  // namespace zkr

@@ -3,8 +3,8 @@
 //
 // The input of zkr_setup_from_powers made and checked here instead of trusted:
 //   * Contribution: one thread per point multiplies it by its own scalar c tau'^k (c = 1, alpha' or beta'), taken from
-//     a two-level table of powers of tau' built once per call, in 4-bit signed windows recoded in registers.  The
-//     record is three Schnorr proofs of knowledge (tau', alpha', beta') with host SHA-256 challenges, as phase 2's.
+//     a two-level table of powers of tau' built once per call (k_scale_points, ceremony.cuh).  The record is three
+//     Schnorr proofs of knowledge (tau', alpha', beta') with host SHA-256 challenges, as phase 2's.
 //   * Verification: one thread per point for range, curve and infinity, and [r]Q = O for G2; then random linear
 //     combinations of consecutive powers by bucketed MSMs (zkr_msm_dev) over slices of at most 2^22 points, and host
 //     pairings (verify.cu).
@@ -14,14 +14,13 @@ using namespace zkr;
 
 namespace {
 
-constexpr int kTabLog = 14;                       // tau'^k = lo[k mod 2^14] * hi[k >> 14], k < 2^28
-constexpr uint32_t kTab = 1u << kTabLog;
 constexpr uint32_t kMaxPowers = 1u << 28;         // 2m G1 powers for the largest domain of zkr_setup_from_powers
 constexpr uint32_t kSlice = 1u << 22;             // MSM bases loaded at a time: bounds the window tables
 const char* const kSecretName[3] = {"tau", "alpha", "beta"};
+const char* const kTag[3] = {"zkr-phase1-tau", "zkr-phase1-alpha", "zkr-phase1-beta"};    // challenge tags
 
 // ------------------------------------------------------------------------------------------------ contribution
-// Device copy of a contribution's secrets and record scalars, std form; zeroed before the call returns.
+// Device copy of a contribution's secrets and record scalars, std form
 struct Secrets {
     Fr s[3];                            // tau', alpha', beta'
     Fr k[3];                            // Schnorr nonces
@@ -48,56 +47,6 @@ __global__ void k_pow_table(const Secrets* s, Fr* lo, Fr* hi) {
     for (int i = 0; i < kTabLog; i++) t14 = t14.sqr();
     pow_small(t, j).store(lo + j);
     pow_small(t14, j).store(hi + j);
-}
-
-// pts[k] = c tau'^k pts[k] in place, key encoding in and out; c = *c_std (std form), or 1 when c_std is null.
-// The scalar's signed 4-bit windows d_w in [-7, 8] are the nibbles of s + 0x77..7 minus 7: the one representation
-// recode() also finds (s < r < 2^254, so the sum does not carry out of 256 bits).  They are read from the top by
-// shifting the sum left, so the digits stay in registers.
-template <class F>
-__global__ void k_powers_mul(Affine<F>* pts, uint32_t n, const Fr* __restrict__ lo, const Fr* __restrict__ hi,
-                             const Fr* c_std) {
-    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n) return;
-    Fr s = Fr::load_ro(lo + (k & (kTab - 1))) * Fr::load_ro(hi + (k >> kTabLog));
-    if (c_std) s = s * Fr::load(c_std).to_mont();
-    s = s.from_mont();
-    uint32_t d[8];
-    uint64_t cy = 0;
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        cy += (uint64_t)s.v[i] + 0x77777777u;
-        d[i] = (uint32_t)cy;
-        cy >>= 32;
-    }
-    const Affine<F> a = Affine<F>::load(pts + k);
-    XYZZ<F> acc = XYZZ<F>::identity();
-    if (!a.is_inf()) {
-        XYZZ<F> t[8];       // t[j - 1] = j a
-        t[0] = XYZZ<F>::from_affine(a);
-#pragma unroll 1
-        for (int j = 1; j < 8; j++) {
-            t[j] = t[j - 1];
-            t[j].madd(a);
-        }
-#pragma unroll 1
-        for (int w = kDigits - 1; w >= 0; w--) {
-#pragma unroll 1
-            for (int b = 0; b < 4; b++) acc = acc.dbl();      // the identity doubles for free
-            const int dg = (int)(d[7] >> 28) - 7;
-#pragma unroll
-            for (int i = 7; i > 0; i--) d[i] = d[i] << 4 | d[i - 1] >> 28;
-            d[0] <<= 4;
-            if (dg > 0) acc.add(t[dg - 1]);
-            else if (dg < 0) acc.add(t[-dg - 1].neg());
-        }
-    }
-    store_key_point(acc, pts + k);
-}
-
-// z = k + c s mod r, for the three secrets
-__global__ void k_powers_z(Secrets* s) {
-    for (int j = 0; j < 3; j++) s->z[j] = (s->k[j].to_mont() + s->c[j].to_mont() * s->s[j].to_mont()).from_mont();
 }
 
 // ------------------------------------------------------------------------------------------------ verification
@@ -208,19 +157,6 @@ int device_point_check(zkr_ctx* ctx, cudaStream_t st, const Section& x, Affine<F
     ZKR_CUDA(cudaStreamSynchronize(st));
     *idx = bad == ~0ull ? x.n : (uint32_t)(bad >> 8);
     *code = (int)(bad & 0xff);
-    return ZKR_OK;
-}
-
-int generators(zkr_ctx* ctx, cudaStream_t st, uint8_t gen[192]) {
-    DevAllocs a;
-    G1Affine* d_g1;
-    G2Affine* d_g2;
-    ZKR_TRY(a.alloc(&d_g1, 64));
-    ZKR_TRY(a.alloc(&d_g2, 128));
-    ZKR_LAUNCH(ctx, k_generators, 1, 1, 0, st, d_g1, d_g2);
-    ZKR_CUDA(cudaMemcpyAsync(gen, d_g1, 64, cudaMemcpyDeviceToHost, st));
-    ZKR_CUDA(cudaMemcpyAsync(gen + 64, d_g2, 128, cudaMemcpyDeviceToHost, st));
-    ZKR_CUDA(cudaStreamSynchronize(st));
     return ZKR_OK;
 }
 
@@ -360,19 +296,6 @@ void schnorr_bases(const zkr_powers* p, uint8_t out[192]) {
     memcpy(out + 128, p->beta_tau_g1, 64);
 }
 
-// c = SHA-256("zkr-phase1-" name | P_old | P_new | R) as a little-endian integer mod r
-void challenge(int j, const uint8_t* p_old, const uint8_t* p_new, const uint8_t* R, uint8_t c[32]) {
-    static const char kTag[] = "zkr-phase1-";
-    Sha256 s;
-    s.update(kTag, sizeof(kTag) - 1);
-    s.update(kSecretName[j], strlen(kSecretName[j]));
-    s.update(p_old, 64);
-    s.update(p_new, 64);
-    s.update(R, 64);
-    s.final(c);
-    reduce_r(c);
-}
-
 }  // namespace
 
 extern "C" int zkr_powers_contribute(zkr_ctx* ctx, const zkr_powers* in, const void* secrets96, void* out_tau_g1,
@@ -393,82 +316,64 @@ extern "C" int zkr_powers_contribute(zkr_ctx* ctx, const zkr_powers* in, const v
         }
     }
     // host secrets: tau', alpha', beta', then the three nonces, all nonzero
-    uint8_t sec[192];
-    int rc = ZKR_OK;
-    if (secrets96) memcpy(sec, secrets96, 96);
-    for (int j = secrets96 ? 3 : 0; j < 6 && rc == ZKR_OK; j++)
-        do rc = draw_scalar(sec + 32 * j);
-        while (rc == ZKR_OK && is_zero32(sec + 32 * j));
-    if (rc != ZKR_OK) {
-        wipe(sec, sizeof(sec));
-        return rc;
-    }
+    HostSecret<192> sec;
+    if (secrets96) memcpy(sec.b, secrets96, 96);
+    for (int j = secrets96 ? 3 : 0; j < 6; j++) ZKR_TRY(draw_nonzero(sec.b + 32 * j));
     uint8_t p_old[192], small[3 * 64];          // Schnorr bases, then R
     schnorr_bases(in, p_old);
 
     DeviceGuard g(ctx->device);
     cudaStream_t st = ctx->s[0];
-    Secrets* d_sec = nullptr;
-    Fr* d_tab = nullptr;                        // lo | hi
-    G1Affine* d_r = nullptr;
-    void* d_pts = nullptr;
-    void* const outs[5] = {out_tau_g1, out_tau_g2, out_alpha_tau_g1, out_beta_tau_g1, out_beta_g2};
-    auto field = [&](size_t off, int j) { return (Fr*)((char*)d_sec + off) + j; };
+    // the secrets, the nonces and the tables of tau'^k are secret buffers; the point buffers hold only public values
+    // (inputs, outputs and R)
     DevAllocs a;
-    auto run = [&]() -> int {
-        ZKR_TRY(a.alloc(&d_sec, sizeof(Secrets)));
-        ZKR_TRY(a.alloc(&d_tab, 2 * sizeof(Fr) * kTab));
-        ZKR_CUDA(cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st));
-        ZKR_CUDA(cudaMemsetAsync(d_tab, 0, 2 * sizeof(Fr) * kTab, st));
-        ZKR_CUDA(cudaMemcpyAsync(d_sec, sec, sizeof(sec), cudaMemcpyHostToDevice, st));      // s[3] | k[3]
-        size_t most = 0;
-        for (const Section& x : s) most = std::max(most, point_bytes(x.group) * x.n);
-        ZKR_TRY(a.alloc(&d_pts, most));
-        ZKR_TRY(a.alloc(&d_r, 3 * sizeof(G1Affine)));
-        const Fr *lo = d_tab, *hi = d_tab + kTab;
-        ZKR_LAUNCH(ctx, k_pow_table, kTab / 128, 128, 0, st, d_sec, d_tab, d_tab + kTab);
-        // tau_g1, tau_g2 by tau'^k; alpha_tau_g1 by alpha' tau'^k; beta_tau_g1 by beta' tau'^k; beta_g2 by beta'
-        const Fr* coef[5] = {nullptr, nullptr, field(offsetof(Secrets, s), 1), field(offsetof(Secrets, s), 2),
-                             field(offsetof(Secrets, s), 2)};
-        for (int i = 0; i < 5; i++) {
-            const Section& x = s[i];
-            const size_t bytes = point_bytes(x.group) * x.n;
-            ZKR_CUDA(cudaMemcpyAsync(d_pts, x.pts, bytes, cudaMemcpyHostToDevice, st));
-            if (x.group == 1)
-                ZKR_LAUNCH(ctx, k_powers_mul<Fq>, ceil_div(x.n, 128), 128, 0, st, (G1Affine*)d_pts, x.n, lo, hi, coef[i]);
-            else
-                ZKR_LAUNCH(ctx, k_powers_mul<Fq2>, ceil_div(x.n, 128), 128, 0, st, (G2Affine*)d_pts, x.n, lo, hi, coef[i]);
-            ZKR_CUDA(cudaMemcpyAsync(outs[i], d_pts, bytes, cudaMemcpyDeviceToHost, st));
-            ZKR_CUDA(cudaStreamSynchronize(st));
-        }
-        // R_j = k_j P_old_j (lo[0] hi[0] = 1)
-        ZKR_CUDA(cudaMemcpyAsync(d_r, p_old, sizeof(p_old), cudaMemcpyHostToDevice, st));
-        for (int j = 0; j < 3; j++) ZKR_LAUNCH(ctx, k_powers_mul<Fq>, 1, 1, 0, st, d_r + j, 1u, lo, hi, field(offsetof(Secrets, k), j));
-        ZKR_CUDA(cudaMemcpyAsync(small, d_r, sizeof(small), cudaMemcpyDeviceToHost, st));
+    Secrets* d_sec;
+    Fr* d_tab;                                  // lo | hi
+    G1Affine* d_r;
+    void* d_pts;
+    ZKR_TRY(a.alloc_secret(&d_sec, sizeof(Secrets), st));
+    ZKR_TRY(a.alloc_secret(&d_tab, 2 * sizeof(Fr) * kTab, st));
+    ZKR_CUDA(cudaMemcpyAsync(d_sec, sec.b, sizeof(sec.b), cudaMemcpyHostToDevice, st));      // s[3] | k[3]
+    size_t most = 0;
+    for (const Section& x : s) most = std::max(most, point_bytes(x.group) * x.n);
+    ZKR_TRY(a.alloc(&d_pts, most));
+    ZKR_TRY(a.alloc(&d_r, 3 * sizeof(G1Affine)));
+    const Fr *lo = d_tab, *hi = d_tab + kTab;
+    ZKR_LAUNCH(ctx, k_pow_table, kTab / 128, 128, 0, st, d_sec, d_tab, d_tab + kTab);
+    // tau_g1, tau_g2 by tau'^k; alpha_tau_g1 by alpha' tau'^k; beta_tau_g1 by beta' tau'^k; beta_g2 by beta'
+    void* const outs[5] = {out_tau_g1, out_tau_g2, out_alpha_tau_g1, out_beta_tau_g1, out_beta_g2};
+    const Fr* coef[5] = {nullptr, nullptr, d_sec->s + 1, d_sec->s + 2, d_sec->s + 2};
+    for (int i = 0; i < 5; i++) {
+        const Section& x = s[i];
+        const size_t bytes = point_bytes(x.group) * x.n;
+        ZKR_CUDA(cudaMemcpyAsync(d_pts, x.pts, bytes, cudaMemcpyHostToDevice, st));
+        if (x.group == 1)
+            ZKR_LAUNCH(ctx, k_scale_points<Fq>, ceil_div(x.n, 128), 128, 0, st, (G1Affine*)d_pts, x.n, lo, hi, coef[i]);
+        else
+            ZKR_LAUNCH(ctx, k_scale_points<Fq2>, ceil_div(x.n, 128), 128, 0, st, (G2Affine*)d_pts, x.n, lo, hi, coef[i]);
+        ZKR_CUDA(cudaMemcpyAsync(outs[i], d_pts, bytes, cudaMemcpyDeviceToHost, st));
         ZKR_CUDA(cudaStreamSynchronize(st));
-        uint8_t p_new[192], c[96];
-        memcpy(p_new, (const uint8_t*)out_tau_g1 + 64, 64);
-        memcpy(p_new + 64, out_alpha_tau_g1, 64);
-        memcpy(p_new + 128, out_beta_tau_g1, 64);
-        for (int j = 0; j < 3; j++) challenge(j, p_old + 64 * j, p_new + 64 * j, small + 64 * j, c + 32 * j);
-        ZKR_CUDA(cudaMemcpyAsync(field(offsetof(Secrets, c), 0), c, sizeof(c), cudaMemcpyHostToDevice, st));
-        ZKR_LAUNCH(ctx, k_powers_z, 1, 1, 0, st, d_sec);
-        uint8_t* rec = (uint8_t*)out_record;
-        for (int j = 0; j < 3; j++) {
-            memcpy(rec + 96 * j, small + 64 * j, 64);
-            ZKR_CUDA(cudaMemcpyAsync(rec + 96 * j + 64, field(offsetof(Secrets, z), j), 32, cudaMemcpyDeviceToHost, st));
-        }
-        ZKR_CUDA(cudaStreamSynchronize(st));
-        return ZKR_OK;
-    };
-    rc = run();
-    wipe(sec, sizeof(sec));
-    // on an error path too: the secrets, the tables of tau'^k and the nonces never outlive the call.  The point
-    // buffers hold only public values (inputs, outputs and R).
-    if (d_sec) cudaMemsetAsync(d_sec, 0, sizeof(Secrets), st);
-    if (d_tab) cudaMemsetAsync(d_tab, 0, 2 * sizeof(Fr) * kTab, st);
-    cudaStreamSynchronize(st);
-    return rc;
+    }
+    // R_j = k_j P_old_j
+    ZKR_CUDA(cudaMemcpyAsync(d_r, p_old, sizeof(p_old), cudaMemcpyHostToDevice, st));
+    for (int j = 0; j < 3; j++)
+        ZKR_LAUNCH(ctx, k_scale_points<Fq>, 1, 1, 0, st, d_r + j, (size_t)1, nullptr, nullptr, d_sec->k + j);
+    ZKR_CUDA(cudaMemcpyAsync(small, d_r, sizeof(small), cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    uint8_t p_new[192], c[96];
+    memcpy(p_new, (const uint8_t*)out_tau_g1 + 64, 64);
+    memcpy(p_new + 64, out_alpha_tau_g1, 64);
+    memcpy(p_new + 128, out_beta_tau_g1, 64);
+    for (int j = 0; j < 3; j++) challenge(kTag[j], p_old + 64 * j, p_new + 64 * j, small + 64 * j, c + 32 * j);
+    ZKR_CUDA(cudaMemcpyAsync(d_sec->c, c, sizeof(c), cudaMemcpyHostToDevice, st));
+    ZKR_LAUNCH(ctx, k_schnorr_z, 1, 1, 0, st, d_sec->s, d_sec->k, d_sec->c, d_sec->z, 3);
+    uint8_t* rec = (uint8_t*)out_record;
+    for (int j = 0; j < 3; j++) {
+        memcpy(rec + 96 * j, small + 64 * j, 64);
+        ZKR_CUDA(cudaMemcpyAsync(rec + 96 * j + 64, d_sec->z + j, 32, cudaMemcpyDeviceToHost, st));
+    }
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    return ZKR_OK;
 }
 
 extern "C" int zkr_powers_verify(zkr_ctx* ctx, const zkr_powers* p, int* valid) {
@@ -517,34 +422,15 @@ extern "C" int zkr_powers_verify_contribution(zkr_ctx* ctx, const zkr_powers* ol
     // z P_old = R + c P_new, for tau, alpha, beta
     {
         DeviceGuard g(ctx->device);
-        cudaStream_t st = ctx->s[0];
-        DevAllocs a;
-        G1Affine* d_pts;
-        Fr* d_zc;
-        int* d_ok;
-        int ok[3] = {0, 0, 0};
-        ZKR_TRY(a.alloc(&d_pts, 3 * 192));
-        ZKR_TRY(a.alloc(&d_zc, 3 * 64));
-        ZKR_TRY(a.alloc(&d_ok, sizeof(ok)));
         for (int j = 0; j < 3; j++) {
-            uint8_t pts[192], zc[64];
-            memcpy(pts, p_old + 64 * j, 64);
-            memcpy(pts + 64, p_new + 64 * j, 64);
-            memcpy(pts + 128, rec + 96 * j, 64);
-            memcpy(zc, rec + 96 * j + 64, 32);
-            challenge(j, p_old + 64 * j, p_new + 64 * j, rec + 96 * j, zc + 32);
-            ZKR_CUDA(cudaMemcpyAsync(d_pts + 3 * j, pts, 192, cudaMemcpyHostToDevice, st));
-            ZKR_CUDA(cudaMemcpyAsync(d_zc + 2 * j, zc, 64, cudaMemcpyHostToDevice, st));
-            ZKR_CUDA(cudaStreamSynchronize(st));             // pts / zc are reused by the next j
-            ZKR_LAUNCH(ctx, k_schnorr_check, 1, 1, 0, st, d_pts + 3 * j, d_zc + 2 * j, d_ok + j);
-        }
-        ZKR_CUDA(cudaMemcpyAsync(ok, d_ok, sizeof(ok), cudaMemcpyDeviceToHost, st));
-        ZKR_CUDA(cudaStreamSynchronize(st));
-        for (int j = 0; j < 3; j++)
-            if (!ok[j]) {
+            bool ok;
+            const uint8_t* R = rec + 96 * j;
+            ZKR_TRY(schnorr_holds(ctx, ctx->s[0], kTag[j], p_old + 64 * j, p_new + 64 * j, R, R + 64, &ok));
+            if (!ok) {
                 set_error("%s: the %s proof of knowledge does not hold", kFn, kSecretName[j]);
                 return ZKR_OK;
             }
+        }
     }
     return verify_powers(ctx, kFn, new_p, valid);
 }

@@ -142,31 +142,26 @@ __global__ void k_setup_scalars(const Fr* at, const Fr* bt, const Fr* ct, const 
 template <class F>
 int fixed_base(zkr_ctx* ctx, cudaStream_t st, Affine<F>* table, const Fr* d_scalars, uint32_t n, void* h_out) {
     if (n == 0) return ZKR_OK;
+    DevAllocs a;
     Affine<F>* d_out;
-    ZKR_CUDA(cudaMalloc(&d_out, sizeof(Affine<F>) * (size_t)n));
+    ZKR_TRY(a.alloc(&d_out, sizeof(Affine<F>) * (size_t)n));
     ZKR_LAUNCH(ctx, k_fb_mul<F>, ceil_div(n, 64), 64, 0, st, d_scalars, table, d_out, n);
     ZKR_CUDA(cudaMemcpyAsync(h_out, d_out, sizeof(Affine<F>) * (size_t)n, cudaMemcpyDeviceToHost, st));
     ZKR_CUDA(cudaStreamSynchronize(st));
-    ZKR_CUDA(cudaFree(d_out));
     return ZKR_OK;
 }
 
+// *table = the fixed-base table of the generator, owned by `owner`
 template <class F>
-int build_table(zkr_ctx* ctx, cudaStream_t st, Affine<F>** table) {
+int build_table(zkr_ctx* ctx, cudaStream_t st, DevAllocs& owner, Affine<F>** table) {
+    DevAllocs a;
     Affine<F>* base;
-    ZKR_CUDA(cudaMalloc(&base, sizeof(Affine<F>) * kFbWin));
-    ZKR_CUDA(cudaMalloc(table, sizeof(Affine<F>) * kFbWin * 256));
+    ZKR_TRY(a.alloc(&base, sizeof(Affine<F>) * kFbWin));
+    ZKR_TRY(owner.alloc(table, sizeof(Affine<F>) * kFbWin * 256));
     ZKR_CUDA(cudaMemsetAsync(*table, 0, sizeof(Affine<F>) * kFbWin * 256, st));
     ZKR_LAUNCH(ctx, k_fb_base<F>, 1, 1, 0, st, base);
     ZKR_LAUNCH(ctx, k_fb_table<F>, kFbWin, 256, 0, st, (const Affine<F>*)base, *table);
     ZKR_CUDA(cudaStreamSynchronize(st));
-    ZKR_CUDA(cudaFree(base));
-    return ZKR_OK;
-}
-
-int up32(const uint32_t* h, size_t count, uint32_t** d, cudaStream_t st) {
-    ZKR_CUDA(cudaMalloc(d, 4 * (count ? count : 1)));
-    if (count) ZKR_CUDA(cudaMemcpyAsync(*d, h, 4 * count, cudaMemcpyHostToDevice, st));
     return ZKR_OK;
 }
 
@@ -188,23 +183,22 @@ extern "C" int zkr_synth_setup(zkr_ctx* ctx, const zkr_r1cs_csc* r, const void* 
     ZKR_TRY(ntt_get_tables(ctx, log_m, &tabs));
     const NttTables* tv = tabs;
 
+    DevAllocs a;
     Fr *d_tox_in, *d_pool, *d_L, *d_at, *d_bt, *d_ct, *sA, *sB, *sC, *sIC, *sH, *sVK;
     Toxic* d_tox;
-    ZKR_CUDA(cudaMalloc(&d_tox_in, 5 * 32));
-    ZKR_CUDA(cudaMalloc(&d_tox, sizeof(Toxic)));
-    ZKR_CUDA(cudaMalloc(&d_pool, 32 * (size_t)(r->n_pool ? r->n_pool : 1)));
-    ZKR_CUDA(cudaMalloc(&d_L, 32 * (size_t)m));
-    ZKR_CUDA(cudaMalloc(&d_at, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&d_bt, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&d_ct, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&sA, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&sB, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&sC, 32 * (size_t)n));
-    ZKR_CUDA(cudaMalloc(&sIC, 32 * (size_t)(l + 1)));
-    ZKR_CUDA(cudaMalloc(&sH, 32 * (size_t)m));
-    ZKR_CUDA(cudaMalloc(&sVK, 32 * 4));
-    ZKR_CUDA(cudaMemcpyAsync(d_tox_in, toxic, 5 * 32, cudaMemcpyHostToDevice, st));
-    ZKR_CUDA(cudaMemcpyAsync(d_pool, r->pool, 32 * (size_t)r->n_pool, cudaMemcpyHostToDevice, st));
+    ZKR_TRY(a.upload(&d_tox_in, toxic, 5, st));
+    ZKR_TRY(a.alloc(&d_tox, sizeof(Toxic)));
+    ZKR_TRY(a.upload(&d_pool, r->pool, r->n_pool, st));
+    ZKR_TRY(a.alloc(&d_L, 32 * (size_t)m));
+    ZKR_TRY(a.alloc(&d_at, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&d_bt, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&d_ct, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&sA, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&sB, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&sC, 32 * (size_t)n));
+    ZKR_TRY(a.alloc(&sIC, 32 * (size_t)(l + 1)));
+    ZKR_TRY(a.alloc(&sH, 32 * (size_t)m));
+    ZKR_TRY(a.alloc(&sVK, 32 * 4));
     ZKR_LAUNCH(ctx, k_to_mont, ceil_div(r->n_pool, 128), 128, 0, st, d_pool, r->n_pool);
     ZKR_LAUNCH(ctx, k_toxic, 1, 1, 0, st, d_tox_in, d_tox, m);
     ZKR_LAUNCH(ctx, k_lagrange, ceil_div(m, 128), 128, 0, st, d_L, m, d_tox, tv->tw_lo_f, tv->tw_hi_f, tv->lb);
@@ -212,23 +206,21 @@ extern "C" int zkr_synth_setup(zkr_ctx* ctx, const zkr_r1cs_csc* r, const void* 
     Fr* outs[3] = {d_at, d_bt, d_ct};
     for (int k = 0; k < 3; k++) {
         const uint32_t nnz = hp[k][0][n];
+        DevAllocs cols;
         uint32_t *dp, *dr, *dc;
-        ZKR_TRY(up32(hp[k][0], (size_t)n + 1, &dp, st));
-        ZKR_TRY(up32(hp[k][1], nnz, &dr, st));
-        ZKR_TRY(up32(hp[k][2], nnz, &dc, st));
+        ZKR_TRY(cols.upload(&dp, hp[k][0], (size_t)n + 1, st));
+        ZKR_TRY(cols.upload(&dr, hp[k][1], nnz, st));
+        ZKR_TRY(cols.upload(&dc, hp[k][2], nnz, st));
         ZKR_LAUNCH(ctx, k_col_eval, ceil_div(n, 128), 128, 0, st, dp, dr, dc, d_pool, d_L, outs[k], n);
         ZKR_CUDA(cudaStreamSynchronize(st));
-        cudaFree(dp);
-        cudaFree(dr);
-        cudaFree(dc);
     }
     const uint32_t top = n > m ? n : m;
     ZKR_LAUNCH(ctx, k_setup_scalars, ceil_div(top, 128), 128, 0, st, d_at, d_bt, d_ct, d_tox, n, l, m, sA, sB, sC, sIC,
                sH, sVK);
     G1Affine* t1;
     G2Affine* t2;
-    ZKR_TRY(build_table<Fq>(ctx, st, &t1));
-    ZKR_TRY(build_table<Fq2>(ctx, st, &t2));
+    ZKR_TRY(build_table<Fq>(ctx, st, a, &t1));
+    ZKR_TRY(build_table<Fq2>(ctx, st, a, &t2));
     char* vk = (char*)out_vk;
     ZKR_TRY(fixed_base<Fq>(ctx, st, t1, sA, n, out_a));
     ZKR_TRY(fixed_base<Fq>(ctx, st, t1, sB, n, out_b1));
@@ -241,8 +233,6 @@ extern "C" int zkr_synth_setup(zkr_ctx* ctx, const zkr_r1cs_csc* r, const void* 
     ZKR_TRY(fixed_base<Fq2>(ctx, st, t2, sVK + 3, 1, vk + 192 + 128));    // gamma2
     ZKR_TRY(fixed_base<Fq2>(ctx, st, t2, sVK + 2, 1, vk + 192 + 256));    // delta2
     ZKR_TRY(fixed_base<Fq>(ctx, st, t1, sIC, l + 1, vk + 192 + 384));
-    void* fr[] = {d_tox_in, d_tox, d_pool, d_L, d_at, d_bt, d_ct, sA, sB, sC, sIC, sH, sVK, t1, t2};
-    for (void* p : fr) cudaFree(p);
     return ZKR_OK;
 }
 
@@ -251,21 +241,15 @@ extern "C" int zkr_synth_points(zkr_ctx* ctx, int group, const void* scalars, si
     if (!ctx || !scalars || !out_points || (group != 1 && group != 2) || n == 0 || n > 0xffffffffull) return ZKR_E_INVALID;
     DeviceGuard g(ctx->device);
     cudaStream_t st = ctx->s[0];
+    DevAllocs a;
     Fr* d_sc;
-    ZKR_CUDA(cudaMalloc(&d_sc, 32 * n));
-    ZKR_CUDA(cudaMemcpyAsync(d_sc, scalars, 32 * n, cudaMemcpyHostToDevice, st));
-    int rc;
+    ZKR_TRY(a.upload(&d_sc, scalars, n, st));
     if (group == 1) {
         G1Affine* t;
-        ZKR_TRY(build_table<Fq>(ctx, st, &t));
-        rc = fixed_base<Fq>(ctx, st, t, d_sc, (uint32_t)n, out_points);
-        cudaFree(t);
-    } else {
-        G2Affine* t;
-        ZKR_TRY(build_table<Fq2>(ctx, st, &t));
-        rc = fixed_base<Fq2>(ctx, st, t, d_sc, (uint32_t)n, out_points);
-        cudaFree(t);
+        ZKR_TRY(build_table<Fq>(ctx, st, a, &t));
+        return fixed_base<Fq>(ctx, st, t, d_sc, (uint32_t)n, out_points);
     }
-    cudaFree(d_sc);
-    return rc;
+    G2Affine* t;
+    ZKR_TRY(build_table<Fq2>(ctx, st, a, &t));
+    return fixed_base<Fq2>(ctx, st, t, d_sc, (uint32_t)n, out_points);
 }
