@@ -12,6 +12,7 @@
  *                                                             operator/src/snarks/common.ts:29
  *                             witnessBin = binarifyWitness()  operator/src/utils/binarify.ts:10-48
  *   zkr_prove_batch       <-> many independent genTxVerifierProof calls (tx.ts:6-10), one per GPU
+ *   zkr_prove_many        <-> the same calls for one small circuit, all in one pass on one GPU
  *   zkr_msm_* / zkr_ntt   <-> websnark g1_multiexp / g2_multiexp / fft_* (inside groth16GenProof);
  *                             exported for the standalone sweeps of BASELINE.json configs[2..3]
  *   zkr_synth_setup       <-> `snarkjs setup --protocol groth`  prover/package.json:34,37
@@ -156,6 +157,29 @@ int zkr_prove_batch(zkr_ctx* const* ctxs, const zkr_pkey* const* pks, int n_ctx,
                     const void* const* witnesses, size_t n_signals, int n_proofs,
                     const void* rs32 /* n_proofs x 64 B (r|s), or NULL = fresh CSPRNG pairs */, void* out_proofs);
 
+/* ---- many proofs of one small circuit in one pass (DESIGN.md 4.10) ----------------------------------------------
+ * A circuit of a few thousand constraints leaves most of a B200 idle and one proof is a chain of ~50 small launches.
+ * zkr_prove_many runs every stage once for a whole batch of witnesses of one key: the number of kernel launches does
+ * not depend on n_proofs, each launch does the work of all of them.
+ * zkr_many_create: device work buffers for proving up to max_proofs witnesses of one key in one pass.  Bound to pk and
+ * to pk's ctx; the key's tables are shared, not copied (free the workspace before the key).  ZKR_E_UNSUPPORTED for a
+ * sharded key (world > 1), a domain smaller than 8, max_proofs > 32767, or when a batch of max_proofs would exceed the
+ * MSM's limits (k x W x n entries >= 2^31 for a base set, sort keys wider than 31 bits), with the limit named;
+ * ZKR_E_NOMEM when the buffers do not fit.  zkr_many_info: max_proofs and the device bytes of the buffers. */
+typedef struct zkr_many zkr_many;
+int zkr_many_create(zkr_ctx* ctx, const zkr_pkey* pk, int max_proofs, zkr_many** out);
+void zkr_many_free(zkr_many* mw);
+int zkr_many_info(const zkr_many* mw, int* max_proofs, uint64_t* device_bytes);
+/* n_proofs (1..max_proofs) proofs of the key: witnesses = n_proofs x n_signals x 32 B std form, HOST memory, contiguous;
+ * rs32 = n_proofs x 64 B (r|s) or NULL (fresh CSPRNG pairs, as zkr_prove_batch); out_proofs = n_proofs x 256 B.
+ * Proof j is byte-identical to zkr_prove(ctx, pk, witness_j, n_signals, r_j, s_j).  Every stage runs once for the whole
+ * batch: the number of kernel launches does not depend on n_proofs (for keys whose MSM windows are at most 20 bits,
+ * i.e. every key below ~2^23 signals).  A witness value >= r or witness[0] != 1 in any proof -> ZKR_E_WITNESS_RANGE
+ * naming the first such proof index (no proofs are returned); the workspace is clean for the next call.  n_proofs out of
+ * range, n_signals != the key's nVars, or an r or s >= r (the proof index is named) -> ZKR_E_INVALID.  Blocking. */
+int zkr_prove_many(zkr_ctx* ctx, zkr_many* mw, const void* witnesses, size_t n_signals, int n_proofs,
+                   const void* rs32, void* out_proofs);
+
 /* ---- witness generation for forward-solvable constraint systems (SURVEY.md 8(f) rank 4) ---------
  * Stands where the reference calls circom's generated calculator, circuit.calculateWitness(inputs)
  * (operator/src/snarks/common.ts:12-17), for circuits whose constraints each introduce at most one new
@@ -223,6 +247,13 @@ int zkr_msm(zkr_ctx* ctx, const zkr_bases* b, const void* scalars, size_t n, int
 /* device-resident, asynchronous variant: result stays on the device as an XYZZ point
  * (4 coordinates Fq-M / Fq2-M: 128 B for G1, 256 B for G2). */
 int zkr_msm_dev(zkr_ctx* ctx, const zkr_bases* b, const void* d_scalars, size_t n, void* d_out_xyzz);
+/* n_vectors MSMs over one base set in one pass: scalars = n_vectors x n x 32 B std form (host, or device if
+ * scalars_on_device); out_affine = n_vectors results, each as zkr_msm writes it.  Result j == zkr_msm(ctx, b,
+ * scalars_j, ...).  The batch's work buffers are kept with the bases: allocated on the first call, re-allocated when a
+ * larger n_vectors comes, freed by zkr_bases_free; zkr_bases_info's device_bytes includes them.  Limits as
+ * zkr_many_create (ZKR_E_UNSUPPORTED, limit named); a scalar >= r -> ZKR_E_WITNESS_RANGE naming the first such vector. */
+int zkr_msm_many(zkr_ctx* ctx, const zkr_bases* b, const void* scalars, size_t n, int n_vectors,
+                 int scalars_on_device, void* out_affine);
 
 /* ---- standalone NTT over Fr ----------------------------------------------------------- */
 #define ZKR_NTT_FORWARD 0       /* evaluations on <omega_n>, natural order in and out          */

@@ -84,6 +84,11 @@ _SIGS = {
     "zkr_witness_solve": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zkr_prove_batch": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int,
                                   C.POINTER(C.c_void_p), C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]),
+    "zkr_many_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "zkr_many_free": (None, [C.c_void_p]),
+    "zkr_many_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_uint64)]),
+    "zkr_prove_many": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]),
+    "zkr_msm_many": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p]),
     "zkr_bases_load": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.POINTER(C.c_void_p)]),
     "zkr_bases_free": (None, [C.c_void_p]),
     "zkr_bases_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_int), C.POINTER(C.c_int),

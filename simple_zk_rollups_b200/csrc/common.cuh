@@ -50,6 +50,9 @@ struct DevBuf {
 };
 
 constexpr int kNumStreams = 6;      // s[0..4]: the proof's five chains, s[5]: witness uploads
+// Vectors of one batched call (zkr_prove_many, zkr_msm_many): the batched H pipeline puts 2 k transforms on one grid's
+// y dimension (<= 65535)
+constexpr int kMaxBatch = 32767;
 
 // Per-kernel device timing for bench.py's roofline: rings of CUDA event pairs recorded on the
 // launching stream around selected kernels while profiling is enabled.

@@ -31,6 +31,7 @@
 
 #include "common.cuh"
 #include "ec.cuh"
+#include "msm_iface.cuh"
 
 namespace zkr {
 
@@ -89,15 +90,9 @@ __global__ void k_precompute(const char* __restrict__ pts, char* __restrict__ ta
     }
 }
 
-// keys[w n + i] = |digit| - 1 (or sentinel for 0), vals[w n + i] = (w n + i) | sign
-static __global__ void k_digits(const uint32_t* __restrict__ scalars, const uint32_t* __restrict__ src_index, uint32_t n,
-                         int c, int W, uint32_t sentinel, uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
-                         int* __restrict__ range_err) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const uint32_t* sp = scalars + 8 * (size_t)(src_index ? src_index[i] : i);
-    Fr k = Fr::load_ro(sp);
-    if (!k.in_range()) *range_err = 1;
+// keys[w n + i] = kofs + |digit| - 1 (or sentinel for 0), vals[w n + i] = (w n + i) | sign
+__device__ __forceinline__ void scalar_digits(const Fr& k, uint32_t i, uint32_t n, int c, int W, uint32_t kofs,
+                                              uint32_t sentinel, uint32_t* __restrict__ keys, uint32_t* __restrict__ vals) {
     uint32_t carry = 0;
     const uint32_t half = 1u << (c - 1), mask = (1u << c) - 1;
     for (int w = 0; w < W; w++) {
@@ -117,9 +112,34 @@ static __global__ void k_digits(const uint32_t* __restrict__ scalars, const uint
         }
         uint32_t pos = (uint32_t)w * n + i;
         // a zero digit gets the sentinel key: it sorts behind every bucket and the accumulation never visits it (see kNegBit)
-        keys[pos] = d ? d - 1 : sentinel;
+        keys[pos] = d ? kofs + d - 1 : sentinel;
         vals[pos] = pos | neg;
     }
+}
+
+static __global__ void k_digits(const uint32_t* __restrict__ scalars, const uint32_t* __restrict__ src_index, uint32_t n,
+                         int c, int W, uint32_t sentinel, uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
+                         int* __restrict__ range_err) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t* sp = scalars + 8 * (size_t)(src_index ? src_index[i] : i);
+    Fr k = Fr::load_ro(sp);
+    if (!k.in_range()) *range_err = 1;
+    scalar_digits(k, i, n, c, W, 0, sentinel, keys, vals);
+}
+
+// Batched form (msm_run_many): vector j = blockIdx.y is read at scalars + 8 stride j and owns the entries
+// [j W n, (j+1) W n) and the buckets [j nb, (j+1) nb); the table reference in vals is the same for every vector.
+static __global__ void k_digits_many(const uint32_t* __restrict__ scalars, size_t stride, const uint32_t* __restrict__ src_index,
+                                     uint32_t n, int c, int W, uint32_t nb, uint32_t sentinel, uint32_t* __restrict__ keys,
+                                     uint32_t* __restrict__ vals, int* __restrict__ range_err) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
+    if (i >= n) return;
+    const uint32_t* sp = scalars + 8 * (stride * j + (src_index ? src_index[i] : i));
+    Fr k = Fr::load_ro(sp);
+    if (!k.in_range()) range_err[j] = 1;
+    const size_t base = (size_t)j * W * n;
+    scalar_digits(k, i, n, c, W, j * nb, sentinel, keys + base, vals + base);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -493,8 +513,7 @@ constexpr int kReduceThreads = 32;
 
 // stage 1: CTA g < 2^lr: Row[g];  CTA 2^lr + l: Col[l]
 template <class F, int NT>
-__global__ void __launch_bounds__(NT)
-k_bucket_sums(const XYZZ<F>* __restrict__ buckets, int lr, int lc, XYZZ<F>* __restrict__ out) {
+__device__ __forceinline__ void bucket_sums(const XYZZ<F>* __restrict__ buckets, int lr, int lc, XYZZ<F>* __restrict__ out) {
     extern __shared__ unsigned char smraw[];
     XYZZ<F>* s0 = reinterpret_cast<XYZZ<F>*>(smraw);
     const uint32_t t = threadIdx.x, g = blockIdx.x;
@@ -509,12 +528,23 @@ k_bucket_sums(const XYZZ<F>* __restrict__ buckets, int lr, int lc, XYZZ<F>* __re
     block_sum_inplace<F, NT>(s0);
     if (t == 0) out[g] = s0[0];
 }
+template <class F, int NT>
+__global__ void __launch_bounds__(NT)
+k_bucket_sums(const XYZZ<F>* __restrict__ buckets, int lr, int lc, XYZZ<F>* __restrict__ out) {
+    bucket_sums<F, NT>(buckets, lr, lc, out);
+}
+// batched: vector blockIdx.y reduces its own nb buckets into its own nred-entry segment of the scratch
+template <class F, int NT>
+__global__ void __launch_bounds__(NT)
+k_bucket_sums_many(const XYZZ<F>* __restrict__ buckets, uint32_t nb, int lr, int lc, XYZZ<F>* __restrict__ red, uint32_t nred) {
+    bucket_sums<F, NT>(buckets + (size_t)blockIdx.y * nb, lr, lc, red + (size_t)blockIdx.y * nred);
+}
 
 // stage 2: CTA j < lr: 2^(j+lc) * sum_{hi: bit j} Row[hi];  CTA lr + j, j < lc: 2^j * sum_{lo: bit j} Col[lo];
 //          CTA lr + lc: sum_hi Row[hi].  terms -> sums[2^lr + 2^lc ..]; the last CTA adds them into *out.
 template <class F, int NT>
-__global__ void __launch_bounds__(NT)
-k_bucket_weighted(XYZZ<F>* __restrict__ sums, int lr, int lc, unsigned int* __restrict__ counter, XYZZ<F>* __restrict__ out) {
+__device__ __forceinline__ void bucket_weighted(XYZZ<F>* __restrict__ sums, int lr, int lc, unsigned int* __restrict__ counter,
+                                                XYZZ<F>* __restrict__ out) {
     extern __shared__ unsigned char smraw[];
     XYZZ<F>* s0 = reinterpret_cast<XYZZ<F>*>(smraw);
     __shared__ bool last;
@@ -556,14 +586,36 @@ k_bucket_weighted(XYZZ<F>* __restrict__ sums, int lr, int lc, unsigned int* __re
         *counter = 0;
     }
 }
+template <class F, int NT>
+__global__ void __launch_bounds__(NT)
+k_bucket_weighted(XYZZ<F>* __restrict__ sums, int lr, int lc, unsigned int* __restrict__ counter, XYZZ<F>* __restrict__ out) {
+    bucket_weighted<F, NT>(sums, lr, lc, counter, out);
+}
+// batched: vector blockIdx.y has its own scratch segment and completion counter, and writes its result at out + y out_stride
+template <class F, int NT>
+__global__ void __launch_bounds__(NT)
+k_bucket_weighted_many(XYZZ<F>* __restrict__ red, uint32_t nred, int lr, int lc, unsigned int* __restrict__ counters,
+                       char* __restrict__ out, size_t out_stride) {
+    const uint32_t j = blockIdx.y;
+    bucket_weighted<F, NT>(red + (size_t)j * nred, lr, lc, counters + j, reinterpret_cast<XYZZ<F>*>(out + j * out_stride));
+}
 
 // XYZZ (Montgomery) -> affine standard form bytes; identity -> zeros.  One thread at the tail of a standalone MSM:
 // the variable-time inversion (fp_inv.cuh) is the whole kernel.
 template <class F>
-__global__ void k_xyzz_to_affine_std(const XYZZ<F>* in, char* out) {
+__device__ __forceinline__ void xyzz_to_affine_std(const XYZZ<F>* in, char* out) {
     Affine<F> a = XYZZ<F>::load(in).to_affine_vartime();
     a.x.from_mont().store(out);
     a.y.from_mont().store(out + sizeof(F));
+}
+template <class F>
+__global__ void k_xyzz_to_affine_std(const XYZZ<F>* in, char* out) {
+    xyzz_to_affine_std(in, out);
+}
+// one single-thread block per result of a batch
+template <class F>
+__global__ void k_xyzz_to_affine_std_many(const XYZZ<F>* in, char* out) {
+    xyzz_to_affine_std(in + blockIdx.x, out + 2 * sizeof(F) * blockIdx.x);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -595,6 +647,30 @@ struct MsmHooks {
     cudaEvent_t ev_sorted = nullptr;
 };
 
+// Work buffers of msm_run_many: up to `cap` scalar vectors over one base set in one pass (DESIGN.md 4.10).  Vector j's
+// digits are keyed j * nbuckets + |digit| - 1, so the k vectors are one MSM over k x W x n entries and k x nbuckets
+// buckets; only the bucket reduction has a batch dimension.
+struct MsmMany {
+    int cap = 0;
+    int logL = 3;                     // level-1 entries per thread, fixed by cap (the bnd buffers are sized for it)
+    uint32_t T1p = 0;
+    uint32_t *keys[2] = {nullptr, nullptr}, *vals[2] = {nullptr, nullptr};   // null: sorts are borrowed (sorted_from)
+    void* cub_tmp = nullptr;
+    size_t cub_bytes = 0;
+    void* buckets = nullptr;          // cap x nbuckets
+    void* bnd[2] = {nullptr, nullptr};
+    uint32_t* bnd_keys[2] = {nullptr, nullptr};
+    void* red = nullptr;              // cap x nred: each vector's row / column sums and weighted terms
+    uint32_t nred = 0;
+    unsigned int* red_counter = nullptr;   // cap completion counters
+    uint32_t* run_lo = nullptr;       // 2 x cap x nbuckets
+    int* range_err = nullptr;         // cap flags: vector j has a scalar >= r
+    void* result = nullptr;           // cap XYZZ results (zkr_msm_many)
+    size_t bytes = 0;
+    const uint32_t* sorted_keys = nullptr;
+    const uint32_t* sorted_vals = nullptr;
+};
+
 }  // namespace zkr
 
 struct zkr_bases {
@@ -610,6 +686,7 @@ struct zkr_bases {
     int logL = 5;
     uint32_t T1p = 0;                 // level-1 threads (padded to whole blocks)
     uint64_t map_hash = 0;            // FNV-1a of the compact -> scalar index map (equal maps <=> shareable sort)
+    zkr::MsmMany* many = nullptr;     // zkr_msm_many's work buffers: grown on first use, freed with the bases
 };
 
 namespace zkr {
@@ -622,6 +699,14 @@ int bases_build(zkr_ctx* ctx, zkr_bases* b, const char* h_points, size_t n_src, 
 template <class F>
 int msm_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* d_scalars, XYZZ<F>* d_out,
             const MsmHooks* hooks = nullptr);
+// Batched MSM over one base set: vector j's scalars at d_scalars + 32 * stride * j bytes (through the same compaction
+// map), its XYZZ result at (char*)d_out + j * out_stride.  sorted_from: take the sorted pairs of another base set's
+// batch of this call (same conditions as MsmHooks::sorted_from); ev_sorted: recorded once this batch's sort is final.
+template <class F>
+int many_alloc(const zkr_bases* b, int cap, bool sorts, cudaStream_t st, MsmMany* w);
+template <class F>
+int msm_run_many(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, MsmMany* w, int k, const uint32_t* d_scalars,
+                 size_t stride, void* d_out, size_t out_stride, const MsmMany* sorted_from, cudaEvent_t ev_sorted);
 void bases_release(zkr_bases* b);
 
 // ---------------------------------------------------------------- implementation (header-only, two TUs)
@@ -732,11 +817,87 @@ int bases_build(zkr_ctx* ctx, zkr_bases* b, const char* h_points, size_t n_src, 
     return ZKR_OK;
 }
 
+// One sorted (bucket, table entry) list -> bucket sums: level-1 accumulation, then the gather or the boundary levels.
+// nbk buckets, nbk is also the sentinel key; msm_run passes its base set's buffers, msm_run_many a batch's.
+struct AccumView {
+    const uint32_t *skeys, *svals;
+    uint32_t total, nbk, T1p;
+    int logL;
+    void* buckets;
+    void* const* bnd;
+    uint32_t* const* bnd_keys;
+    uint32_t* run_lo;
+};
+
+template <class F>
+int accumulate(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const AccumView& v) {
+    constexpr size_t XB = 4 * sizeof(F);
+    constexpr bool kPrefetch = sizeof(F) == 32;    // G2 is register-bound; no software prefetch there
+    const int c = b->plan.c;
+    const uint32_t nb = v.nbk, total = v.total;
+    const uint32_t *skeys = v.skeys, *svals = v.svals;
+    ZKR_CUDA(cudaMemsetAsync(v.buckets, 0, XB * (size_t)nb, st));
+
+    // level 1
+    const int L = 1 << v.logL;
+    const size_t smem = (size_t)(kAccumThreads / 32) * 2 * 32 * (L + 1) * 4;
+    XYZZ<F>* buckets = (XYZZ<F>*)v.buckets;
+    const int pslot = ctx->prof_begin(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, st, (double)total);
+    // Boundary partials -> buckets: the one-launch gather up to 20-bit windows (every proof size), the round-1 recursive
+    // levels above: at 22-bit windows the 12-bit top window puts n / 4096 extra entries into each of the 4096 lowest buckets,
+    // i.e. thousands of moderately heavy buckets, which the whole-CTA heavy path handles badly (2^24: 48 vs 40.6 ms,
+    // profiles/r02_msm_gather_vs_levels.json).
+    // ZKR_MSM_LEVELS = 0 / 1 forces the gather / the levels (A/B knob).
+    static const int force_levels = getenv("ZKR_MSM_LEVELS") ? atoi(getenv("ZKR_MSM_LEVELS")) : -1;
+    const bool use_levels = force_levels >= 0 ? force_levels != 0 : c > 20;
+    if (!use_levels) ZKR_CUDA(cudaMemsetAsync(v.run_lo, 0xff, 4 * (size_t)nb, st));
+    // ZKR_LAZY: bit 0 = G1, bit 1 = G2 use the lazily reduced mixed addition, bit 2 = G1 additionally squares with
+    // mont_sqr_raw (A/B knob; bit-identical results)
+    const char* lazy_env = getenv("ZKR_LAZY");             // read per call: the GPU tests flip it inside one process
+    const int lazy_mask = lazy_env ? atoi(lazy_env) : kLazyDefault;
+    const int variant = !(lazy_mask & (sizeof(F) == 32 ? 1 : 2)) ? 0 : (sizeof(F) == 32 && (lazy_mask & 4)) ? 2 : 1;
+    auto launch = [&](auto kern) -> int {
+        ZKR_LAUNCH(ctx, kern, v.T1p / kAccumThreads, kAccumThreads, smem, st, skeys, svals, total, v.logL, b->table, buckets,
+                   (XYZZ<F>*)v.bnd[0], use_levels ? v.bnd_keys[0] : nullptr, nb, use_levels ? nullptr : v.run_lo);
+        return ZKR_OK;
+    };
+    int lrc;
+    if (variant == 2) lrc = launch(k_accum_affine<F, kPrefetch, sizeof(F) == 32 ? 2 : 1>);
+    else if (variant == 1) lrc = launch(k_accum_affine<F, kPrefetch, 1>);
+    else lrc = launch(k_accum_affine<F, kPrefetch, 0>);
+    if (lrc != ZKR_OK) return lrc;
+    ctx->prof_end(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, pslot, st);
+    if (!use_levels) {
+        ZKR_LAUNCH(ctx, k_bucket_gather<F>, kHeavyBlocks + ceil_div(nb, kGatherThreads), kGatherThreads, XB * kGatherThreads,
+                   st, skeys, total, v.logL, v.run_lo, (const XYZZ<F>*)v.bnd[0], buckets, nb);
+    }
+    // boundary levels (round-1 path)
+    size_t cnt = 2 * (size_t)v.T1p;
+    int cur = 0;
+    for (; use_levels;) {
+        const int llog = level_log(cnt);
+        const size_t lvl = (size_t)1 << llog;
+        if (cnt <= kFinishMax) {
+            ZKR_LAUNCH(ctx, k_accum_finish<F>, 1, kFinishThreads, 0, st, v.bnd_keys[cur], (XYZZ<F>*)v.bnd[cur],
+                       v.bnd_keys[cur ^ 1], (XYZZ<F>*)v.bnd[cur ^ 1], (uint32_t)cnt, buckets, nb);
+            break;
+        }
+        const bool fin = cnt <= lvl;
+        const size_t T = (cnt + lvl - 1) / lvl;
+        const unsigned blocks = (unsigned)((T + 63) / 64);
+        ZKR_LAUNCH(ctx, k_accum_xyzz<F>, blocks, 64, 0, st, v.bnd_keys[cur], (const XYZZ<F>*)v.bnd[cur],
+                   (uint32_t)cnt, llog, buckets, (XYZZ<F>*)v.bnd[cur ^ 1], v.bnd_keys[cur ^ 1], nb, fin);
+        if (fin) break;
+        cnt = 2 * T;          // threads past T only pad their block; their slots are never read
+        cur ^= 1;
+    }
+    return ZKR_OK;
+}
+
 template <class F>
 int msm_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* d_scalars, XYZZ<F>* d_out,
             const MsmHooks* hooks) {
     constexpr size_t XB = 4 * sizeof(F);
-    constexpr bool kPrefetch = sizeof(F) == 32;    // G2 is register-bound; no software prefetch there
     const uint32_t n = b->n;
     if (n == 0) {
         ZKR_CUDA(cudaMemsetAsync(d_out, 0, XB, st));
@@ -766,67 +927,144 @@ int msm_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, const uint32_t* d
         svals = wk.sorted_vals = dv.Current();
         if (hooks && hooks->ev_sorted) ZKR_CUDA(cudaEventRecord(hooks->ev_sorted, st));
     }
-    ZKR_CUDA(cudaMemsetAsync(wk.buckets, 0, XB * (size_t)nb, st));
-
-    // level 1
-    const int L = 1 << b->logL;
-    const size_t smem = (size_t)(kAccumThreads / 32) * 2 * 32 * (L + 1) * 4;
-    XYZZ<F>* buckets = (XYZZ<F>*)wk.buckets;
-    const int pslot = ctx->prof_begin(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, st, (double)total);
-    // Boundary partials -> buckets: the one-launch gather up to 20-bit windows (every proof size), the round-1 recursive
-    // levels above: at 22-bit windows the 12-bit top window puts n / 4096 extra entries into each of the 4096 lowest buckets,
-    // i.e. thousands of moderately heavy buckets, which the whole-CTA heavy path handles badly (2^24: 48 vs 40.6 ms,
-    // profiles/r02_msm_gather_vs_levels.json).
-    // ZKR_MSM_LEVELS = 0 / 1 forces the gather / the levels (A/B knob).
-    static const int force_levels = getenv("ZKR_MSM_LEVELS") ? atoi(getenv("ZKR_MSM_LEVELS")) : -1;
-    const bool use_levels = force_levels >= 0 ? force_levels != 0 : c > 20;
-    if (!use_levels) ZKR_CUDA(cudaMemsetAsync(wk.run_lo, 0xff, 4 * (size_t)nb, st));
-    // ZKR_LAZY: bit 0 = G1, bit 1 = G2 use the lazily reduced mixed addition, bit 2 = G1 additionally squares with
-    // mont_sqr_raw (A/B knob; bit-identical results)
-    const char* lazy_env = getenv("ZKR_LAZY");             // read per call: the GPU tests flip it inside one process
-    const int lazy_mask = lazy_env ? atoi(lazy_env) : kLazyDefault;
-    const int variant = !(lazy_mask & (sizeof(F) == 32 ? 1 : 2)) ? 0 : (sizeof(F) == 32 && (lazy_mask & 4)) ? 2 : 1;
-    auto launch = [&](auto kern) -> int {
-        ZKR_LAUNCH(ctx, kern, b->T1p / kAccumThreads, kAccumThreads, smem, st, skeys, svals, total, b->logL, b->table, buckets,
-                   (XYZZ<F>*)wk.bnd[0], use_levels ? wk.bnd_keys[0] : nullptr, nb, use_levels ? nullptr : wk.run_lo);
-        return ZKR_OK;
-    };
-    int lrc;
-    if (variant == 2) lrc = launch(k_accum_affine<F, kPrefetch, sizeof(F) == 32 ? 2 : 1>);
-    else if (variant == 1) lrc = launch(k_accum_affine<F, kPrefetch, 1>);
-    else lrc = launch(k_accum_affine<F, kPrefetch, 0>);
-    if (lrc != ZKR_OK) return lrc;
-    ctx->prof_end(sizeof(F) == 32 ? PROF_ACCUM_G1 : PROF_ACCUM_G2, pslot, st);
-    if (!use_levels) {
-        ZKR_LAUNCH(ctx, k_bucket_gather<F>, kHeavyBlocks + ceil_div(nb, kGatherThreads), kGatherThreads, XB * kGatherThreads,
-                   st, skeys, total, b->logL, wk.run_lo, (const XYZZ<F>*)wk.bnd[0], buckets, nb);
-    }
-    // boundary levels (round-1 path)
-    size_t cnt = 2 * (size_t)b->T1p;
-    int cur = 0;
-    for (; use_levels;) {
-        const int llog = level_log(cnt);
-        const size_t lvl = (size_t)1 << llog;
-        if (cnt <= kFinishMax) {
-            ZKR_LAUNCH(ctx, k_accum_finish<F>, 1, kFinishThreads, 0, st, wk.bnd_keys[cur], (XYZZ<F>*)wk.bnd[cur],
-                       wk.bnd_keys[cur ^ 1], (XYZZ<F>*)wk.bnd[cur ^ 1], (uint32_t)cnt, buckets, nb);
-            break;
-        }
-        const bool fin = cnt <= lvl;
-        const size_t T = (cnt + lvl - 1) / lvl;
-        const unsigned blocks = (unsigned)((T + 63) / 64);
-        ZKR_LAUNCH(ctx, k_accum_xyzz<F>, blocks, 64, 0, st, wk.bnd_keys[cur], (const XYZZ<F>*)wk.bnd[cur],
-                   (uint32_t)cnt, llog, buckets, (XYZZ<F>*)wk.bnd[cur ^ 1], wk.bnd_keys[cur ^ 1], nb, fin);
-        if (fin) break;
-        cnt = 2 * T;          // threads past T only pad their block; their slots are never read
-        cur ^= 1;
-    }
+    const AccumView v = {skeys, svals, total, nb, b->T1p, b->logL, wk.buckets, wk.bnd, wk.bnd_keys, wk.run_lo};
+    ZKR_TRY(accumulate<F>(ctx, st, b, v));
     // bucket reduction: row / column sums, then bit-decomposed weighted sums (see k_bucket_sums)
     const int lc = (c - 1) / 2, lr = c - 1 - lc;
-    ZKR_LAUNCH(ctx, (k_bucket_sums<F, kReduceThreads>), (1u << lr) + (1u << lc), kReduceThreads, XB * kReduceThreads, st, buckets, lr, lc,
-               (XYZZ<F>*)wk.red);
+    ZKR_LAUNCH(ctx, (k_bucket_sums<F, kReduceThreads>), (1u << lr) + (1u << lc), kReduceThreads, XB * kReduceThreads, st,
+               (const XYZZ<F>*)wk.buckets, lr, lc, (XYZZ<F>*)wk.red);
     ZKR_LAUNCH(ctx, (k_bucket_weighted<F, kReduceThreads>), lr + lc + 1, kReduceThreads, XB * kReduceThreads, st, (XYZZ<F>*)wk.red, lr, lc,
                wk.red_counter, d_out);
+    return ZKR_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ batched MSM
+// Sort keys of a batch of k vectors: k * nbuckets + 1 values (the zero-digit sentinel is k * nbuckets).
+inline int many_key_bits(int c, int k) {
+    int lg = 0;
+    while ((1 << lg) < k) lg++;
+    return c - 1 + lg + 1;
+}
+
+// ZKR_E_UNSUPPORTED, with the limit named, when k vectors over b do not fit one sort.
+inline int many_limits(const zkr_bases* b, int k) {
+    if (k < 1 || k > kMaxBatch) {
+        set_error("batch of %d vectors: 1 .. %d per call", k, kMaxBatch);
+        return k < 1 ? ZKR_E_INVALID : ZKR_E_UNSUPPORTED;
+    }
+    const uint64_t entries = (uint64_t)k * b->plan.W * b->n;
+    if (entries >= (1ull << 31)) {
+        set_error("batch of %d vectors: %d x %d windows x %u points = %llu sort entries, the limit is < 2^31", k, k,
+                  b->plan.W, b->n, (unsigned long long)entries);
+        return ZKR_E_UNSUPPORTED;
+    }
+    if (many_key_bits(b->plan.c, k) > 31) {
+        set_error("batch of %d vectors: sort keys of %d bits at %d-bit windows, the limit is 31 bits", k,
+                  many_key_bits(b->plan.c, k), b->plan.c);
+        return ZKR_E_UNSUPPORTED;
+    }
+    return ZKR_OK;
+}
+
+template <class F>
+int many_alloc(const zkr_bases* b, int cap, bool sorts, cudaStream_t st, MsmMany* w) {
+    constexpr size_t XB = 4 * sizeof(F);
+    ZKR_TRY(many_limits(b, cap));
+    w->cap = cap;
+    const uint32_t n = b->n;
+    if (n == 0) return ZKR_OK;
+    const int c = b->plan.c;
+    const size_t nbk = (size_t)cap * b->plan.nbuckets;
+    const size_t total = (size_t)cap * b->plan.W * n;
+    auto dmalloc = [&](auto** p, size_t bytes) -> int {
+        ZKR_CUDA(cudaMalloc(p, bytes ? bytes : 1));
+        w->bytes += bytes;
+        return ZKR_OK;
+    };
+    // as bases_build, for the batch's entry count
+    w->logL = total >= (1u << 22) ? 5 : (total >= (1u << 16) ? 4 : 3);
+    const size_t L = (size_t)1 << w->logL;
+    const size_t T1 = (total + L - 1) / L;
+    w->T1p = (uint32_t)(((T1 + kAccumThreads - 1) / kAccumThreads) * kAccumThreads);
+    if (sorts) {
+        for (int i = 0; i < 2; i++) {
+            ZKR_TRY(dmalloc(&w->keys[i], 4 * total));
+            ZKR_TRY(dmalloc(&w->vals[i], 4 * total));
+        }
+        cub::DoubleBuffer<uint32_t> dk(w->keys[0], w->keys[1]), dv(w->vals[0], w->vals[1]);
+        ZKR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, w->cub_bytes, dk, dv, (int)total, 0, many_key_bits(c, cap), st));
+        ZKR_TRY(dmalloc(&w->cub_tmp, w->cub_bytes));
+    }
+    ZKR_TRY(dmalloc(&w->buckets, XB * nbk));
+    const size_t bnd0 = 2 * (size_t)w->T1p;
+    size_t bnd1 = 2 * (((bnd0 + 1) / 2 + 63) / 64 * 64);
+    if (bnd1 < 2 * (size_t)kFinishThreads) bnd1 = 2 * (size_t)kFinishThreads;
+    ZKR_TRY(dmalloc(&w->bnd[0], XB * bnd0));
+    ZKR_TRY(dmalloc(&w->bnd[1], XB * bnd1));
+    ZKR_TRY(dmalloc(&w->bnd_keys[0], 4 * bnd0));
+    ZKR_TRY(dmalloc(&w->bnd_keys[1], 4 * bnd1));
+    const int rlc = (c - 1) / 2, rlr = c - 1 - rlc;
+    w->nred = (1u << rlr) + (1u << rlc) + 32;
+    ZKR_TRY(dmalloc(&w->red, XB * w->nred * (size_t)cap));
+    ZKR_TRY(dmalloc(&w->red_counter, sizeof(unsigned int) * cap));
+    ZKR_CUDA(cudaMemsetAsync(w->red_counter, 0, sizeof(unsigned int) * cap, st));
+    ZKR_TRY(dmalloc(&w->run_lo, 8 * nbk));
+    ZKR_TRY(dmalloc(&w->range_err, sizeof(int) * cap));
+    ZKR_CUDA(cudaMemsetAsync(w->range_err, 0, sizeof(int) * cap, st));
+    ZKR_TRY(dmalloc(&w->result, XB * cap));
+    ZKR_CUDA(cudaFuncSetAttribute((k_bucket_sums_many<F, kReduceThreads>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(XB * kReduceThreads)));
+    ZKR_CUDA(cudaFuncSetAttribute((k_bucket_weighted_many<F, kReduceThreads>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(XB * kReduceThreads)));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    return ZKR_OK;
+}
+
+template <class F>
+int msm_run_many(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, MsmMany* w, int k, const uint32_t* d_scalars,
+                 size_t stride, void* d_out, size_t out_stride, const MsmMany* sorted_from, cudaEvent_t ev_sorted) {
+    constexpr size_t XB = 4 * sizeof(F);
+    if (k < 1 || k > w->cap) {
+        set_error("msm_run_many: %d vectors, the work buffers hold %d", k, w->cap);
+        return ZKR_E_INVALID;
+    }
+    const uint32_t n = b->n;
+    if (n == 0) {
+        ZKR_CUDA(cudaMemset2DAsync(d_out, out_stride, 0, XB, k, st));
+        return ZKR_OK;
+    }
+    const int c = b->plan.c, W = b->plan.W;
+    const uint32_t nb = b->plan.nbuckets, nbk = nb * (uint32_t)k;
+    const uint32_t total = (uint32_t)k * W * n;
+    if (sorted_from) {
+        if (!sorted_from->sorted_keys) {
+            set_error("msm_run_many: the base set to share a sort with has not sorted this batch");
+            return ZKR_E_INVALID;
+        }
+        w->sorted_keys = sorted_from->sorted_keys;
+        w->sorted_vals = sorted_from->sorted_vals;
+    } else {
+        ZKR_LAUNCH(ctx, k_digits_many, dim3(ceil_div(n, 128), k), 128, 0, st, d_scalars, stride, b->src_index, n, c, W, nb,
+                   nbk, w->keys[0], w->vals[0], w->range_err);
+        cub::DoubleBuffer<uint32_t> dk(w->keys[0], w->keys[1]), dv(w->vals[0], w->vals[1]);
+        const int bits = many_key_bits(c, k);
+        size_t need = 0;
+        ZKR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, dk, dv, (int)total, 0, bits, st));
+        if (need > w->cub_bytes) {
+            set_error("msm_run_many: the sort needs %zu bytes of scratch, %zu were sized", need, w->cub_bytes);
+            return ZKR_E_INVALID;
+        }
+        ZKR_CUDA(cub::DeviceRadixSort::SortPairs(w->cub_tmp, need, dk, dv, (int)total, 0, bits, st));
+        ctx->launches += 4;   // CUB, counted as a block (as msm_run)
+        w->sorted_keys = dk.Current();
+        w->sorted_vals = dv.Current();
+        if (ev_sorted) ZKR_CUDA(cudaEventRecord(ev_sorted, st));
+    }
+    const AccumView v = {w->sorted_keys, w->sorted_vals, total, nbk, w->T1p, w->logL, w->buckets, w->bnd, w->bnd_keys, w->run_lo};
+    ZKR_TRY(accumulate<F>(ctx, st, b, v));
+    const int lc = (c - 1) / 2, lr = c - 1 - lc;
+    ZKR_LAUNCH(ctx, (k_bucket_sums_many<F, kReduceThreads>), dim3((1u << lr) + (1u << lc), k), kReduceThreads, XB * kReduceThreads,
+               st, (const XYZZ<F>*)w->buckets, nb, lr, lc, (XYZZ<F>*)w->red, w->nred);
+    ZKR_LAUNCH(ctx, (k_bucket_weighted_many<F, kReduceThreads>), dim3(lr + lc + 1, k), kReduceThreads, XB * kReduceThreads, st,
+               (XYZZ<F>*)w->red, w->nred, lr, lc, w->red_counter, (char*)d_out, out_stride);
     return ZKR_OK;
 }
 

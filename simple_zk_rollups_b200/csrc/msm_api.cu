@@ -88,6 +88,45 @@ extern "C" int zkr_msm(zkr_ctx* ctx, const zkr_bases* b, const void* scalars, si
     return ZKR_OK;
 }
 
+extern "C" int zkr_msm_many(zkr_ctx* ctx, const zkr_bases* b, const void* scalars, size_t n, int n_vectors,
+                            int scalars_on_device, void* out_affine) {
+    if (!ctx || !b || !scalars || !out_affine || bases_ctx(b) != ctx || n != bases_n_src(b) || n_vectors < 1) {
+        set_error("zkr_msm_many: bad arguments (n_vectors >= 1, scalar count per vector = the number of loaded points)");
+        return ZKR_E_INVALID;
+    }
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = ctx->user_stream;
+    const int group = bases_group(b);
+    const size_t ob = group == 1 ? 64 : 128, xb = 2 * ob;
+    const size_t k = (size_t)n_vectors;
+    MsmMany* w;
+    ZKR_TRY(bases_many_work(const_cast<zkr_bases*>(b), n_vectors, st, &w));
+    if (bases_result_buf(b) == nullptr) {     // no finite point: every result is infinity
+        memset(out_affine, 0, ob * k);
+        return ZKR_OK;
+    }
+    const uint32_t* d_sc = (const uint32_t*)scalars;
+    if (!scalars_on_device) {
+        void* p;
+        ZKR_TRY(ctx->scratch_get("msm_scalars", k * n * 32 + 32, &p));
+        ZKR_CUDA(cudaMemcpyAsync(p, scalars, k * n * 32, cudaMemcpyHostToDevice, st));
+        d_sc = (const uint32_t*)p;
+    }
+    void* d_aff;
+    ZKR_TRY(ctx->scratch_get("msm_many_out", ob * k, &d_aff));
+    void* res = msm_many_result_buf(w);
+    ZKR_TRY(msm_many_run(ctx, st, b, w, n_vectors, d_sc, n, res, xb));
+    ZKR_TRY(results_to_affine_std_many(ctx, st, group, res, n_vectors, d_aff));
+    ZKR_CUDA(cudaMemcpyAsync(out_affine, d_aff, ob * k, cudaMemcpyDeviceToHost, st));
+    int bad = -1;
+    ZKR_TRY(msm_many_range_error(w, n_vectors, st, &bad));
+    if (bad >= 0) {
+        set_error("vector %d has a scalar >= r", bad);
+        return ZKR_E_WITNESS_RANGE;
+    }
+    return ZKR_OK;
+}
+
 extern "C" int zkr_test_bases_peek(const zkr_bases* b, int what, size_t offset, void* out, size_t bytes) {
     if (!b || !out) return ZKR_E_INVALID;
     DeviceGuard g(bases_ctx(b)->device);

@@ -7,6 +7,66 @@ int g1_result_to_affine_std(zkr_ctx* ctx, cudaStream_t st, const void* d_xyzz, v
     ZKR_LAUNCH(ctx, k_xyzz_to_affine_std<Fq>, 1, 1, 0, st, (const XYZZ<Fq>*)d_xyzz, (char*)d_out64);
     return ZKR_OK;
 }
+// G2 instantiations of the batched MSM (msm_g2.cu)
+int many_alloc_g2(const zkr_bases* b, int cap, bool sorts, cudaStream_t st, MsmMany* w);
+int msm_run_many_g2(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, MsmMany* w, int k, const uint32_t* sc, size_t stride,
+                    void* out, size_t out_stride, const MsmMany* sorted_from, cudaEvent_t ev_sorted);
+int g2_results_to_affine_std_many(zkr_ctx* ctx, cudaStream_t st, const void* d_xyzz, int k, void* d_out);
+
+int msm_many_alloc(const zkr_bases* b, int cap, bool sorts, cudaStream_t st, MsmMany** out) {
+    MsmMany* w = new MsmMany();
+    const int rc = b->group == 1 ? many_alloc<Fq>(b, cap, sorts, st, w) : many_alloc_g2(b, cap, sorts, st, w);
+    if (rc != ZKR_OK) {
+        msm_many_free(w);
+        return rc;
+    }
+    *out = w;
+    return ZKR_OK;
+}
+void msm_many_free(MsmMany* w) {
+    if (!w) return;
+    void* ps[] = {w->keys[0], w->keys[1], w->vals[0], w->vals[1], w->cub_tmp, w->buckets, w->bnd[0], w->bnd[1],
+                  w->bnd_keys[0], w->bnd_keys[1], w->red, w->red_counter, w->run_lo, w->range_err, w->result};
+    for (void* p : ps) cudaFree(p);
+    delete w;
+}
+uint64_t msm_many_bytes(const MsmMany* w) { return w ? w->bytes : 0; }
+void* msm_many_result_buf(const MsmMany* w) { return w->result; }
+int msm_many_run(zkr_ctx* ctx, cudaStream_t st, const zkr_bases* b, MsmMany* w, int k, const uint32_t* sc, size_t stride,
+                 void* out, size_t out_stride, const MsmMany* sorted_from, cudaEvent_t ev_sorted) {
+    return b->group == 1 ? msm_run_many<Fq>(ctx, st, b, w, k, sc, stride, out, out_stride, sorted_from, ev_sorted)
+                         : msm_run_many_g2(ctx, st, b, w, k, sc, stride, out, out_stride, sorted_from, ev_sorted);
+}
+int msm_many_range_error(const MsmMany* w, int k, cudaStream_t st, int* first_bad) {
+    *first_bad = -1;
+    if (!w->range_err) return ZKR_OK;
+    std::vector<int> f(k);
+    ZKR_CUDA(cudaMemcpyAsync(f.data(), w->range_err, sizeof(int) * k, cudaMemcpyDeviceToHost, st));
+    ZKR_CUDA(cudaStreamSynchronize(st));
+    for (int j = 0; j < k && *first_bad < 0; j++)
+        if (f[j]) *first_bad = j;
+    if (*first_bad >= 0) ZKR_CUDA(cudaMemsetAsync(w->range_err, 0, sizeof(int) * k, st));
+    return ZKR_OK;
+}
+int bases_many_work(zkr_bases* b, int k, cudaStream_t st, MsmMany** out) {
+    if (!b->many || b->many->cap < k) {
+        if (b->many) {
+            ZKR_CUDA(cudaStreamSynchronize(st));
+            b->bytes -= b->many->bytes;
+            msm_many_free(b->many);
+            b->many = nullptr;
+        }
+        ZKR_TRY(msm_many_alloc(b, k, true, st, &b->many));
+        b->bytes += b->many->bytes;
+    }
+    *out = b->many;
+    return ZKR_OK;
+}
+int results_to_affine_std_many(zkr_ctx* ctx, cudaStream_t st, int group, const void* d_xyzz, int k, void* d_out) {
+    if (group != 1) return g2_results_to_affine_std_many(ctx, st, d_xyzz, k, d_out);
+    ZKR_LAUNCH(ctx, k_xyzz_to_affine_std_many<Fq>, k, 1, 0, st, (const XYZZ<Fq>*)d_xyzz, (char*)d_out);
+    return ZKR_OK;
+}
 }  // namespace zkr
 
 // non-template glue used by msm_api.cu / prover.cu (they do not include msm.cuh)
@@ -80,6 +140,7 @@ void bases_release(zkr_bases* b) {
                   w.bnd[0], w.bnd[1], w.bnd_keys[0], w.bnd_keys[1], w.red, w.red_counter, w.result, w.range_err,
                   w.run_lo};
     for (void* p : ps) cudaFree(p);
+    msm_many_free(b->many);
     delete b;
 }
 }  // namespace zkr

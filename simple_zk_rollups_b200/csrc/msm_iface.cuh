@@ -32,4 +32,21 @@ void bases_info(const zkr_bases* b, uint64_t* n, int* c, int* W, uint64_t* bytes
 void* bases_result_buf(const zkr_bases* b);
 uint64_t bases_n_src(const zkr_bases* b);
 int bases_peek(const zkr_bases* b, int what, size_t offset, void* out, size_t bytes);
+
+// Batched MSM (msm.cuh msm_run_many): k <= kMaxBatch scalar vectors over one base set in one pass.
+struct MsmMany;
+// work buffers for up to `cap` vectors; sorts == false: no digit / sort buffers (the batch borrows another set's sort)
+int msm_many_alloc(const zkr_bases* b, int cap, bool sorts, cudaStream_t st, MsmMany** out);
+void msm_many_free(MsmMany* w);
+uint64_t msm_many_bytes(const MsmMany* w);
+// vector j: scalars at d_scalars + 32 * stride * j bytes, XYZZ result at (char*)d_out + j * out_stride
+int msm_many_run(zkr_ctx*, cudaStream_t, const zkr_bases*, MsmMany*, int k, const uint32_t* d_scalars, size_t stride,
+                 void* d_out, size_t out_stride, const MsmMany* sorted_from = nullptr, cudaEvent_t ev_sorted = nullptr);
+// first vector of the last batch with a scalar >= r, or -1; clears the flags (synchronises st)
+int msm_many_range_error(const MsmMany* w, int k, cudaStream_t st, int* first_bad);
+// zkr_msm_many: the bases' own work buffers, grown to at least k vectors
+int bases_many_work(zkr_bases* b, int k, cudaStream_t st, MsmMany** out);
+void* msm_many_result_buf(const MsmMany* w);
+// k XYZZ results (contiguous) -> k affine standard-form points (64 / 128 B each), one single-thread block per result
+int results_to_affine_std_many(zkr_ctx*, cudaStream_t, int group, const void* d_xyzz, int k, void* d_out);
 }  // namespace zkr

@@ -120,6 +120,7 @@ __device__ __forceinline__ int slot_of(int e) { return e + (e >> 3); }
 //   1  COLS slab in, push to the peers' ROWS buffers: row i of the first DIF pass belongs to rank i >> (k - g)
 //   2  push to the peers' COLS buffers: column j of the last-but-one DIT pass belongs to rank j >> (s0 - g)
 //   3  in place on a COLS slab (last DIT pass)
+//   4  in place, batched: blockIdx.y selects one of gridDim.y vectors (PassFuse::vstride; h_pipeline_many)
 // On a COLS slab (modes 1, 3) ls_ = log2 of the row stride in memory (s0 - g) and ctw_ = global column of
 // this rank's first local column (twiddles use global coordinates); otherwise ls == s and ctw == 0.
 // Fused element-wise work (H pipeline: no separate sweeps over memory).  Runtime values, uniform per launch:
@@ -140,8 +141,18 @@ struct PassFuse {
     Fr* out;             // ST_HFINAL: destination (null = data)
     const Fr* twfull;    // full inter-pass twiddle table of this pass (null = two-level)
     Fr* data2;           // second vector transformed by the same launch (blockIdx.y == 1); null = one vector
+    size_t vstride;      // MODE 4 (batched): gridDim.y / (data2 ? 2 : 1) vectors per array at this stride, the same for
+                         // data, data2, src, in2 and out (tab, twfull, kconst are shared)
     int ld_op, st_op;
 };
+
+// vectors per array of a batched launch (MODE 4), and the element offset of this CTA's vector, recomputed where it is
+// used from the grid and the parameters (kept live across the pass it cost the DIT kernel stack)
+__device__ __forceinline__ unsigned batch_count(const PassFuse& fz) { return fz.data2 ? gridDim.y >> 1 : gridDim.y; }
+__device__ __forceinline__ size_t batch_offset(const PassFuse& fz) {
+    const unsigned nv = batch_count(fz);
+    return (size_t)(blockIdx.y >= nv ? blockIdx.y - nv : blockIdx.y) * fz.vstride;
+}
 
 // RL = log2 of the register-stage radix.  RL = 3 (the only instantiation): a thread holds 8 elements = 3 butterfly levels
 // between two barriers, 112-128 registers, 2 CTAs / SM (4 warps per scheduler).  RL = 2 (two groups of 4 elements,
@@ -153,6 +164,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
            int kw, const Fr* __restrict__ tlo, const Fr* __restrict__ thi, int lb, int tw_shift, NttXchg xp, PassFuse fz) {
     extern __shared__ uint32_t sm[];
     constexpr bool kSlab = MODE == 1 || MODE == 3;
+    constexpr bool kBatch = MODE == 4;
     const int ls = kSlab ? ls_ : s;
     const unsigned ctw = kSlab ? ctw_ : 0u;
     const int T = k + c;
@@ -165,6 +177,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
     // two independent transforms of one size can share a launch (the H pipeline's A and B): twice the CTAs per wave
     // quantum, half the launches
     if (MODE == 0 && blockIdx.y) data = fz.data2;
+    if (kBatch && blockIdx.y) data = (blockIdx.y >= batch_count(fz) ? fz.data2 : data) + batch_offset(fz);
     Fr* chunk = data + (q << chunk_log);
     const unsigned cm = cg << c;             // first column of the tile in memory
     const unsigned c0 = ctw + cm;            // ... and in the transform's global coordinates
@@ -179,7 +192,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
         // Whole elements per thread.  DIT applies the inter-pass twiddle omega_N'^(col * rev(row)) BEFORE its butterflies:
         // do it on the way in, so the register stages below hold nothing but the 8 butterfly operands (with the twiddle
         // inside the first stage ptxas spilled 272 B per thread).  The fused load operations ride on the same path.
-        const Fr* src = fz.src ? fz.src + qbase : chunk;
+        const Fr* src = fz.src ? fz.src + (kBatch ? batch_offset(fz) : 0) + qbase : chunk;
 #pragma unroll 1
         for (int g = 0; g < 2; g++) {
             Fr v[4];
@@ -192,7 +205,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
             }
             if (fz.ld_op == LD_MUL2) {
 #pragma unroll
-                for (int i = 0; i < 4; i++) v[i] = v[i] * Fr::load(fz.in2 + qbase + off[i]);
+                for (int i = 0; i < 4; i++) v[i] = v[i] * Fr::load(fz.in2 + (kBatch ? batch_offset(fz) : 0) + qbase + off[i]);
             } else if (fz.ld_op == LD_TAB) {
 #pragma unroll
                 for (int i = 0; i < 4; i++) v[i] = v[i] * Fr::load_ro(fz.tab + qbase + off[i]);
@@ -331,10 +344,10 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
     }
 
     // ---- shared -> global
-    if (MODE == 0 && fz.st_op == ST_HFINAL) {
+    if ((MODE == 0 || kBatch) && fz.st_op == ST_HFINAL) {
         // whole elements: out[pos] = S[pos] * K - x * tab[pos]
         const Fr K = Fr::load_ro(fz.kconst);
-        Fr* outp = (fz.out ? fz.out : data) + qbase;
+        Fr* outp = (fz.out ? fz.out + (kBatch ? batch_offset(fz) : 0) : data) + qbase;
 #pragma unroll 2
         for (int e = tid; e < tile; e += blockDim.x) {
             const size_t off = ((size_t)(e >> c) << ls) + cm + (e & cmask);
@@ -342,7 +355,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
             const uint32_t* d = sm + slot_of(e);
 #pragma unroll
             for (int l = 0; l < 8; l++) x.v[l] = d[l * plane];
-            const Fr v = Fr::load(fz.in2 + qbase + off) * K - x * Fr::load_ro(fz.tab + qbase + off);
+            const Fr v = Fr::load(fz.in2 + (kBatch ? batch_offset(fz) : 0) + qbase + off) * K - x * Fr::load_ro(fz.tab + qbase + off);
             v.store(outp + off);
         }
         return;
@@ -353,7 +366,7 @@ k_ntt_pass(Fr* data, int k, int c, int s, int ls_, int chunk_log, unsigned ctw_,
         const uint32_t* d = sm + (4 * half) * plane + slot_of(e);
         uint4 v = make_uint4(d[0], d[plane], d[2 * plane], d[3 * plane]);
         Fr* dp;
-        if (MODE == 0 || MODE == 3) {
+        if (MODE == 0 || MODE == 3 || kBatch) {
             dp = chunk + ((size_t)row << ls) + cm + col;
         } else if (MODE == 1) {
             const int rl = k - xp.g;         // log2 rows per rank
@@ -539,6 +552,8 @@ int ntt_get_tables(zkr_ctx* ctx, int log_n, NttTables** out) {
         ZKR_NTT_ATTR(false, 1, 3);
         ZKR_NTT_ATTR(true, 2, 3);
         ZKR_NTT_ATTR(true, 3, 3);
+        ZKR_NTT_ATTR(false, 4, 3);
+        ZKR_NTT_ATTR(true, 4, 3);
 #undef ZKR_NTT_ATTR
     }
     NttTables* t = new NttTables();
@@ -579,7 +594,7 @@ struct PassGeom {
 
 template <int MODE>
 static int launch_pass(zkr_ctx* ctx, cudaStream_t st, const NttTables* t, Fr* data, const PassGeom& g, bool dit,
-                       bool inverse, const NttXchg& xp, double prof_units, const PassFuse& fz = PassFuse{}) {
+                       bool inverse, const NttXchg& xp, double prof_units, const PassFuse& fz = PassFuse{}, unsigned nvec = 1) {
     const Fr* W = inverse ? t->wsub_i : t->wsub_f;
     const Fr* tlo = inverse ? t->tw_lo_i : t->tw_lo_f;
     const Fr* thi = inverse ? t->tw_hi_i : t->tw_hi_f;
@@ -588,7 +603,7 @@ static int launch_pass(zkr_ctx* ctx, cudaStream_t st, const NttTables* t, Fr* da
     const size_t smem = (size_t)8 * (tile + (tile >> 3) + 4) * sizeof(uint32_t);
     // the pass whose write-back is the all-to-all (remote stores) is timed on its own: bench.py's exchange GB/s
     const int pid = (MODE == 1 || MODE == 2) ? PROF_NTT_XCHG : PROF_NTT_PASS;
-    const dim3 grid(g.blocks, (MODE == 0 && fz.data2) ? 2 : 1);
+    const dim3 grid(g.blocks, (MODE == 0 || MODE == 4) ? (fz.data2 ? 2 : 1) * nvec : 1);
     const int pslot = ctx->prof_begin(pid, st, prof_units * grid.y);
     if (dit) {
         ZKR_LAUNCH(ctx, (k_ntt_pass<true, MODE == 1 ? 3 : MODE, 3>), grid, threads, smem, st, data, g.k, g.c, g.s,
@@ -629,8 +644,9 @@ static int get_twfull(zkr_ctx* ctx, cudaStream_t st, NttTables* t, int i, int ch
 // inverse selects omega^-1; no 1/N scaling is applied here.
 // first / last (nullable): fused element-wise work of the first executed pass's load (ld_op, src, in2, tab) and of the
 // last executed pass's store (st_op, in2, tab, kconst, out).
+// nvec > 1: data (and data2) hold nvec vectors of 2^log_n elements back to back, all transformed by the same launches.
 static int ntt_run_ex(zkr_ctx* ctx, cudaStream_t st, Fr* data, int log_n, bool dit, bool inverse, const PassFuse* first,
-                      const PassFuse* last, Fr* data2 = nullptr) {
+                      const PassFuse* last, Fr* data2 = nullptr, unsigned nvec = 1) {
     NttTables* t;
     ZKR_TRY(ntt_get_tables(ctx, log_n, &t));
     if (log_n < 3) {
@@ -661,6 +677,7 @@ static int ntt_run_ex(zkr_ctx* ctx, cudaStream_t st, Fr* data, int log_n, bool d
         g.blocks = 1u << (log_n - g.k - g.c);
         PassFuse fz = {};
         fz.data2 = data2;
+        fz.vstride = nvec > 1 ? (size_t)1 << log_n : 0;
         if (first && step == 0) {
             fz.ld_op = first->ld_op;
             fz.src = first->src;
@@ -675,7 +692,8 @@ static int ntt_run_ex(zkr_ctx* ctx, cudaStream_t st, Fr* data, int log_n, bool d
             fz.out = last->out;
         }
         if (g.s > 0 && log_n <= twfull_maxlog()) ZKR_TRY(get_twfull(ctx, st, t, i, g.chunk_log, g.k, inverse, &fz.twfull));
-        ZKR_TRY(launch_pass<0>(ctx, st, t, data, g, dit, inverse, none, (double)((size_t)1 << log_n), fz));
+        if (nvec > 1) ZKR_TRY(launch_pass<4>(ctx, st, t, data, g, dit, inverse, none, (double)((size_t)1 << log_n), fz, nvec));
+        else ZKR_TRY(launch_pass<0>(ctx, st, t, data, g, dit, inverse, none, (double)((size_t)1 << log_n), fz));
     }
     return ZKR_OK;
 }
@@ -795,44 +813,59 @@ int ntt_scale_const(zkr_ctx* ctx, cudaStream_t st, Fr* x, size_t n, const Fr* cs
 // pass of their transform loads its tile (LD_MUL2), the coset scaling g^j / m is a table multiply in the load of the DIT
 // transforms' first pass (LD_TAB), and h is assembled in the store of the last pass (ST_HFINAL).  A single-pass transform
 // (m <= 2^11) would need both LD_MUL2's and ST_HFINAL's second operand in one launch: there P is formed by the sweep.
+// The fused pipeline over k vectors of each operand stored back to back (k = 1: the prover's single proof).
+static int h_pipeline_fused(zkr_ctx* ctx, cudaStream_t st, NttTables* t, Fr* A, Fr* B, Fr* S, Fr* h, int log_m, unsigned k) {
+    const size_t m = (size_t)1 << log_m;
+    if (!t->cs_br) {      // cold path: the two position-ordered tables of this size
+        ZKR_CUDA(cudaMalloc(&t->cs_br, m * sizeof(Fr)));
+        ZKR_CUDA(cudaMalloc(&t->hf_br, m * sizeof(Fr)));
+        t->bytes += 2 * m * sizeof(Fr);
+        ZKR_LAUNCH(ctx, k_pow_bitrev, ceil_div(m, 256), 256, 0, st, t->cs_br, log_m, t->cs_lo, t->cs_hi_n, t->lb);
+        ZKR_LAUNCH(ctx, k_pow_bitrev, ceil_div(m, 256), 256, 0, st, t->hf_br, log_m, t->ci_lo, t->ci_hi_h, t->lb);
+    }
+    int ks[4];
+    const bool single = plan_passes(log_m, ks) == 1;
+    PassFuse mulAB = {};
+    mulAB.ld_op = LD_MUL2;
+    mulAB.src = A;
+    mulAB.in2 = B;
+    ZKR_TRY(ntt_run_ex(ctx, st, S, log_m, false, true, &mulAB, nullptr, nullptr, k));  // S <- DIF^-1(A_T . B_T)
+    ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, false, true, nullptr, nullptr, B, k));       // A and B share every launch
+    PassFuse coset = {};
+    coset.ld_op = LD_TAB;
+    coset.tab = t->cs_br;
+    ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, true, false, &coset, nullptr, B, k));       // A, B on the coset g<omega>
+    PassFuse mulP = {}, fin = {};
+    mulP.ld_op = LD_MUL2;
+    mulP.in2 = B;
+    fin.st_op = ST_HFINAL;
+    fin.in2 = S;
+    fin.tab = t->hf_br;
+    fin.kconst = &t->roots->hconst;
+    fin.out = h;
+    if (single) ZKR_LAUNCH(ctx, k_pointwise_mul, ceil_div(k * m, 128), 128, 0, st, A, A, B, k * m);
+    ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, false, true, single ? nullptr : &mulP, &fin, nullptr, k));
+    return ZKR_OK;
+}
+
+int h_pipeline_many(zkr_ctx* ctx, cudaStream_t st, Fr* A, Fr* B, Fr* S, Fr* h, int log_m, int k) {
+    NttTables* t;
+    ZKR_TRY(ntt_get_tables(ctx, log_m, &t));
+    if (log_m < 3 || k < 1 || k > kMaxBatch) {
+        set_error("batched H pipeline: 2^%d points x %d vectors unsupported (2^3 .. 2^27 points, 1 .. %d vectors)", log_m, k,
+                  kMaxBatch);
+        return ZKR_E_UNSUPPORTED;
+    }
+    return h_pipeline_fused(ctx, st, t, A, B, S, h, log_m, (unsigned)k);
+}
+
 int h_pipeline(zkr_ctx* ctx, cudaStream_t st, Fr* A, Fr* B, Fr* S, Fr* h, int log_m, bool bitrev_out) {
     NttTables* t;
     ZKR_TRY(ntt_get_tables(ctx, log_m, &t));
     const size_t m = (size_t)1 << log_m;
     const int blk = 128, grid = ceil_div(m, blk);
     static const bool unfused = getenv("ZKR_H_UNFUSED") && atoi(getenv("ZKR_H_UNFUSED")) != 0;   // A/B knob: round-1 pipeline
-    if (log_m >= 3 && bitrev_out && !unfused) {
-        if (!t->cs_br) {      // cold path: the two position-ordered tables of this size
-            ZKR_CUDA(cudaMalloc(&t->cs_br, m * sizeof(Fr)));
-            ZKR_CUDA(cudaMalloc(&t->hf_br, m * sizeof(Fr)));
-            t->bytes += 2 * m * sizeof(Fr);
-            ZKR_LAUNCH(ctx, k_pow_bitrev, ceil_div(m, 256), 256, 0, st, t->cs_br, log_m, t->cs_lo, t->cs_hi_n, t->lb);
-            ZKR_LAUNCH(ctx, k_pow_bitrev, ceil_div(m, 256), 256, 0, st, t->hf_br, log_m, t->ci_lo, t->ci_hi_h, t->lb);
-        }
-        int ks[4];
-        const bool single = plan_passes(log_m, ks) == 1;
-        PassFuse mulAB = {};
-        mulAB.ld_op = LD_MUL2;
-        mulAB.src = A;
-        mulAB.in2 = B;
-        ZKR_TRY(ntt_run_ex(ctx, st, S, log_m, false, true, &mulAB, nullptr));     // S <- DIF^-1(A_T . B_T)
-        ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, false, true, nullptr, nullptr, B));  // A and B share every launch
-        PassFuse coset = {};
-        coset.ld_op = LD_TAB;
-        coset.tab = t->cs_br;
-        ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, true, false, &coset, nullptr, B));  // A, B on the coset g<omega>
-        PassFuse mulP = {}, fin = {};
-        mulP.ld_op = LD_MUL2;
-        mulP.in2 = B;
-        fin.st_op = ST_HFINAL;
-        fin.in2 = S;
-        fin.tab = t->hf_br;
-        fin.kconst = &t->roots->hconst;
-        fin.out = h;
-        if (single) ZKR_LAUNCH(ctx, k_pointwise_mul, grid, blk, 0, st, A, A, B, m);
-        ZKR_TRY(ntt_run_ex(ctx, st, A, log_m, false, true, single ? nullptr : &mulP, &fin));
-        return ZKR_OK;
-    }
+    if (log_m >= 3 && bitrev_out && !unfused) return h_pipeline_fused(ctx, st, t, A, B, S, h, log_m, 1);
     ZKR_LAUNCH(ctx, k_pointwise_mul, grid, blk, 0, st, S, A, B, m);
     ZKR_TRY(ntt_run(ctx, st, A, log_m, false, true));
     ZKR_TRY(ntt_run(ctx, st, B, log_m, false, true));

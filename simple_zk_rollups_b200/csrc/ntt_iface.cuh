@@ -54,5 +54,8 @@ int ntt_scale_pow_sharded(zkr_ctx* ctx, cudaStream_t st, Fr* x, const NttXchg& g
                           const Fr* lo, const Fr* hi, int lb);
 int ntt_scale_const(zkr_ctx* ctx, cudaStream_t st, Fr* x, size_t n, const Fr* cst);
 int h_pipeline(zkr_ctx* ctx, cudaStream_t st, Fr* A, Fr* B, Fr* S, Fr* h, int log_m, bool bitrev_out);
+// k pipelines in the launches of one: A, B, S, h each hold k vectors of 2^log_m elements back to back; h comes out in
+// bit-reversed order per vector.  The 2 k transforms of A and B share one grid's y dimension.
+int h_pipeline_many(zkr_ctx* ctx, cudaStream_t st, Fr* A, Fr* B, Fr* S, Fr* h, int log_m, int k);
 
 }  // namespace zkr

@@ -62,6 +62,13 @@ namespace {
 enum { R_A = 0, R_B1 = 128, R_C = 256, R_H = 384, R_T1 = 512, R_T2 = 640, R_B2 = 768, R_TOTAL = 1024 };
 
 // A_T[c] = sum_k coef[k] * w[sig[k]]  (coef Montgomery x w standard -> standard)
+__device__ __forceinline__ void sparse_lc(uint32_t c, const uint32_t* __restrict__ ptr, const uint32_t* __restrict__ sig,
+                                          const Fr* __restrict__ coef, const Fr* __restrict__ w, Fr* __restrict__ out) {
+    Fr acc = Fr::zero();
+    const uint32_t e = ptr[c + 1];
+    for (uint32_t k = ptr[c]; k < e; k++) acc = acc + Fr::load_ro(coef + k) * Fr::load_ro(w + sig[k]);
+    acc.store(out + c);
+}
 __global__ void k_sparse_lc(const uint32_t* __restrict__ a_ptr, const uint32_t* __restrict__ a_sig,
                             const Fr* __restrict__ a_coef, const uint32_t* __restrict__ b_ptr,
                             const uint32_t* __restrict__ b_sig, const Fr* __restrict__ b_coef,
@@ -69,33 +76,56 @@ __global__ void k_sparse_lc(const uint32_t* __restrict__ a_ptr, const uint32_t* 
     const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= m) return;
     const bool isb = blockIdx.y != 0;
-    const uint32_t* ptr = isb ? b_ptr : a_ptr;
-    const uint32_t* sig = isb ? b_sig : a_sig;
-    const Fr* coef = isb ? b_coef : a_coef;
-    Fr acc = Fr::zero();
-    const uint32_t e = ptr[c + 1];
-    for (uint32_t k = ptr[c]; k < e; k++) acc = acc + Fr::load_ro(coef + k) * Fr::load_ro(w + sig[k]);
-    acc.store((isb ? bt : at) + c);
+    sparse_lc(c, isb ? b_ptr : a_ptr, isb ? b_sig : a_sig, isb ? b_coef : a_coef, w, isb ? bt : at);
+}
+// batched: proof blockIdx.z reads its witness at w + z wstride and writes its A_T / B_T at at / bt + z m
+__global__ void k_sparse_lc_many(const uint32_t* __restrict__ a_ptr, const uint32_t* __restrict__ a_sig,
+                                 const Fr* __restrict__ a_coef, const uint32_t* __restrict__ b_ptr,
+                                 const uint32_t* __restrict__ b_sig, const Fr* __restrict__ b_coef,
+                                 const Fr* __restrict__ w, size_t wstride, Fr* __restrict__ at, Fr* __restrict__ bt, uint32_t m) {
+    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= m) return;
+    const bool isb = blockIdx.y != 0;
+    const size_t j = blockIdx.z;
+    sparse_lc(c, isb ? b_ptr : a_ptr, isb ? b_sig : a_sig, isb ? b_coef : a_coef, w + j * wstride, (isb ? bt : at) + j * m);
 }
 
-// wext[n] = 1, wext[n+1] = r, wext[n+2] = s, wext[n+3] = -(r s) mod r_order; validates w_0, r, s
-__global__ void k_prep_scalars(Fr* wext, uint32_t n, const Fr* rs, int* err) {
+// wext[n] = 1, wext[n+1] = r, wext[n+2] = s, wext[n+3] = -(r s) mod r_order; returns 1 if r or s >= r, 2 if w_0 != 1
+__device__ __forceinline__ int prep_scalars(Fr* wext, uint32_t n, const Fr* rs) {
     Fr r = Fr::load(rs), s = Fr::load(rs + 1);
-    if (!r.in_range() || !s.in_range()) *err = 1;
+    int e = 0;
+    if (!r.in_range() || !s.in_range()) e = 1;
     Fr one = Fr::zero();
     one.v[0] = 1;
-    if (Fr::load(wext) != one) *err = 2;
+    if (Fr::load(wext) != one) e = 2;
     Fr rsm = (r.to_mont() * s.to_mont()).from_mont();
     one.store(wext + n);
     r.store(wext + n + 1);
     s.store(wext + n + 2);
     rsm.neg().store(wext + n + 3);
+    return e;
+}
+__global__ void k_prep_scalars(Fr* wext, uint32_t n, const Fr* rs, int* err) {
+    const int e = prep_scalars(wext, n, rs);
+    if (e) *err = e;
+}
+// batched: one thread per proof, extended witness j at wext + j (n + 4), (r | s) at rs + 2 j; err[j] |= 1 (r / s), 2 (w_0)
+__global__ void k_prep_scalars_many(Fr* wext, uint32_t n, const Fr* rs, int* err, int k) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= k) return;
+    const int e = prep_scalars(wext + (size_t)j * (n + 4), n, rs + 2 * j);
+    if (e) atomicOr(err + j, e == 2 ? 2 : 1);
 }
 
 // every witness value must be < r (signals that touch no base are read by no MSM)
 __global__ void k_witness_range(const Fr* __restrict__ w, uint32_t n, int* err) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n && !Fr::load_ro(w + i).in_range()) *err = 1;
+}
+// batched: proof blockIdx.y, witness at w + y wstride; err[y] |= 1
+__global__ void k_witness_range_many(const Fr* __restrict__ w, uint32_t n, size_t wstride, int* err) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && !Fr::load_ro(w + blockIdx.y * wstride + i).in_range()) atomicOr(err + blockIdx.y, 1);
 }
 
 // block 0: T1 = s * pi_a ; block 1: T2 = r * pib1.
@@ -106,12 +136,11 @@ __global__ void k_witness_range(const Fr* __restrict__ w, uint32_t n, int* err) 
 // (1.3 ms -> 0.8 ms); it is on the critical path of the small circuits (tx.circom, withdraw.circom), hidden behind
 // the G2 MSM at 2^20 and above.  One active lane per warp on purpose: divergent lanes of one warp would serialise.
 constexpr int kBlindWarps = 8;
-__global__ void __launch_bounds__(32 * kBlindWarps) k_blind_muls(char* res, const Fr* wext, uint32_t n) {
+__device__ __forceinline__ void blind_mul(char* res, const Fr* wext, uint32_t n, bool second) {
     extern __shared__ unsigned char blind_sm[];
     G1XYZZ* chain = reinterpret_cast<G1XYZZ*>(blind_sm);            // [256]
     G1XYZZ* part = chain + 256;                                      // [kBlindWarps]
     __shared__ volatile int ready;                                   // chain[0 .. ready) are published
-    const bool second = blockIdx.x != 0;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const Fr k = Fr::load(wext + n + (second ? 1 : 2));
     int top = 255;
@@ -153,18 +182,26 @@ __global__ void __launch_bounds__(32 * kBlindWarps) k_blind_muls(char* res, cons
         acc.store(res + (second ? R_T2 : R_T1));
     }
 }
+__global__ void __launch_bounds__(32 * kBlindWarps) k_blind_muls(char* res, const Fr* wext, uint32_t n) {
+    blind_mul(res, wext, n, blockIdx.x != 0);
+}
+// batched: blocks 2 j and 2 j + 1 blind proof j (results at res + j R_TOTAL, extended witness at wext + j (n + 4))
+__global__ void __launch_bounds__(32 * kBlindWarps) k_blind_muls_many(char* res, const Fr* wext, uint32_t n) {
+    const uint32_t j = blockIdx.x >> 1;
+    blind_mul(res + (size_t)j * R_TOTAL, wext + (size_t)j * (n + 4), n, blockIdx.x & 1);
+}
 constexpr size_t kBlindSmem = sizeof(G1XYZZ) * (256 + kBlindWarps);
 
 // block 0: pi_a, block 1: pi_b, block 2: pi_c = C + H + T1 + T2; affine, standard form
 // Three single-thread blocks, nothing left to overlap them: the inversion is the whole kernel, so it is the binary
 // extended Euclid of fp_inv.cuh (faster than the a^(p-2) ladder here: profiles/r01_small_circuits_finish_ab.json).
-__global__ void k_finish(const char* res, char* proof) {
-    if (blockIdx.x == 0) {
+__device__ __forceinline__ void finish(const char* res, char* proof, unsigned part) {
+    if (part == 0) {
         const G1XYZZ p = G1XYZZ::load(res + R_A);
         G1Affine a = p.to_affine_vartime();
         a.x.from_mont().store(proof);
         a.y.from_mont().store(proof + 32);
-    } else if (blockIdx.x == 1) {
+    } else if (part == 1) {
         const G2XYZZ p = G2XYZZ::load(res + R_B2);
         G2Affine a = p.to_affine_vartime();
         a.x.from_mont().store(proof + 64);
@@ -177,6 +214,12 @@ __global__ void k_finish(const char* res, char* proof) {
         a.x.from_mont().store(proof + 192);
         a.y.from_mont().store(proof + 224);
     }
+}
+__global__ void k_finish(const char* res, char* proof) { finish(res, proof, blockIdx.x); }
+// batched: blocks 3 j .. 3 j + 2 assemble proof j
+__global__ void k_finish_many(const char* res, char* proof) {
+    const uint32_t j = blockIdx.x / 3;
+    finish(res + (size_t)j * R_TOTAL, proof + (size_t)j * ZKR_PROOF_BYTES, blockIdx.x - 3 * j);
 }
 
 // sharded prove: res[e] = sum over ranks of the gathered partial results (block e: B2 in G2; A, B1, C, H, T1, T2 in
@@ -852,5 +895,204 @@ extern "C" int zkr_prove_batch(zkr_ctx* const* ctxs, const zkr_pkey* const* pks,
             set_error("proof batch failed on context %d: %s", c, msgs[c].c_str());
             return rcs[c];
         }
+    return ZKR_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ many proofs, one pass
+// zkr_prove_many: the k proofs of one call go through every stage together (DESIGN.md 4.10).  Each buffer holds k
+// per-proof slices back to back: extended witnesses at stride n + 4, A_T / B_T / S / h at stride m, results at stride
+// R_TOTAL.  The five MSMs key proof j's digits j * nbuckets + |digit| - 1 over the key's own tables; every kernel takes
+// the proof index from its grid, so the launch count does not depend on k.
+struct zkr_many {
+    zkr_ctx* ctx = nullptr;
+    const zkr_pkey* pk = nullptr;
+    int max_proofs = 0;
+    MsmMany *A = nullptr, *B1 = nullptr, *B2 = nullptr, *C = nullptr, *H = nullptr;
+    Fr* wext = nullptr;                       // k x (n + 4)
+    Fr *at = nullptr, *bt = nullptr, *st = nullptr, *h = nullptr;   // k x m each
+    char* res = nullptr;                      // k x R_TOTAL
+    char* proof = nullptr;                    // k x 256
+    Fr* rs_dev = nullptr;                     // k x 64
+    int* err = nullptr;                       // k flags: 1 a witness value or r / s >= r, 2 witness[0] != 1
+    char* pinned = nullptr;                   // k x (256 proof + 64 r|s + 4 flag)
+    cudaEvent_t ev_b2_sorted = nullptr;
+    size_t bytes = 0;
+};
+
+static void many_release(zkr_many* mw) {
+    if (!mw) return;
+    for (MsmMany* w : {mw->A, mw->B1, mw->B2, mw->C, mw->H}) msm_many_free(w);
+    void* ps[] = {mw->wext, mw->at, mw->bt, mw->st, mw->h, mw->res, mw->proof, mw->rs_dev, mw->err};
+    for (void* p : ps) cudaFree(p);
+    if (mw->pinned) cudaFreeHost(mw->pinned);
+    if (mw->ev_b2_sorted) cudaEventDestroy(mw->ev_b2_sorted);
+    delete mw;
+}
+
+extern "C" int zkr_many_create(zkr_ctx* ctx, const zkr_pkey* pk, int max_proofs, zkr_many** out) {
+    if (!ctx || !pk || !out || pk->ctx != ctx || max_proofs < 1) return ZKR_E_INVALID;
+    *out = nullptr;
+    if (pk->world != 1) {
+        set_error("zkr_many_create: the key is sharded (rank %d of %d); batches need a whole key", pk->rank, pk->world);
+        return ZKR_E_UNSUPPORTED;
+    }
+    if (pk->log_m < 3) {
+        set_error("zkr_many_create: domain size %u; the batched H pipeline needs at least 8", pk->domain_size);
+        return ZKR_E_UNSUPPORTED;
+    }
+    DeviceGuard g(ctx->device);
+    cudaStream_t st = ctx->s[0];
+    zkr_many* mw = new zkr_many();
+    mw->ctx = ctx;
+    mw->pk = pk;
+    mw->max_proofs = max_proofs;
+    const size_t k = (size_t)max_proofs, n = pk->n_vars, m = pk->domain_size;
+    int rc = ZKR_OK;
+#define MANY_TRY(expr)             \
+    do {                           \
+        rc = (expr);               \
+        if (rc != ZKR_OK) {        \
+            many_release(mw);      \
+            return rc;             \
+        }                          \
+    } while (0)
+    // B1' borrows B2''s sort when the two share one (as prove_enqueue does)
+    const bool share = pk->share_b_sort;
+    struct { const zkr_bases* b; MsmMany** w; bool sorts; } sets[] = {
+        {pk->A, &mw->A, true}, {pk->B1, &mw->B1, !share}, {pk->B2, &mw->B2, true}, {pk->C, &mw->C, true}, {pk->H, &mw->H, true}};
+    for (auto& s : sets) {
+        rc = msm_many_alloc(s.b, max_proofs, s.sorts, st, s.w);
+        if (rc != ZKR_OK) {
+            if (rc == ZKR_E_UNSUPPORTED) {
+                std::string why = zkr_last_error();
+                set_error("zkr_many_create: %s", why.c_str());
+            }
+            many_release(mw);
+            return rc;
+        }
+        mw->bytes += msm_many_bytes(*s.w);
+    }
+    auto dmalloc = [&](void** p, size_t bytes) -> int {
+        ZKR_CUDA(cudaMalloc(p, bytes));
+        mw->bytes += bytes;
+        return ZKR_OK;
+    };
+    MANY_TRY(dmalloc((void**)&mw->wext, 32 * k * (n + 4)));
+    MANY_TRY(dmalloc((void**)&mw->at, 32 * k * m));
+    MANY_TRY(dmalloc((void**)&mw->bt, 32 * k * m));
+    MANY_TRY(dmalloc((void**)&mw->st, 32 * k * m));
+    MANY_TRY(dmalloc((void**)&mw->h, 32 * k * m));
+    MANY_TRY(dmalloc((void**)&mw->res, R_TOTAL * k));
+    MANY_TRY(dmalloc((void**)&mw->proof, ZKR_PROOF_BYTES * k));
+    MANY_TRY(dmalloc((void**)&mw->rs_dev, 64 * k));
+    MANY_TRY(dmalloc((void**)&mw->err, sizeof(int) * k));
+    if (cudaMallocHost((void**)&mw->pinned, (ZKR_PROOF_BYTES + 64 + sizeof(int)) * k) != cudaSuccess) {
+        cudaGetLastError();
+        many_release(mw);
+        set_error("zkr_many_create: no pinned host memory for %d proofs", max_proofs);
+        return ZKR_E_NOMEM;
+    }
+    if (cudaEventCreateWithFlags(&mw->ev_b2_sorted, cudaEventDisableTiming) != cudaSuccess) {
+        many_release(mw);
+        return ZKR_E_CUDA;
+    }
+#undef MANY_TRY
+    *out = mw;
+    return ZKR_OK;
+}
+
+extern "C" void zkr_many_free(zkr_many* mw) {
+    if (!mw) return;
+    DeviceGuard g(mw->ctx->device);
+    cudaDeviceSynchronize();
+    many_release(mw);
+}
+
+extern "C" int zkr_many_info(const zkr_many* mw, int* max_proofs, uint64_t* device_bytes) {
+    if (!mw) return ZKR_E_INVALID;
+    if (max_proofs) *max_proofs = mw->max_proofs;
+    if (device_bytes) *device_bytes = mw->bytes;
+    return ZKR_OK;
+}
+
+static bool below_r(const uint8_t* v32) {
+    for (int i = 7; i >= 0; i--) {
+        uint32_t x;
+        memcpy(&x, v32 + 4 * i, 4);
+        if (x != kRModulus[i]) return x < kRModulus[i];
+    }
+    return false;
+}
+
+extern "C" int zkr_prove_many(zkr_ctx* ctx, zkr_many* mw, const void* witnesses, size_t n_signals, int n_proofs,
+                              const void* rs32, void* out_proofs) {
+    if (!ctx || !mw || !witnesses || !out_proofs || mw->ctx != ctx) return ZKR_E_INVALID;
+    const zkr_pkey* pk = mw->pk;
+    if (n_proofs < 1 || n_proofs > mw->max_proofs) {
+        set_error("zkr_prove_many: %d proofs, the workspace holds 1 .. %d", n_proofs, mw->max_proofs);
+        return ZKR_E_INVALID;
+    }
+    if (n_signals != pk->n_vars) {
+        set_error("witness has %zu signals, key expects %u", n_signals, pk->n_vars);
+        return ZKR_E_INVALID;
+    }
+    const int k = n_proofs;
+    const uint32_t n = pk->n_vars, m = pk->domain_size;
+    const size_t ws = (size_t)n + 4;
+    char* pin_proof = mw->pinned;
+    char* pin_rs = pin_proof + (size_t)ZKR_PROOF_BYTES * mw->max_proofs;
+    int* pin_err = (int*)(pin_rs + 64ull * mw->max_proofs);
+    if (rs32) {
+        for (int j = 0; j < k; j++)
+            for (int h = 0; h < 2; h++)
+                if (!below_r((const uint8_t*)rs32 + 64ull * j + 32 * h)) {
+                    set_error("proof %d: blinding scalar %s is >= r", j, h ? "s" : "r");
+                    return ZKR_E_INVALID;
+                }
+        memcpy(pin_rs, rs32, 64ull * k);
+    } else {
+        for (int j = 0; j < k; j++) ZKR_TRY(stage_blinding(pin_rs + 64ull * j, nullptr, nullptr));
+    }
+    DeviceGuard g(ctx->device);
+    cudaStream_t us = ctx->user_stream;
+    ZKR_CUDA(cudaMemsetAsync(mw->err, 0, sizeof(int) * k, us));
+    // k witnesses into their n + 4 slots: one strided copy
+    ZKR_CUDA(cudaMemcpy2DAsync(mw->wext, 32 * ws, witnesses, 32ull * n, 32ull * n, k, cudaMemcpyHostToDevice, us));
+    ZKR_CUDA(cudaMemcpyAsync(mw->rs_dev, pin_rs, 64ull * k, cudaMemcpyHostToDevice, us));
+    ZKR_LAUNCH(ctx, k_prep_scalars_many, ceil_div(k, 64), 64, 0, us, mw->wext, n, (const Fr*)mw->rs_dev, mw->err, k);
+    ZKR_LAUNCH(ctx, k_witness_range_many, dim3(ceil_div(n, 256), k), 256, 0, us, mw->wext, n, ws, mw->err);
+    // the streams and the order of prove_enqueue: s[0] = H, s[1] = A, s[2] = B1, s[3] = B2, s[4] = C
+    const bool par = !ctx->serial;
+    if (par) ZKR_TRY(ctx->fork(5));
+    cudaStream_t sH = par ? ctx->s[0] : us, sA = par ? ctx->s[1] : us, sB1 = par ? ctx->s[2] : us,
+                 sB2 = par ? ctx->s[3] : us, sC = par ? ctx->s[4] : us;
+    const uint32_t* w = (const uint32_t*)mw->wext;
+    const bool share = pk->share_b_sort;
+    ZKR_TRY(msm_many_run(ctx, sB2, pk->B2, mw->B2, k, w, ws, mw->res + R_B2, R_TOTAL, nullptr,
+                         share ? mw->ev_b2_sorted : nullptr));
+    ZKR_LAUNCH(ctx, k_sparse_lc_many, dim3(ceil_div(m, 128), 2, k), 128, 0, sH, pk->a_ptr, pk->a_sig, pk->a_coef, pk->b_ptr,
+               pk->b_sig, pk->b_coef, mw->wext, ws, mw->at, mw->bt, m);
+    ZKR_TRY(h_pipeline_many(ctx, sH, mw->at, mw->bt, mw->st, mw->h, pk->log_m, k));
+    ZKR_TRY(msm_many_run(ctx, sH, pk->H, mw->H, k, (const uint32_t*)mw->h, m, mw->res + R_H, R_TOTAL));
+    ZKR_TRY(msm_many_run(ctx, sA, pk->A, mw->A, k, w, ws, mw->res + R_A, R_TOTAL));
+    if (share) ZKR_CUDA(cudaStreamWaitEvent(sB1, mw->ev_b2_sorted, 0));
+    ZKR_TRY(msm_many_run(ctx, sB1, pk->B1, mw->B1, k, w, ws, mw->res + R_B1, R_TOTAL, share ? mw->B2 : nullptr));
+    ZKR_TRY(msm_many_run(ctx, sC, pk->C, mw->C, k, w, ws, mw->res + R_C, R_TOTAL));
+    if (par) {
+        ZKR_CUDA(cudaEventRecord(ctx->ev_join[2], sB1));
+        ZKR_CUDA(cudaStreamWaitEvent(sA, ctx->ev_join[2], 0));
+    }
+    ZKR_LAUNCH(ctx, k_blind_muls_many, 2 * k, 32 * kBlindWarps, kBlindSmem, sA, mw->res, mw->wext, n);
+    if (par) ZKR_TRY(ctx->join(5));
+    ZKR_LAUNCH(ctx, k_finish_many, 3 * k, 1, 0, us, (const char*)mw->res, mw->proof);
+    ZKR_CUDA(cudaMemcpyAsync(pin_proof, mw->proof, (size_t)ZKR_PROOF_BYTES * k, cudaMemcpyDeviceToHost, us));
+    ZKR_CUDA(cudaMemcpyAsync(pin_err, mw->err, sizeof(int) * k, cudaMemcpyDeviceToHost, us));
+    ZKR_CUDA(cudaStreamSynchronize(us));
+    for (int j = 0; j < k; j++)
+        if (pin_err[j]) {
+            set_error(pin_err[j] & 2 ? "proof %d: witness[0] must be 1" : "proof %d: a witness value is >= r", j);
+            return ZKR_E_WITNESS_RANGE;
+        }
+    memcpy(out_proofs, pin_proof, (size_t)ZKR_PROOF_BYTES * k);
     return ZKR_OK;
 }

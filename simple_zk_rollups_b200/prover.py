@@ -31,8 +31,11 @@ class Groth16Prover:
         self.device = device
         self._keys = []
         self._vkeys = []
+        self._manys = []
 
     def close(self):
+        for h in list(self._manys):                   # workspaces share their key's tables: freed before the keys
+            h.close()
         for k in self._keys:
             self.L.zkr_pkey_free(k)
         self._keys = []
@@ -131,6 +134,65 @@ class Groth16Prover:
 
     def kernel_launches(self):
         return int(self.L.zkr_ctx_kernel_launches(self.ctx))
+
+    def create_many(self, key, max_proofs):
+        """Work buffers for proving up to max_proofs witnesses of `key` in one pass (zkr_many_create).  The key's
+        tables are shared; close the handle before the key is freed."""
+        h = C.c_void_p()
+        _lib.check(self.L.zkr_many_create(self.ctx, key, int(max_proofs), C.byref(h)))
+        m = ManyHandle(self, h)
+        self._manys.append(m)
+        return m
+
+    def prove_many(self, handle, witness_bins, rs=None):
+        """zkr_prove_many: every witness of the list proved in one pass through every stage.  witness_bins:
+        binarifyWitness outputs of one key; rs: optional list of (r, s) ints, None draws a fresh CSPRNG pair per proof.
+        -> list of 256-byte proofs, proof j byte-identical to prove(key, witness_bins[j], *rs[j])."""
+        n = len(witness_bins)
+        ws = [np.frombuffer(w, dtype=np.uint8) if isinstance(w, (bytes, bytearray)) else np.asarray(w, dtype=np.uint8)
+              for w in witness_bins]
+        if n == 0:
+            return []
+        if any(w.size != ws[0].size for w in ws):
+            raise ValueError("all witnesses of a batch must have the same length")
+        flat = np.ascontiguousarray(np.concatenate(ws))
+        rsb = None
+        if rs is not None:
+            if len(rs) != n:
+                raise ValueError("rs must give one (r, s) pair per witness")
+            rsb = np.frombuffer(b"".join(int(r).to_bytes(32, "little") + int(s).to_bytes(32, "little") for r, s in rs),
+                                dtype=np.uint8)
+        out = np.zeros(n * _lib.PROOF_BYTES, dtype=np.uint8)
+        _lib.check(self.L.zkr_prove_many(self.ctx, handle.h, _lib.buf_ptr(flat), ws[0].size // 32, n, _lib.buf_ptr(rsb),
+                                         _lib.buf_ptr(out)))
+        return [out[i * _lib.PROOF_BYTES:(i + 1) * _lib.PROOF_BYTES].tobytes() for i in range(n)]
+
+    def msm_many(self, bases, scalars, n, n_vectors, group=1):
+        """zkr_msm_many: n_vectors MSMs over one base set (a zkr_bases handle of this context).  scalars: n_vectors x n
+        x 32 bytes, std form.  -> list of affine std-form results (64 bytes for G1, 128 for G2), one per vector."""
+        sc = np.frombuffer(scalars, dtype=np.uint8) if isinstance(scalars, (bytes, bytearray)) else np.ascontiguousarray(scalars)
+        ob = 64 if group == 1 else 128
+        out = np.zeros(n_vectors * ob, dtype=np.uint8)
+        _lib.check(self.L.zkr_msm_many(self.ctx, bases, _lib.buf_ptr(sc), n, n_vectors, 0, _lib.buf_ptr(out)))
+        return [out[i * ob:(i + 1) * ob].tobytes() for i in range(n_vectors)]
+
+
+class ManyHandle:
+    """A zkr_many workspace (Groth16Prover.create_many); close() frees it."""
+
+    def __init__(self, prover, h):
+        self.prover, self.h = prover, h
+
+    def info(self):
+        k, b = C.c_int(), C.c_uint64()
+        _lib.check(self.prover.L.zkr_many_info(self.h, C.byref(k), C.byref(b)))
+        return dict(max_proofs=k.value, device_bytes=b.value)
+
+    def close(self):
+        if self.h:
+            self.prover.L.zkr_many_free(self.h)
+            self.h = C.c_void_p()
+            self.prover._manys.remove(self)
 
 
 def prove_batch(provers, keys, witness_bins, rs=None):

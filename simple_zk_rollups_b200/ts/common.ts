@@ -95,3 +95,19 @@ export const genProof = async (provingKey, witness, r?: Uint8Array, s?: Uint8Arr
     publicSignals: witness.slice(1, provingKey.nPublic + 1)
   };
 };
+
+// Many witnesses of one circuit in one pass on the GPU (zkr_prove_many): key = a zkr.loadKey handle, witnesses =
+// binarifyWitness outputs, rs = optional (r|s) pairs of 64 bytes (absent: fresh CSPRNG pairs in libzkr).
+// -> one 256-byte proof per witness, in input order.
+export const proveMany = async (key, witnesses: ArrayBuffer[], rs?: Uint8Array[]): Promise<Uint8Array[]> => {
+  const wb = witnesses.length ? witnesses[0].byteLength : 0;
+  const all = new Uint8Array(wb * witnesses.length);
+  witnesses.forEach((w, j) => all.set(new Uint8Array(w), wb * j));
+  let rsAll: Uint8Array | undefined;
+  if (rs) {
+    rsAll = new Uint8Array(64 * rs.length);
+    rs.forEach((x, j) => rsAll.set(x, 64 * j));
+  }
+  const p: Uint8Array = await zkr.proveMany(key, all.buffer, rsAll);
+  return witnesses.map((_, j) => p.subarray(256 * j, 256 * (j + 1)));
+};

@@ -23,9 +23,15 @@
 //   loadVerifyingKey(vkJsonText: Buffer) -> vkHandle               zkr_vkey_load_json, once per circuit
 //   verify(vk, proof: Uint8Array(256), publicSignalsBin: ArrayBuffer) -> boolean
 //        zkr_verify: replaces groth.isValid (common.ts:30-34); ~ms, synchronous
+//   proveMany(key, witnessesBin: ArrayBuffer, rs?: Uint8Array(64 k)) -> Promise<Uint8Array(256 k)>
+//        zkr_prove_many: k witnesses of the key back to back (k x nVars x 32 B), proved in one pass on a worker thread,
+//        under the same mutex as prove; proof j is bytes [256 j, 256 (j+1)).  rs: k (r|s) pairs, or absent = CSPRNG.
+//        The key's batch workspace (zkr_many) is created on first use, grown to the largest batch seen and freed with
+//        the key.  common.ts's proveMany(key, witnesses[], rs?) -> Promise<Uint8Array[]> wraps it.
 #include <node_api.h>
 
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -37,6 +43,11 @@ namespace {
 zkr_ctx* g_ctx = nullptr;
 std::mutex g_mu;             // serialises every zkr_* call on g_ctx (see "Threading" above)
 using Lock = std::lock_guard<std::mutex>;
+struct Many {
+    zkr_many* mw = nullptr;
+    int cap = 0;
+};
+std::map<zkr_pkey*, Many> g_many;          // proveMany's workspace per key, grown to the largest batch seen (under g_mu)
 
 bool ensure_ctx(napi_env env) {
     Lock lk(g_mu);
@@ -51,7 +62,10 @@ bool ensure_ctx(napi_env env) {
 
 void free_key(napi_env, void* data, void*) {
     Lock lk(g_mu);
-    zkr_pkey_free(static_cast<zkr_pkey*>(data));
+    zkr_pkey* pk = static_cast<zkr_pkey*>(data);
+    zkr_many_free(g_many[pk].mw);        // proveMany's workspace shares the key's tables: freed first (null: none)
+    g_many.erase(pk);
+    zkr_pkey_free(pk);
 }
 
 napi_value LoadKey(napi_env env, napi_callback_info info) {
@@ -243,6 +257,91 @@ napi_value Prove(napi_env env, napi_callback_info info) {
     return promise;
 }
 
+struct ProveManyJob {
+    napi_async_work work;
+    napi_deferred deferred;
+    zkr_pkey* pk;
+    std::vector<uint8_t> witnesses, rs, proofs;
+    int rc;
+    std::string err;
+    // whole witnesses of n_vars signals in the buffer (and as many (r|s) pairs, if given); 0 and rc set otherwise
+    int count(uint32_t n_vars) {
+        const size_t wb = 32ull * n_vars, k = wb ? witnesses.size() / wb : 0;
+        if (k == 0 || k > 32767 || witnesses.size() != k * wb || (!rs.empty() && rs.size() != 64 * k)) {
+            rc = ZKR_E_INVALID;
+            err = "proveMany: witnessesBin must hold 1 .. 32767 whole witnesses of the key, rs one (r|s) pair per witness";
+            return 0;
+        }
+        proofs.resize(ZKR_PROOF_BYTES * k);
+        return (int)k;
+    }
+};
+
+void ProveManyExecute(napi_env, void* data) {   // worker thread
+    ProveManyJob* j = static_cast<ProveManyJob*>(data);
+    Lock lk(g_mu);
+    uint32_t n = 0;
+    Many& m = g_many[j->pk];
+    j->rc = zkr_pkey_info(j->pk, &n, nullptr, nullptr, nullptr);
+    const int k = j->rc == ZKR_OK ? j->count(n) : 0;
+    if (k > m.cap) zkr_many_free(m.mw), m = Many{}, j->rc = zkr_many_create(g_ctx, j->pk, k, &m.mw), m.cap = j->rc ? 0 : k;
+    if (k > 0 && j->rc == ZKR_OK) j->rc = zkr_prove_many(g_ctx, m.mw, j->witnesses.data(), n, k, j->rs.empty() ? nullptr : j->rs.data(), j->proofs.data());
+    if (j->rc != ZKR_OK && j->err.empty()) j->err = zkr_last_error();
+}
+
+void ProveManyComplete(napi_env env, napi_status, void* data) {
+    ProveManyJob* j = static_cast<ProveManyJob*>(data);
+    if (j->rc == ZKR_OK) {
+        void* out;
+        napi_value ab, u8;
+        napi_create_arraybuffer(env, j->proofs.size(), &out, &ab);
+        memcpy(out, j->proofs.data(), j->proofs.size());
+        napi_create_typedarray(env, napi_uint8_array, j->proofs.size(), ab, 0, &u8);
+        napi_resolve_deferred(env, j->deferred, u8);
+    } else {
+        napi_value msg, err;
+        napi_create_string_utf8(env, j->err.c_str(), NAPI_AUTO_LENGTH, &msg);
+        napi_create_error(env, nullptr, msg, &err);
+        napi_reject_deferred(env, j->deferred, err);
+    }
+    napi_delete_async_work(env, j->work);
+    delete j;
+}
+
+napi_value ProveMany(napi_env env, napi_callback_info info) {
+    size_t argc = 3;
+    napi_value argv[3];
+    napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
+    void *pkv, *wbuf, *rdata = nullptr;
+    size_t wlen, rlen = 0;
+    bool ok = argc >= 2 && napi_get_value_external(env, argv[0], &pkv) == napi_ok &&
+              napi_get_arraybuffer_info(env, argv[1], &wbuf, &wlen) == napi_ok;
+    if (ok && argc > 2) {
+        napi_valuetype t;
+        napi_typeof(env, argv[2], &t);
+        if (t != napi_undefined && t != napi_null) {
+            napi_typedarray_type ty;
+            napi_value ab;
+            size_t off;
+            ok = napi_get_typedarray_info(env, argv[2], &ty, &rlen, &rdata, &ab, &off) == napi_ok && ty == napi_uint8_array;
+        }
+    }
+    if (!ok) {
+        napi_throw_type_error(env, nullptr, "proveMany(key, witnessesBin: ArrayBuffer, rs?: Uint8Array)");
+        return nullptr;
+    }
+    ProveManyJob* j = new ProveManyJob();
+    j->pk = static_cast<zkr_pkey*>(pkv);
+    j->witnesses.assign(static_cast<uint8_t*>(wbuf), static_cast<uint8_t*>(wbuf) + wlen);   // JS may GC the buffers
+    if (rdata) j->rs.assign(static_cast<uint8_t*>(rdata), static_cast<uint8_t*>(rdata) + rlen);
+    napi_value promise, name;
+    napi_create_promise(env, &j->deferred, &promise);
+    napi_create_string_utf8(env, "zkr_prove_many", NAPI_AUTO_LENGTH, &name);
+    napi_create_async_work(env, nullptr, name, ProveManyExecute, ProveManyComplete, j, &j->work);
+    napi_queue_async_work(env, j->work);
+    return promise;
+}
+
 napi_value Init(napi_env env, napi_value exports) {
     napi_value f;
     napi_create_function(env, "loadKey", NAPI_AUTO_LENGTH, LoadKey, nullptr, &f);
@@ -255,6 +354,8 @@ napi_value Init(napi_env env, napi_value exports) {
     napi_set_named_property(env, exports, "loadVerifyingKey", f);
     napi_create_function(env, "verify", NAPI_AUTO_LENGTH, Verify, nullptr, &f);
     napi_set_named_property(env, exports, "verify", f);
+    napi_create_function(env, "proveMany", NAPI_AUTO_LENGTH, ProveMany, nullptr, &f);
+    napi_set_named_property(env, exports, "proveMany", f);
     return exports;
 }
 
